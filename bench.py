@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # B200 arm (libgenpose_b200.so)
     python bench.py --impl reference --gpus N ...             # the reference's CPU path on the host cores
+    python bench.py ... --dump-outputs DIR                    # also writes the last timed step's outputs as DIR/*.npy
 
 A "step" is one pass of the full path (PointNet++ encoder x2 -> RK45 ScoreNet sampling, 50 hypotheses/object ->
 EnergyNet scoring -> aggregation -> ScaleNet) over one batch of synthetic objects.
@@ -60,21 +61,26 @@ OBJECT_ONCE_FLOP = 2 * 786432
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps, all of which run (after the warm-up), in either arm")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", type=str, default="b200", choices=["b200", "reference"])
     ap.add_argument("--objects", type=int, default=OBJECTS_PER_GPU, help="objects per GPU per step")
     ap.add_argument("--mlp_mode", type=str, default="fp32", choices=["fp32", "fp32_ffma", "bf16"])
     ap.add_argument("--cpu_sample_objects", type=int, default=8, help="cpu_baseline sample of the B200 arm")
     ap.add_argument("--ref_objects", type=int, default=OBJECTS_PER_GPU, help="objects per step of --impl reference")
-    ap.add_argument("--ref_budget_s", type=float, default=200.0, help="wall-clock cap of --impl reference")
     ap.add_argument("--no_cpu_baseline", action="store_true")
     ap.add_argument("--single_mode", action="store_true", help="skip the measurement of the other mlp_mode")
     ap.add_argument("--no_extras", action="store_true", help="skip other_configs and reference_gpu")
     ap.add_argument("--c5_objects", type=int, default=C5_OBJECTS)
     ap.add_argument("--graph", type=str, default="on", choices=["on", "off"],
                     help="replay the step as one CUDA graph (PosePipeline(use_graph=True)); falls back to eager launches if the capture fails")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (aggregated_pose [B,4,4], "
+                         "length [B,3], all ranks' objects in order) as DIR/<name>.npy in float32, in either arm")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def measured_peaks():
@@ -198,7 +204,7 @@ class CpuReference:
                 print("reference modules not loadable, timing the oracle port instead:", e, file=sys.stderr)
 
     def step(self, n):
-        """-> (seconds, seconds spent in the two encoder passes)"""
+        """-> (seconds, seconds spent in the two encoder passes, (aggregated_pose, length))"""
         import torch
         from oracle import pose_oracle as po
         pts, center = self.pts[:n], self.center[:n]
@@ -206,15 +212,15 @@ class CpuReference:
         if self.agents is None:
             torch.manual_seed(1)
             noise = po.ve_prior((n * REPEAT, 9), T=T0)
-            po.full_pipeline(self.sds[0], self.sds[1], self.sds[2], pts, center, noise, repeat_num=REPEAT, T0=T0,
-                             integrator="scipy")
-            return time.perf_counter() - t0, None
+            out = po.full_pipeline(self.sds[0], self.sds[1], self.sds[2], pts, center, noise, repeat_num=REPEAT, T0=T0,
+                                   integrator="scipy")
+            return time.perf_counter() - t0, None, (out["aggregated_pose"], out["length"])
         with torch.no_grad():
             sfeat = po.pointnet2_encoder(self.sds[0], pts)
             efeat = po.pointnet2_encoder(self.sds[1], pts)
         t_enc = time.perf_counter() - t0
-        self.agents.full(pts, center, REPEAT, T0, noise_seed=1, score_feat=sfeat, energy_feat=efeat)
-        return time.perf_counter() - t0, t_enc
+        out = self.agents.full(pts, center, REPEAT, T0, noise_seed=1, score_feat=sfeat, energy_feat=efeat)
+        return time.perf_counter() - t0, t_enc, (out["aggregated_pose"], out["length"])
 
     def describe(self, n, steps, enc_share):
         what = ("reference modules (oracle/_ref/refpkg): torch-CPU nets + scipy RK45 + sklearn DBSCAN; the CUDA-only "
@@ -233,16 +239,14 @@ def run_reference(args):
     import torch
     n = args.ref_objects
     ref = CpuReference(n)
-    t_begin = time.perf_counter()
-    ref.step(min(n, 4))  # warm-up (thread pools, imports); a full-size warm-up step would not fit the time budget
+    ref.step(min(n, 4))  # warm-up (thread pools, imports) on a few objects: a full-size step takes seconds on the host
     times, encs = [], []
-    for _ in range(max(1, args.steps)):
-        dt, enc = ref.step(n)
+    for _ in range(args.steps):
+        dt, enc, outputs = ref.step(n)
         times.append(dt)
         encs.append(enc)
-        # bounded: the whole run must end within a few minutes whatever K the driver passes
-        if time.perf_counter() - t_begin + dt > args.ref_budget_s:
-            break
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *outputs, rank)
     total = sum(times)
     value = n * len(times) / total
     cores = torch.get_num_threads()
@@ -253,8 +257,7 @@ def run_reference(args):
         "steps_timed": len(times), "warmup": args.warmup, "ms_per_step": 1e3 * total / len(times),
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": f"C2: {OBJECTS_PER_GPU} objects x {REPEAT} hypotheses, full path, T0={T0}",
-                   "objects_per_step": n, "same_config": n == OBJECTS_PER_GPU,
-                   "note": f"steps are capped by a {args.ref_budget_s:.0f} s wall-clock budget (steps_timed of steps ran)"},
+                   "objects_per_step": n, "same_config": n == OBJECTS_PER_GPU},
         "cpu_baseline": {"value": value, "unit": UNIT, "cores": cores, "kind": ref.kind, "sample": sample,
                          "os_cpu_count": os.cpu_count()},
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
@@ -296,6 +299,19 @@ def load_ref_ext():
         return pointnet2_cuda
     except Exception:  # noqa: BLE001
         return None
+
+
+def dump_outputs(out_dir, pose, length, rank):
+    """--dump-outputs: the last timed step's results, gathered over the ranks in object order, as float32 .npy files.
+    The clouds, weights and prior noise depend on the arguments alone, so two builds can be compared output for output."""
+    import numpy as np
+    from genpose2_b200.pipeline import gather_results
+    pose, length = gather_results(pose, length)
+    if rank != 0:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("aggregated_pose", pose), ("length", length)):
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def sampler_inputs(net, feat, center_d, B, T, seed=99):
@@ -638,7 +654,7 @@ def run_b200(args):
         for s, e in evs:
             flush.zero_()  # L2 flush between timed iterations (inputs are far smaller than the 126 MB L2)
             s.record()
-            fn()
+            out = fn()
             e.record()
         torch.cuda.synchronize()
         clocks = sampler.stop() if sampler else None
@@ -650,6 +666,7 @@ def run_b200(args):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             total_ms = float(t.item())
         timed.last_spread = {"min": min(per_step), "median": sorted(per_step)[len(per_step) // 2], "max": max(per_step)}
+        timed.last_out = out
         return total_ms, clocks
 
     def measure(mlp_mode, with_e2e, with_clocks):
@@ -687,7 +704,7 @@ def run_b200(args):
         total_ms, clocks = timed(step_resident, args.steps, sampler)
         from genpose2_b200 import samplers as _s
         launches = pipe.graph_launches * args.steps if pipe.use_graph else _lib.launch_count()
-        res = {"launches": launches, "graph": graph_note, "total_ms": total_ms, "clocks": clocks,
+        res = {"launches": launches, "graph": graph_note, "total_ms": total_ms, "clocks": clocks, "outputs": timed.last_out,
                "value": world * B * args.steps / (total_ms * 1e-3), "step_ms_spread": timed.last_spread,
                "last_step_ode": {k: v for k, v in _s.ode_stats().items() if k in ("nfev", "accepted", "rejected", "status")}}
         if with_e2e:
@@ -714,6 +731,8 @@ def run_b200(args):
         return res
 
     main_res = measure(args.mlp_mode, True, True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *main_res["outputs"], rank)
     other_mode = "bf16" if args.mlp_mode != "bf16" else "fp32"
     other_res = measure(other_mode, False, False) if not args.single_mode else None
     value, total_ms, clocks, launches = main_res["value"], main_res["total_ms"], main_res["clocks"], main_res["launches"]
@@ -752,7 +771,7 @@ def run_b200(args):
         ref = CpuReference(n)
         ref.step(min(n, 2))  # warm-up
         reps = [ref.step(n) for _ in range(3)]
-        med, enc = sorted(reps, key=lambda r: r[0])[1]
+        med, enc, _ = sorted(reps, key=lambda r: r[0])[1]
         cpu_baseline = {"value": n / med, "unit": UNIT, "cores": torch.get_num_threads(), "kind": ref.kind,
                         "sample": ref.describe(n, 3, None if enc is None else enc / med) + ", median",
                         "os_cpu_count": os.cpu_count()}

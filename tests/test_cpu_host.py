@@ -306,3 +306,40 @@ def test_trajectory_buffer_is_bounded_by_a_byte_budget():
     slots = samplers._traj_slots(n)
     assert 64 <= slots < samplers.MAX_TRAJ and slots * n * 72 <= samplers.TRAJ_BYTES_BUDGET + 64 * n * 72
     assert samplers._traj_slots(10 ** 9) == 64
+
+
+def test_bench_rejects_zero_timed_steps():
+    """bench.py refuses, before any work, a run with no timed step"""
+    run = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True)
+    assert run.returncode == 2 and "--steps" in run.stderr, run.stderr
+
+
+def test_bench_reference_arm_runs_every_step_and_dumps_the_last(tmp_path):
+    """bench.py --impl reference times exactly --steps steps, and --dump-outputs writes what the last one returned:
+    the CPU path on the bench's first cloud with the prior noise drawn after torch.manual_seed(1)"""
+    import json
+    import numpy as np
+    from genpose2_b200 import synthetic
+    from oracle import pose_oracle as po
+    run = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2",
+                          "--ref_objects", "1", "--dump-outputs", str(tmp_path)], capture_output=True, text=True)
+    assert run.returncode == 0, run.stderr[-3000:]
+    line = json.loads([s for s in run.stdout.splitlines() if s.startswith("{")][-1])
+    assert line["steps"] == line["steps_timed"] == 2
+    pose, length = np.load(tmp_path / "aggregated_pose.npy"), np.load(tmp_path / "length.npy")
+    assert pose.dtype == length.dtype == np.float32 and pose.shape == (1, 4, 4) and length.shape == (1, 3)
+    if line["cpu_baseline"]["kind"] != "port":
+        return   # the reference's own modules computed it: compared with the port by tests/test_gpu_reference.py
+    pts, center = synthetic.make_point_clouds(1, 1024, seed=0)
+    threads = torch.get_num_threads()
+    torch.set_num_threads(os.cpu_count() or 1)   # the bench's setting: torch-CPU sums in a thread-count-dependent order
+    try:
+        torch.manual_seed(1)
+        noise = po.ve_prior((50, 9), T=0.55)
+        want = po.full_pipeline(synthetic.random_gfobjectpose_state_dict(100), synthetic.random_gfobjectpose_state_dict(200),
+                                synthetic.random_scalenet_state_dict(300), pts, center, noise, repeat_num=50, T0=0.55,
+                                integrator="scipy")
+    finally:
+        torch.set_num_threads(threads)
+    np.testing.assert_array_equal(pose, want["aggregated_pose"].float().numpy())
+    np.testing.assert_array_equal(length, want["length"].float().numpy())

@@ -224,3 +224,30 @@ def test_cuda_graph_step_equals_eager_step():
     torch.manual_seed(9)
     g_pose, g_len = graph(dict(data), repeat_num=50, T0=0.25, init_x=init.cuda())
     assert torch.equal(a_pose, g_pose) and torch.equal(a_len, g_len)
+
+
+def test_bench_dump_outputs_are_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs writes what its last timed step returned: bit-identical to an eager PosePipeline making
+    the same calls from the same seed (the warm-up steps, at least 3, then --steps timed steps)."""
+    import json
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    B, steps = 4, 2
+    run = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", str(steps),
+                          "--warmup", "1", "--objects", str(B), "--single_mode", "--no_extras", "--no_cpu_baseline",
+                          "--dump-outputs", str(tmp_path)], capture_output=True, text=True)
+    assert run.returncode == 0, run.stderr[-3000:]
+    line = json.loads([s for s in run.stdout.splitlines() if s.startswith("{")][-1])
+    assert line["steps"] == steps and line["warmup"] == 3
+    pose, length = np.load(tmp_path / "aggregated_pose.npy"), np.load(tmp_path / "length.npy")
+    assert pose.dtype == length.dtype == np.float32 and pose.shape == (B, 4, 4) and length.shape == (B, 3)
+    pipe = make_pipeline()
+    pts, center = synthetic.make_point_clouds(B, 1024, seed=0)
+    data = {"pts": pts.cuda(), "pts_center": center.cuda()}
+    torch.manual_seed(1234)
+    for _ in range(3 + steps):
+        want_pose, want_len = pipe(dict(data), repeat_num=50, T0=0.55)
+    np.testing.assert_array_equal(pose, want_pose.cpu().numpy())
+    np.testing.assert_array_equal(length, want_len.cpu().numpy())

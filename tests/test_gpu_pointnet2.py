@@ -32,7 +32,7 @@ def ref_bq(ext, radius, ns, xyz, new_xyz):
     return idx
 
 
-@pytest.mark.parametrize("N", [1, 2, 5, 33, 64, 128, 256, 512, 1000, 1024, 1500, 2048, 4096])
+@pytest.mark.parametrize("N", [1, 2, 5, 33, 64, 128, 256, 512, 1000, 1024, 1500, 2048, 4096, 8192, 16384])
 def test_fps_bit_exact_vs_oracle(N):
     from genpose2_b200 import pointnet2_utils as pu
     B = 6 if N <= 1024 else 2

@@ -12,6 +12,17 @@ from genpose2_b200 import synthetic
 from oracle import pose_oracle as po
 
 
+@pytest.fixture(autouse=True)
+def golden_thread_count():
+    """tests/golden/make_golden.py ran the reference with torch.set_num_threads(8), and torch-CPU's summation order
+    depends on the thread count: the restatement runs with the same count so that it agrees with the goldens to
+    rounding on a host with any number of cores."""
+    n = torch.get_num_threads()
+    torch.set_num_threads(8)
+    yield
+    torch.set_num_threads(n)
+
+
 def load(golden_dir, name):
     return dict(np.load(os.path.join(golden_dir, name + ".npz")))
 
