@@ -651,7 +651,7 @@ __device__ __noinline__ double ode_error_part(const double *y, const double *yne
 }
 
 // Dense output of an accepted step (scipy rk.py:715-737, RkDenseOutput): y(te) = y_old + h * Q . [x, x^2, x^3, x^4],
-// Q = K^T . P, x = (te - t_old) / h, for the quads of one tile -> dst (rows of the whole batch).
+// Q = K^T . P, x = (te - t_old) / h, for the quads of one tile -> dst (the tile's first row).
 template <class EV>
 __device__ __noinline__ void ode_dense_point(const double *y, const double *k0, const double *k1, const double *k2,
                                              const double *k3, const double *k4, const double *k5, const double *k6,
@@ -675,7 +675,7 @@ __device__ __noinline__ void ode_dense_point(const double *y, const double *k0, 
 #pragma unroll
             for (int c = 0; c < 4; ++c) qc[c] += kv[j].v[e] * c_P[j][c];
         const double v = yv.v[e] + h * (((qc[0] * p1 + qc[1] * p2) + qc[2] * p3) + qc[3] * p4);
-        if (4 * q + e < nvalid) dst[g + e] = v;
+        if (4 * q + e < nvalid) dst[4 * q + e] = v;
     }
 }
 
@@ -911,9 +911,10 @@ __global__ void __launch_bounds__(EV::NT, 1) ode_rk45_kernel(OdeArgs a) {
                         for (int tile = tile0; tile < a.ntiles; tile += tile_step) {
                             if (EV::writer(ctx))
                                 ode_dense_point<EV>(ycur, K0, K1, K2, K3, K4, K5, K6, tile, N, h, xe,
-                                                    a.dense + (size_t)next_eval * N * 9);
+                                                    a.dense + ((size_t)next_eval * N + (size_t)tile * RT) * 9);
                             if (next_eval == a.n_eval - 1 && t_new == t_bound)
-                                ode_dense_point<EV>(ycur, K0, K1, K2, K3, K4, K5, K6, tile, N, h, xe, ynew);
+                                ode_dense_point<EV>(ycur, K0, K1, K2, K3, K4, K5, K6, tile, N, h, xe,
+                                                    ynew + (size_t)tile * RT * 9);
                         }
                         ++next_eval;
                     }
@@ -999,6 +1000,330 @@ __global__ void __launch_bounds__(EV::NT, 1) ode_rk45_kernel(OdeArgs a) {
     }
     EV::report(ctx, a.stats);
     EV::teardown(S, ctx);
+}
+
+// ------------------------------------------------------------------------------------------
+// Per-object step control: every object is integrated as if the sampler had been called with that object alone.
+// Object b (rows b*R .. b*R+R-1 of the caller's arrays) is integrated by one CTA (or one cluster) from start to end,
+// with its own t, h, error norm, accept / reject sequence and statistics; no grid barrier.  Its rows are split into
+// `nsub` consecutive tiles of EV::RT rows (one tile for the tensor-core evaluators, R <= 128; the FFMA evaluator
+// uses the tile height a one-object batch call would pick).  In the workspace the object owns nsub whole tiles
+// (padded tile b*nsub + j), so the batch kernel's per-tile device functions apply unchanged: they see a batch whose
+// rows end R rows into the object's first tile.  Norms are summed exactly as the batch kernel sums them for a batch
+// of nsub tiles (per-tile block_sum, then block_sum of the tile partials), so the result is bit-identical to a
+// batch call with that object alone on the same evaluator shape.
+// ------------------------------------------------------------------------------------------
+constexpr int OBJ_MAX_SUB = 16;   // 128 rows in tiles of at least 8 rows
+
+struct OdeObjArgs {
+    OdeArgs a;          // N = B * R, rpo = R; traj unused; y / K hold nobj * nsub padded tiles
+    int nobj, nsub;
+    double *obj_stats;  // [nobj][GP_STAT_COUNT]
+};
+
+template <class EV>
+__global__ void __launch_bounds__(EV::NT, 1) ode_rk45_obj_kernel(OdeObjArgs oa) {
+    constexpr int RT = EV::RT, NT = EV::NT, XS = EV::XS;
+    const OdeArgs &a = oa.a;
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    typename EV::Smem &S = EV::smem(smem_raw);
+    typename EV::Ctx ctx;
+    const int tid = threadIdx.x;
+    const float *P = a.P;
+    const int R = a.rpo, nsub = oa.nsub;
+    const double n_total = (double)R * 9.0;
+    EV::setup(S, ctx, P);
+    float *const tqtab = EV::tq(S);
+    float *const xin = EV::xin(S);
+    const float *const fo = EV::outp(S);
+    const double direction = (a.eps > a.T) ? 1.0 : ((a.eps < a.T) ? -1.0 : 1.0);
+    const double t_bound = a.eps;
+    const size_t roff = EV::replica_index(ctx) * a.replica;
+    __shared__ double s_coef[8];
+    __shared__ float s_std[8];
+    __shared__ double s_part[3][OBJ_MAX_SUB];   // per-tile partial sums of the current object
+    // grid_total() of the batch kernel over this object's tile partials (tid < nsub <= NT: one partial per thread)
+    auto total = [&](int k) {
+        __syncthreads();
+        const double v = tid < nsub ? 0.0 + s_part[k][tid] : 0.0;
+        return block_sum(v, S.red);
+    };
+
+    for (int b = EV::tile_first(); b < oa.nobj; b += EV::tile_step()) {
+        double *ycur = a.y[0] + roff, *ynew = a.y[1] + roff;
+        double *K0 = a.K[0] + roff, *K6 = a.K[6] + roff;
+        double *const K1 = a.K[1] + roff, *const K2 = a.K[2] + roff, *const K3 = a.K[3] + roff,
+                     *const K4 = a.K[4] + roff, *const K5 = a.K[5] + roff;
+        // tile j of the object is padded tile b*nsub + j; `Nv` is where the object's rows end in the padded numbering
+        const int Nv = b * nsub * RT + R;
+        auto set_obj = [&](int j) { EV::begin_tile(S, ctx, a.proj, b * R + j * RT, b * R + R, R); };
+        auto stage_eval = [&](int tile, double t_stage, double *Kd) {
+            const double g = diffusion_f64(t_stage);
+            EV::forward(P, a.proj, S, ctx, tqtab);
+            ode_store_k<EV>(fo, Kd, tile, Nv, sigma_f32((float)t_stage), 0.5 * (g * g));
+        };
+        double nfev = 0, n_acc = 0, n_rej = 0;
+        int next_eval = 0;
+        int status = 0;
+
+        // ---- f0 = fun(T, y0), d0, d1 (select_initial_step, common.py:68-134) ----
+        double t = a.T;
+        if (tid == 0) S.times[0] = (float)t;
+        __syncthreads();
+        EV::stage_tq(P, S, ctx, 1);
+        for (int j = 0; j < nsub; ++j) {
+            const int tile = b * nsub + j, r0 = tile * RT, c0 = b * R + j * RT;   // padded / caller's first row
+            set_obj(j);
+            for (int i = tid; i < RT * XS; i += NT) {
+                const int r = i / XS, c = i - XS * r;
+                float v = 0.f;
+                if (r0 + r < Nv && c < 9) {
+                    const double yv = a.x0[(size_t)(c0 + r) * 9 + c];
+                    ycur[(size_t)(r0 + r) * 9 + c] = yv;
+                    v = (float)yv;
+                }
+                xin[i] = v;
+            }
+            __syncthreads();
+            stage_eval(tile, t, K0);
+            double s0 = 0.0, s1 = 0.0;
+            for (int i = tid; i < RT * 9; i += NT) {
+                const int r = i / 9;
+                if (r0 + r < Nv) {
+                    const size_t g = (size_t)r0 * 9 + i;
+                    const double yv = ycur[g], fv = K0[g];
+                    const double sc = a.atol + fabs(yv) * a.rtol;
+                    s0 += (yv / sc) * (yv / sc);
+                    s1 += (fv / sc) * (fv / sc);
+                }
+            }
+            s0 = block_sum(s0, S.red);
+            s1 = block_sum(s1, S.red);
+            if (tid == 0) { s_part[0][j] = s0; s_part[1][j] = s1; }
+        }
+        nfev += 1;
+        const double d0 = sqrt(total(0) / n_total);
+        const double d1 = sqrt(total(1) / n_total);
+        const double interval = fabs(t_bound - a.T);
+        double h0 = (d0 < 1e-5 || d1 < 1e-5) ? 1e-6 : 0.01 * d0 / d1;
+        h0 = fmin(h0, interval);
+
+        // ---- f1 = fun(t0 + h0*dir, y0 + h0*dir*f0), d2 ----
+        {
+            const double t1 = t + h0 * direction;
+            if (tid == 0) S.times[0] = (float)t1;
+            __syncthreads();
+            EV::stage_tq(P, S, ctx, 1);
+            for (int j = 0; j < nsub; ++j) {
+                const int tile = b * nsub + j, r0 = tile * RT;
+                set_obj(j);
+                for (int i = tid; i < RT * XS; i += NT) {
+                    const int r = i / XS, c = i - XS * r;
+                    float v = 0.f;
+                    if (r0 + r < Nv && c < 9) {
+                        const size_t g = (size_t)(r0 + r) * 9 + c;
+                        v = (float)(ycur[g] + h0 * direction * K0[g]);
+                    }
+                    xin[i] = v;
+                }
+                __syncthreads();
+                stage_eval(tile, t1, K1);
+                double s2 = 0.0;
+                for (int i = tid; i < RT * 9; i += NT) {
+                    const int r = i / 9;
+                    if (r0 + r < Nv) {
+                        const size_t g = (size_t)r0 * 9 + i;
+                        const double sc = a.atol + fabs(ycur[g]) * a.rtol;
+                        const double d = (K1[g] - K0[g]) / sc;
+                        s2 += d * d;
+                    }
+                }
+                s2 = block_sum(s2, S.red);
+                if (tid == 0) s_part[2][j] = s2;
+            }
+            nfev += 1;
+        }
+        const double d2 = sqrt(total(2) / n_total) / h0;
+        double h1;
+        if (d1 <= 1e-15 && d2 <= 1e-15) h1 = fmax(1e-6, h0 * 1e-3);
+        else h1 = pow(0.01 / fmax(d1, d2), 1.0 / 5.0);
+        double h_abs = fmin(fmin(100.0 * h0, h1), interval);
+        const double h_initial = h_abs;
+        double h_last = 0.0;
+
+        // ---- main loop (ivp.py while status is None; rk.py _step_impl) ----
+        long attempts = 0;
+        while (direction * (t - t_bound) < 0.0 && status == 0) {
+            const double min_step = 10.0 * fabs(nextafter(t, direction * INFINITY) - t);
+            if (h_abs < min_step) h_abs = min_step;
+            bool step_rejected = false;
+            while (true) {
+                if (h_abs < min_step) { status = -1; break; }
+                if (++attempts > 100000) { status = -2; break; }
+                double h = h_abs * direction;
+                double t_new = t + h;
+                if (direction * (t_new - t_bound) > 0.0) t_new = t_bound;
+                h = t_new - t;
+                h_abs = fabs(h);
+
+                if (tid < 6) {
+                    const double ts = tid < 5 ? t + c_C[tid + 1] * h : t + h;
+                    S.times[tid] = (float)ts;
+                } else if (tid >= 32 && tid < 38) {
+                    const int sI = tid - 32;
+                    const double ts = sI < 5 ? t + c_C[sI + 1] * h : t + h;
+                    s_std[sI] = sigma_f32((float)ts);
+                } else if (tid >= 64 && tid < 70) {
+                    const int sI = tid - 64;
+                    const double ts = sI < 5 ? t + c_C[sI + 1] * h : t + h;
+                    const double g = diffusion_f64(ts);
+                    s_coef[sI] = 0.5 * (g * g);
+                }
+                __syncthreads();
+                EV::stage_tq(P, S, ctx, 6);
+
+                for (int j = 0; j < nsub; ++j) {
+                    const int tile = b * nsub + j;
+                    set_obj(j);
+                    auto fwd = [&](int slot) { EV::forward(P, a.proj, S, ctx, tqtab + slot * EV::TQW); };
+                    ode_stage_input<EV, 1>(ycur, ynew, K0, K1, K2, K3, K4, K5, xin, tile, Nv, h, fo, nullptr, 0.f, 0.0);
+                    fwd(0);
+                    ode_stage_input<EV, 2>(ycur, ynew, K0, K1, K2, K3, K4, K5, xin, tile, Nv, h, fo, K1, s_std[0], s_coef[0]);
+                    fwd(1);
+                    ode_stage_input<EV, 3>(ycur, ynew, K0, K1, K2, K3, K4, K5, xin, tile, Nv, h, fo, K2, s_std[1], s_coef[1]);
+                    fwd(2);
+                    ode_stage_input<EV, 4>(ycur, ynew, K0, K1, K2, K3, K4, K5, xin, tile, Nv, h, fo, K3, s_std[2], s_coef[2]);
+                    fwd(3);
+                    ode_stage_input<EV, 5>(ycur, ynew, K0, K1, K2, K3, K4, K5, xin, tile, Nv, h, fo, K4, s_std[3], s_coef[3]);
+                    fwd(4);
+                    ode_stage_input<EV, 6>(ycur, ynew, K0, K1, K2, K3, K4, K5, xin, tile, Nv, h, fo, K5, s_std[4], s_coef[4]);
+                    fwd(5);
+                    double se = ode_error_part<EV>(ycur, ynew, K0, K1, K2, K3, K4, K5, K6, tile, Nv, h, a.atol, a.rtol,
+                                                   nullptr, fo, s_std[5], s_coef[5]);
+                    se = block_sum(se, S.red);
+                    if (tid == 0) s_part[0][j] = se;
+                }
+                nfev += 6;
+                const double error_norm = sqrt(total(0) / n_total);
+                if (error_norm < 1.0) {
+                    double factor = (error_norm == 0.0) ? 10.0 : fmin(10.0, 0.9 * pow(error_norm, -0.2));
+                    if (step_rejected) factor = fmin(1.0, factor);
+                    h_abs *= factor;
+                    if (a.t_eval != nullptr) {
+                        while (next_eval < a.n_eval && direction * (a.t_eval[next_eval] - t_new) <= 0.0) {
+                            const double xe = (a.t_eval[next_eval] - t) / h;
+                            for (int j = 0; j < nsub; ++j) {
+                                const int tile = b * nsub + j;
+                                if (EV::writer(ctx))
+                                    ode_dense_point<EV>(ycur, K0, K1, K2, K3, K4, K5, K6, tile, Nv, h, xe,
+                                                        a.dense + ((size_t)next_eval * a.N + (size_t)b * R + (size_t)j * RT) * 9);
+                                if (next_eval == a.n_eval - 1 && t_new == t_bound)
+                                    ode_dense_point<EV>(ycur, K0, K1, K2, K3, K4, K5, K6, tile, Nv, h, xe,
+                                                        ynew + (size_t)tile * RT * 9);
+                            }
+                            ++next_eval;
+                        }
+                        __syncthreads();
+                    }
+                    double *ty = ycur; ycur = ynew; ynew = ty;
+                    double *tk = K0; K0 = K6; K6 = tk;
+                    t = t_new;
+                    h_last = h;
+                    n_acc += 1;
+                    break;
+                } else {
+                    const double f = 0.9 * pow(error_norm, -0.2);
+                    h_abs *= (f > 0.2) ? f : 0.2;
+                    step_rejected = true;
+                    n_rej += 1;
+                }
+            }
+        }
+
+        // ---- denoise (samplers.py:238-249), Gram-Schmidt and centre (:251-257) ----
+        const float eps_f = (float)a.eps;
+        if (a.denoise) {
+            if (tid == 0) S.times[0] = eps_f;
+            __syncthreads();
+            EV::stage_tq(P, S, ctx, 1);
+        }
+        for (int j = 0; j < nsub; ++j) {
+            const int r0 = (b * nsub + j) * RT, c0 = b * R + j * RT;
+            if (a.denoise) {
+                set_obj(j);
+                for (int i = tid; i < RT * XS; i += NT) {
+                    const int r = i / XS, c = i - XS * r;
+                    float v = 0.f;
+                    if (r0 + r < Nv && c < 9) v = (float)ycur[(size_t)(r0 + r) * 9 + c];
+                    xin[i] = v;
+                }
+                __syncthreads();
+                EV::forward(P, a.proj, S, ctx, tqtab);
+            }
+            for (int r = tid; r < RT; r += NT) {
+                if (r0 + r >= Nv) continue;
+                double v[9];
+#pragma unroll
+                for (int c = 0; c < 9; ++c) v[c] = ycur[(size_t)(r0 + r) * 9 + c];
+                if (a.denoise) {
+                    const float std = sigma_f32(eps_f);
+                    const float dif = diffusion_f32(eps_f);
+                    const float step = (float)((1.0 - a.eps) / a.denoise_steps);
+#pragma unroll
+                    for (int c = 0; c < 9; ++c) {
+                        const float grad = fo[r * XS + c] / (std + 1e-7f);
+                        const float drift = 0.f - (dif * dif) * grad;
+                        v[c] = v[c] + (double)(drift * step);
+                    }
+                }
+                gram_schmidt6<double>(v);
+#pragma unroll
+                for (int c = 0; c < 3; ++c) v[6 + c] += (double)a.center[(size_t)(c0 + r) * 3 + c];
+                if (status != 0) {   // this object failed: poison its rows only
+#pragma unroll
+                    for (int c = 0; c < 9; ++c) v[c] = __longlong_as_double(0x7ff8000000000000LL);
+                }
+#pragma unroll
+                for (int c = 0; c < 9; ++c) a.x_out[(size_t)(c0 + r) * 9 + c] = v[c];
+            }
+            __syncthreads();
+        }
+        if (EV::writer(ctx) && tid == 0) {
+            double *st = oa.obj_stats + (size_t)b * GP_STAT_COUNT;
+            st[GP_STAT_NFEV] = nfev;
+            st[GP_STAT_ACCEPTED] = n_acc;
+            st[GP_STAT_REJECTED] = n_rej;
+            st[GP_STAT_STATUS] = (double)status;
+            st[GP_STAT_T_FINAL] = t;
+            st[GP_STAT_H_INITIAL] = h_initial;
+            st[GP_STAT_H_LAST] = h_last;
+        }
+    }
+    EV::teardown(S, ctx);
+}
+
+// Summary of the per-object statistics: nfev = max, accepted / rejected = sums, status = the first non-zero one;
+// t_final / h_initial / h_last are those of the first failed object, else of object 0.
+__global__ void ode_obj_summary_kernel(const double *__restrict__ obj_stats, int nobj, double *__restrict__ stats) {
+    if (threadIdx.x != 0) return;
+    double nfev = 0, acc = 0, rej = 0;
+    int first = 0;
+    bool failed = false;
+    for (int b = 0; b < nobj; ++b) {
+        const double *st = obj_stats + (size_t)b * GP_STAT_COUNT;
+        nfev = fmax(nfev, st[GP_STAT_NFEV]);
+        acc += st[GP_STAT_ACCEPTED];
+        rej += st[GP_STAT_REJECTED];
+        if (!failed && st[GP_STAT_STATUS] != 0.0) { failed = true; first = b; }
+    }
+    const double *f = obj_stats + (size_t)first * GP_STAT_COUNT;
+    stats[GP_STAT_NFEV] = nfev;
+    stats[GP_STAT_ACCEPTED] = acc;
+    stats[GP_STAT_REJECTED] = rej;
+    stats[GP_STAT_STATUS] = f[GP_STAT_STATUS];
+    stats[GP_STAT_T_FINAL] = f[GP_STAT_T_FINAL];
+    stats[GP_STAT_H_INITIAL] = f[GP_STAT_H_INITIAL];
+    stats[GP_STAT_H_LAST] = f[GP_STAT_H_LAST];
 }
 
 // xs = normalise(traj) + centre, transposed to [N,S,9]            (samplers.py:251-255)
@@ -1196,6 +1521,19 @@ static int launch_ode(OdeArgs &a, cudaStream_t st) {
     return launch_tiles<EV>(ode_rk45_kernel<EV>, a.ntiles, true, a, st, "gp_scorenet_ode");
 }
 
+// One CTA (or cluster) per object, no grid barrier: an ordinary launch whose CTAs the hardware hands out as SMs free
+// up, which balances objects that finish at different step counts.
+template <class EV>
+static int launch_ode_obj(OdeObjArgs &oa, cudaStream_t st) {
+    oa.nsub = (oa.a.rpo + EV::RT - 1) / EV::RT;
+    if (oa.nsub * EV::RT > 128 || oa.nsub > OBJ_MAX_SUB) {
+        set_error("gp_scorenet_ode_objects: %d rows per object do not fit whole %d-row tiles in 128 rows", oa.a.rpo, EV::RT);
+        return GP_ERR_UNSUPPORTED;
+    }
+    oa.a.ntiles = oa.nobj * oa.nsub;
+    return launch_tiles<EV>(ode_rk45_obj_kernel<EV>, oa.nobj, false, oa, st, "gp_scorenet_ode_objects");
+}
+
 static size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
 
 // `mode` of the public entries: bits 0..1 = arithmetic (0 FFMA, 1 bf16, 2 split-bf16), GP_MODE_SOLO / GP_MODE_CLUSTER
@@ -1376,6 +1714,95 @@ extern "C" int gp_scorenet_ode_dense(const void *packed, const float *proj, cons
     GP_REQUIRE(t_eval && dense && n_eval >= 1, "gp_scorenet_ode_dense: t_eval / dense missing");
     return scorenet_ode_impl(packed, proj, x0, pts_center, N, rows_per_object, T, eps, rtol, atol, denoise, x_out, nullptr,
                              0, t_eval, n_eval, dense, stats, workspace, workspace_bytes, mode, s);
+}
+
+// Per-object step control.  Each object owns 128 padded rows of every state array (one 128-row tile, or whole
+// FFMA tiles of at most 128 rows), replicated per cluster rank like the batch workspace.
+static size_t ode_obj_state_bytes(int B) { return align256((size_t)B * 128 * 9 * sizeof(double)); }
+
+extern "C" size_t gp_scorenet_ode_objects_workspace_bytes(int B, int R) {
+    if (B < 1 || R < 1 || R > 128) return 0;
+    return ode_obj_state_bytes(B) * 9 * tc::CL + 256;
+}
+
+static int scorenet_ode_objects_impl(const void *packed, const float *proj, const double *x0, const float *pts_center,
+                                     int N, int rows_per_object, double T, double eps, double rtol, double atol,
+                                     int denoise, double *x_out, const double *t_eval, int n_eval, double *dense,
+                                     double *stats, double *obj_stats, void *workspace, size_t workspace_bytes,
+                                     int mode, gp_stream_t s) {
+    GP_REQUIRE(packed && proj && x0 && pts_center && x_out && stats && obj_stats && workspace,
+               "gp_scorenet_ode_objects: null pointer");
+    GP_REQUIRE(N >= 1 && rows_per_object >= 1 && N % rows_per_object == 0,
+               "gp_scorenet_ode_objects: bad sizes N=%d rows_per_object=%d (N must be B * rows_per_object)", N, rows_per_object);
+    if (rows_per_object > 128) {
+        set_error("gp_scorenet_ode_objects: rows_per_object=%d > 128 (an object must fit one 128-row tile)", rows_per_object);
+        return GP_ERR_UNSUPPORTED;
+    }
+    GP_REQUIRE(rtol > 0 && atol > 0, "gp_scorenet_ode_objects: tolerances must be positive");
+    GP_REQUIRE(mode_ok(mode), "gp_scorenet_ode_objects: mode must be 0 (fp32 FFMA), 1 (bf16 tcgen05) or 2 (split-bf16 x3 tcgen05) [| GP_MODE_SOLO / GP_MODE_CLUSTER / GP_MODE_SMEM_A]");
+    GP_REQUIRE((t_eval == nullptr) == (dense == nullptr) && (t_eval == nullptr || n_eval >= 1),
+               "gp_scorenet_ode_dense_objects: t_eval / dense / n_eval inconsistent");
+    const int B = N / rows_per_object;
+    if (workspace_bytes < gp_scorenet_ode_objects_workspace_bytes(B, rows_per_object)) {
+        set_error("gp_scorenet_ode_objects: workspace too small (%zu < %zu)", workspace_bytes,
+                  gp_scorenet_ode_objects_workspace_bytes(B, rows_per_object));
+        return GP_ERR_WORKSPACE;
+    }
+    if (rtol < 100 * 2.220446049250313e-16) rtol = 100 * 2.220446049250313e-16;
+    OdeObjArgs oa = {};
+    OdeArgs &a = oa.a;
+    a.P = (const float *)packed; a.proj = proj; a.x0 = x0; a.center = pts_center;
+    a.N = N; a.rpo = rows_per_object; a.T = T; a.eps = eps; a.rtol = rtol; a.atol = atol;
+    a.denoise = denoise; a.x_out = x_out; a.traj = nullptr; a.max_traj = 0; a.stats = stats;
+    a.t_eval = t_eval; a.n_eval = t_eval ? n_eval : 0; a.dense = dense;
+    a.denoise_steps = t_eval ? (double)n_eval : 1000.0;
+    unsigned char *w = (unsigned char *)(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
+    const size_t state = ode_obj_state_bytes(B);
+    a.y[0] = (double *)w; w += state;
+    a.y[1] = (double *)w; w += state;
+    for (int k = 0; k < 7; ++k) { a.K[k] = (double *)w; w += state; }
+    a.replica = 9 * state / sizeof(double);
+    a.part = nullptr; a.gbar = nullptr;
+    oa.nobj = B;
+    oa.obj_stats = obj_stats;
+    cudaStream_t st = as_stream(s);
+    // the evaluator shape follows the tile count B exactly as the batch rule follows its tile count
+    const int solo_shape = use_solo(mode, B * tc::RT);
+    mode &= 3;
+    int rc;
+    if (mode == 1) rc = solo_shape == 2 ? launch_ode_obj<TcSoloT<1>>(oa, st) : solo_shape ? launch_ode_obj<TcSolo<1>>(oa, st) : launch_ode_obj<TcEval<1>>(oa, st);
+    else if (mode == 2) rc = solo_shape == 2 ? launch_ode_obj<TcSoloT<3>>(oa, st) : solo_shape ? launch_ode_obj<TcSolo<3>>(oa, st) : launch_ode_obj<TcEval<3>>(oa, st);
+    else {
+        // the FFMA tile height of a batch call with this one object, so that the two agree bit for bit
+        switch (simt_rows_per_thread(rows_per_object, num_sms())) {
+            case 2: rc = launch_ode_obj<SimtEval<2>>(oa, st); break;
+            case 4: rc = launch_ode_obj<SimtEval<4>>(oa, st); break;
+            case 6: rc = launch_ode_obj<SimtEval<6>>(oa, st); break;
+            default: rc = launch_ode_obj<SimtEval<8>>(oa, st); break;
+        }
+    }
+    if (rc != GP_OK) return rc;
+    ode_obj_summary_kernel<<<1, 32, 0, st>>>(obj_stats, B, stats);
+    GP_CHECK_LAUNCH("gp_scorenet_ode_objects");
+    return GP_OK;
+}
+
+extern "C" int gp_scorenet_ode_objects(const void *packed, const float *proj, const double *x0, const float *pts_center,
+                                       int N, int rows_per_object, double T, double eps, double rtol, double atol,
+                                       int denoise, double *x_out, double *stats, double *obj_stats, void *workspace,
+                                       size_t workspace_bytes, int mode, gp_stream_t s) {
+    return scorenet_ode_objects_impl(packed, proj, x0, pts_center, N, rows_per_object, T, eps, rtol, atol, denoise,
+                                     x_out, nullptr, 0, nullptr, stats, obj_stats, workspace, workspace_bytes, mode, s);
+}
+
+extern "C" int gp_scorenet_ode_dense_objects(const void *packed, const float *proj, const double *x0,
+                                             const float *pts_center, int N, int rows_per_object, double T, double eps,
+                                             double rtol, double atol, int denoise, double *x_out, const double *t_eval,
+                                             int n_eval, double *dense, double *stats, double *obj_stats,
+                                             void *workspace, size_t workspace_bytes, int mode, gp_stream_t s) {
+    GP_REQUIRE(t_eval && dense && n_eval >= 1, "gp_scorenet_ode_dense_objects: t_eval / dense missing");
+    return scorenet_ode_objects_impl(packed, proj, x0, pts_center, N, rows_per_object, T, eps, rtol, atol, denoise,
+                                     x_out, t_eval, n_eval, dense, stats, obj_stats, workspace, workspace_bytes, mode, s);
 }
 
 extern "C" int gp_traj_finalize(const double *traj, const float *pts_center, int S, int N, double *xs, gp_stream_t s) {

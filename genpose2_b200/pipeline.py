@@ -49,14 +49,19 @@ def gather_results(pose, length, group=None):
 class PosePipeline:
     """score + energy + scale agents wired together; every stage runs on libgenpose_b200.so."""
 
-    def __init__(self, cfg=None, device="cuda", mlp_mode="fp32", use_graph=False):
+    def __init__(self, cfg=None, device="cuda", mlp_mode="fp32", use_graph=False, step_control="batch"):
         """use_graph: replay the whole step as ONE CUDA graph per input signature (batch size, points, hypotheses, T0):
         ~80 kernel launches, the two-stream fork / join and the cooperative sampler launch become one graph launch; the
         only host work left per step is drawing the prior noise with the CPU generator (exactly like the reference,
-        sde.py:34) and one pinned upload.  The captured graph bakes in the packed weights: load_state_dicts() drops it."""
+        sde.py:34) and one pinned upload.  The captured graph bakes in the packed weights: load_state_dicts() drops it.
+        step_control: "batch" (the reference's RK45 controller over the whole batch) or "object" (every object integrated
+        as if it were alone: its poses do not depend on the other objects of the step), see samplers.STEP_CONTROLS."""
+        from .samplers import check_step_control
+        check_step_control(step_control)
         cfg = copy.copy(cfg) if cfg is not None else get_config()
         cfg.device = device
         cfg.mlp_mode = mlp_mode
+        cfg.step_control = step_control
         if not getattr(cfg, "sampler_mode", None):
             cfg.sampler_mode = ["ode"]
         self.cfg = cfg
@@ -112,13 +117,17 @@ class PosePipeline:
             return self._graph_step(data, R, float(T0), init_x)
         return self._step(data, R, T0, init_x, return_all)
 
+    def _graph_key(self, pts, R, T0, init_x):
+        """One captured graph per input signature and sampler step control."""
+        return (pts.shape[0], pts.shape[1], R, T0, init_x is not None, pts.device.index, self.score_agent.cfg.step_control)
+
     def _graph_step(self, data, R, T0, init_x):
         """The step as a CUDA graph: copy the inputs into the graph's static buffers, draw + upload the prior noise,
         replay.  Returns clones of the two small results (the static ones are overwritten by the next replay)."""
         from . import samplers
         pts, center = data["pts"], data["pts_center"]
         B, N = pts.shape[0], pts.shape[1]
-        key = (B, N, R, T0, init_x is not None, pts.device.index)
+        key = self._graph_key(pts, R, T0, init_x)
         ent = self._graphs.get(key)
         net = self.score_agent.net
         real_prior = net.prior_fn
@@ -149,7 +158,7 @@ class PosePipeline:
                 with torch.cuda.graph(graph):
                     out = self._step(sdata, R, T0, st["init"], False)
                 self.graph_launches = _lib.launch_count() - n0   # kernels of this library inside one replay
-                stats = samplers.last_ode_stats.get("device_stats")
+                stats = {k: v for k, v in samplers.last_ode_stats.items() if k in ("device_stats", "device_obj_stats")}
             finally:
                 net.prior_fn = real_prior
             ent = self._graphs[key] = (graph, st, out, stats)
@@ -168,9 +177,9 @@ class PosePipeline:
         st["noise_event"] = torch.cuda.Event()
         st["noise_event"].record()
         graph.replay()
-        if stats is not None:
+        if stats:
             samplers.last_ode_stats.clear()
-            samplers.last_ode_stats["device_stats"] = stats
+            samplers.last_ode_stats.update(stats)
         return out[0].clone(), out[1].clone()
 
     def _step(self, data, R, T0, init_x, return_all):

@@ -53,14 +53,14 @@ class GFObjectPose(nn.Module):
             return cond_pc_sampler(
                 score_model=self, data=data, prior=self.prior_fn, sde_coeff=self.sde_fn,
                 num_steps=self.cfg.sampling_steps, snr=snr, device=self.device, eps=self.sampling_eps,
-                pose_mode=self.cfg.pose_mode, init_x=init_x)
+                pose_mode=self.cfg.pose_mode, init_x=init_x, step_control=getattr(self.cfg, "step_control", "batch"))
         if sampler == "ode":
             T0 = self.T if T0 is None else T0
             return cond_ode_sampler(
                 score_model=self, data=data, prior=self.prior_fn, sde_coeff=self.sde_fn, atol=atol, rtol=rtol,
                 device=self.device, eps=self.sampling_eps, T=T0, num_steps=self.cfg.sampling_steps,
                 pose_mode=self.cfg.pose_mode, denoise=denoise, init_x=init_x,
-                return_trajectory=return_trajectory)
+                return_trajectory=return_trajectory, step_control=getattr(self.cfg, "step_control", "batch"))
         raise NotImplementedError
 
     def forward(self, data, mode="score", init_x=None, T0=None, **kw):

@@ -28,6 +28,31 @@ def _traj_slots(batch_size):
 
 last_ode_stats = {}  # statistics of the most recent cond_ode_sampler call (nfev, accepted, ...)
 
+# RK45 step-size control of cond_ode_sampler (not in the reference):
+#   "batch"  one step size and one RMS error norm over the whole flattened batch, as scipy's solve_ivp on the
+#            reference's [N*9] state does (the default);
+#   "object" every object integrated as if the sampler had been called with that object alone, so that its poses
+#            depend only on its own features, noise and the weights (gp_scorenet_ode_objects).
+STEP_CONTROLS = ("batch", "object")
+MAX_ROWS_PER_OBJECT = 128   # "object": an object's hypotheses must fit one 128-row tile of the integrator
+
+
+def check_step_control(step_control, sampler="ode", rows_per_object=1, num_steps=None, return_trajectory=False):
+    """Raises for an unknown mode and for what "object" does not support, before any device work."""
+    if step_control not in STEP_CONTROLS:
+        raise ValueError(f"step_control must be one of {STEP_CONTROLS}, got {step_control!r}")
+    if step_control == "batch":
+        return
+    if sampler == "pc":
+        raise NotImplementedError("step_control='object' is implemented for the ODE sampler only")
+    if rows_per_object > MAX_ROWS_PER_OBJECT:
+        raise NotImplementedError(f"step_control='object' supports up to {MAX_ROWS_PER_OBJECT} hypotheses per object, "
+                                  f"got {rows_per_object}")
+    if return_trajectory and num_steps is None:
+        raise NotImplementedError("step_control='object' records no trajectory of accepted steps (objects accept "
+                                  "different numbers of steps): pass num_steps for dense output on a common grid, or "
+                                  "return_trajectory=False")
+
 # Failure of the device integrator (status -1: step size underflow, -2: attempt cap) must not pass silently, and
 # checking it must not stall the stream: every call copies its statistics to pinned host memory asynchronously; the
 # copies that have landed are inspected at the next sampler call / ode_stats() and a failed integration raises there.
@@ -104,22 +129,27 @@ def _to_device_async(t, device):
 
 def cond_ode_sampler(score_model, data, prior, sde_coeff, atol=1e-5, rtol=1e-5, device="cuda", eps=1e-5,
                      T=1.0, num_steps=None, pose_mode="quat_wxyz", denoise=True, init_x=None,
-                     return_trajectory=True):
+                     return_trajectory=True, *, step_control="batch"):
     """-> (xs [N, S, 9] f64, x [N, 9] f64).  num_steps=None: xs holds every accepted step (scipy's res.y);
     num_steps=n: scipy's dense output on t_eval = linspace(T, eps, n) (samplers.py:222-235).
-    `return_trajectory=False` (not in the reference) skips recording and returns xs = x[:, None]."""
+    `return_trajectory=False` (not in the reference) skips recording and returns xs = x[:, None].
+    `step_control` (not in the reference): "batch" or "object", see STEP_CONTROLS.  "object" needs
+    num_steps or return_trajectory=False, and at most MAX_ROWS_PER_OBJECT rows per object."""
     if pose_mode != "rot_matrix":
         raise NotImplementedError("accelerated sampler supports pose_mode='rot_matrix' only")
     net = _score_net(score_model)
-    check_pending()
     batch_size = data["pts"].shape[0]
+    feat, rpo = _object_features(data, batch_size)
+    check_step_control(step_control, "ode", rpo, num_steps, return_trajectory)
+    check_pending()
     noise = _to_device_async(prior((batch_size, POSE_DIM), T=T), device)  # CPU generator, like samplers.py:197-201
     x0 = noise if init_x is None else init_x + noise
     dev = x0.device
     x0 = x0.to(torch.float64).contiguous()  # scipy casts y0 to float64
-    feat, rpo = _object_features(data, batch_size)
     proj = net.project(feat.to(dev))
     center = _lib.check_cuda(data["pts_center"].to(torch.float32).contiguous(), "pts_center", torch.float32)
+    if step_control == "object":
+        return _ode_objects(net, score_model, proj, x0, center, batch_size, rpo, T, eps, rtol, atol, denoise, num_steps)
 
     x_out = torch.empty((batch_size, POSE_DIM), dtype=torch.float64, device=dev)
     stats = torch.zeros(_lib.GP_STAT_COUNT, dtype=torch.float64, device=dev)
@@ -164,12 +194,46 @@ def cond_ode_sampler(score_model, data, prior, sde_coeff, atol=1e-5, rtol=1e-5, 
     return xs, x_out
 
 
-def _record_stats(st):
+def _ode_objects(net, score_model, proj, x0, center, batch_size, rpo, T, eps, rtol, atol, denoise, num_steps):
+    """step_control="object": gp_scorenet_ode_objects / gp_scorenet_ode_dense_objects."""
+    dev = x0.device
+    B = batch_size // rpo
+    x_out = torch.empty((batch_size, POSE_DIM), dtype=torch.float64, device=dev)
+    stats = torch.zeros(_lib.GP_STAT_COUNT, dtype=torch.float64, device=dev)
+    obj_stats = torch.zeros((B, _lib.GP_STAT_COUNT), dtype=torch.float64, device=dev)
+    ws_bytes = _lib.load().gp_scorenet_ode_objects_workspace_bytes(B, rpo)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    args = (_lib.ptr(net.packed()), _lib.ptr(proj), _lib.ptr(x0), _lib.ptr(center), batch_size, rpo, float(T),
+            float(eps), float(rtol), float(atol), 1 if denoise else 0, _lib.ptr(x_out))
+    if num_steps is not None:
+        t_eval = torch.from_numpy(np.linspace(T, eps, int(num_steps))).to(dev)
+        dense = torch.empty((int(num_steps), batch_size, POSE_DIM), dtype=torch.float64, device=dev)
+        _lib.call("gp_scorenet_ode_dense_objects", *args, _lib.ptr(t_eval), int(num_steps), _lib.ptr(dense),
+                  _lib.ptr(stats), _lib.ptr(obj_stats), _lib.ptr(ws), ws_bytes, _mlp_mode(score_model), device=dev)
+        xs = torch.empty((batch_size, int(num_steps), POSE_DIM), dtype=torch.float64, device=dev)
+        _lib.call("gp_traj_finalize", _lib.ptr(dense), _lib.ptr(center), int(num_steps), batch_size, _lib.ptr(xs),
+                  device=dev)
+    else:
+        _lib.call("gp_scorenet_ode_objects", *args, _lib.ptr(stats), _lib.ptr(obj_stats), _lib.ptr(ws), ws_bytes,
+                  _mlp_mode(score_model), device=dev)
+        xs = x_out.unsqueeze(1)
+    last_ode_stats.clear()
+    last_ode_stats["device_stats"] = stats
+    last_ode_stats["device_obj_stats"] = obj_stats
+    _watch(stats)
+    return xs, x_out
+
+
+def _record_stats(st, obj=None):
     last_ode_stats.clear()
     last_ode_stats.update(
         nfev=int(st[_lib.STAT_NFEV]), accepted=int(st[_lib.STAT_ACCEPTED]), rejected=int(st[_lib.STAT_REJECTED]),
         status=int(st[_lib.STAT_STATUS]), t_final=float(st[_lib.STAT_T_FINAL]),
         h_initial=float(st[_lib.STAT_H_INITIAL]), h_last=float(st[_lib.STAT_H_LAST]))
+    if obj is not None:   # step_control="object": per-object arrays [B] beside the summary (nfev max, sums, first status)
+        for key, col in (("obj_nfev", _lib.STAT_NFEV), ("obj_accepted", _lib.STAT_ACCEPTED),
+                         ("obj_rejected", _lib.STAT_REJECTED), ("obj_status", _lib.STAT_STATUS)):
+            last_ode_stats[key] = obj[:, col].astype(np.int64)
     if last_ode_stats["status"] != 0:
         # the reference ignores solve_ivp's status (samplers.py:226-236); here a failed integration is an error
         raise RuntimeError(f"device RK45 integration failed with status {last_ode_stats['status']} "
@@ -180,18 +244,22 @@ def ode_stats():
     """Statistics of the last cond_ode_sampler call as a dict (synchronises if still on device)."""
     if "device_stats" in last_ode_stats:
         st = last_ode_stats["device_stats"].cpu()
+        obj = last_ode_stats.get("device_obj_stats")
+        obj = None if obj is None else obj.cpu().numpy()
         _pending_stats.clear()   # the call being read is the newest one; older ones were checked when it was issued
-        _record_stats(st)
+        _record_stats(st, obj)
     return dict(last_ode_stats)
 
 
 def cond_pc_sampler(score_model, data, prior, sde_coeff, num_steps=500, snr=0.16, device="cuda", eps=1e-5,
-                    pose_mode="quat_wxyz", init_x=None, noise=None):
+                    pose_mode="quat_wxyz", init_x=None, noise=None, *, step_control="batch"):
     """-> (xs [N, num_steps, 9] f32, mean_x [N, 9] f32).  `noise` (not in the reference):
     [num_steps, 2, N, 9] tensor replacing the per-step `torch.randn_like` draws; by default they are
-    drawn with torch on `device` in the reference's call order."""
+    drawn with torch on `device` in the reference's call order.  `step_control`: "batch" only (the
+    Langevin step size is one batch-wide reduction); "object" raises NotImplementedError."""
     if pose_mode != "rot_matrix":
         raise NotImplementedError("accelerated sampler supports pose_mode='rot_matrix' only")
+    check_step_control(step_control, "pc")
     net = _score_net(score_model)
     batch_size = data["pts"].shape[0]
     x0 = _to_device_async(prior((batch_size, POSE_DIM)), device) if init_x is None else init_x

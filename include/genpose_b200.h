@@ -309,6 +309,33 @@ GP_API int gp_scorenet_ode_dense(const void *packed, const float *proj, const do
                           int n_eval, double *dense, double *stats, void *workspace, size_t workspace_bytes,
                           int mode, gp_stream_t s);
 
+/* Per-object step control.  The entries above share one step size and one RMS error norm over the whole flattened
+ * batch (scipy's controller applied to all N*9 components), so an object's poses depend on which other objects share
+ * the call.  These entries integrate every object as if the sampler had been called with that object alone: its own
+ * select_initial_step, t, h, error norm over its R*9 components, accept / reject sequence, denoise step and
+ * statistics.  Object b (rows b*R .. b*R+R-1, R = rows_per_object, N = B*R) is integrated start to end by one CTA (or
+ * one 4-CTA cluster) on its own 128-row tile; the result is bit-identical to a gp_scorenet_ode call with that object
+ * alone on the same evaluator shape.  The tensor-core shape follows the tile count B by the batch rule (clusters for
+ * B <= 32, one CTA per object above); GP_MODE_SOLO / GP_MODE_CLUSTER force it.
+ *   rows_per_object  R <= 128 (GP_ERR_UNSUPPORTED above: an object spanning tiles is not supported)
+ *   stats       [GP_STAT_COUNT] f64 (device): summary -- nfev is the maximum over objects, accepted / rejected are
+ *               sums, status is the first non-zero one; t_final / h_initial / h_last are those of that object
+ *               (object 0 when none failed)
+ *   obj_stats   [B, GP_STAT_COUNT] f64 (device): the statistics of each object, fields as in gp_ode_stat
+ *   x_out       [N,9] f64; the rows of a failed object (status != 0) are NaN, the other objects are unaffected
+ * The trajectory of accepted steps is not offered (objects accept different numbers of steps); the dense-output
+ * variant takes a grid common to all objects.  The other arguments are those of gp_scorenet_ode / _dense. */
+GP_API size_t gp_scorenet_ode_objects_workspace_bytes(int B, int R);
+GP_API int gp_scorenet_ode_objects(const void *packed, const float *proj, const double *x0,
+                            const float *pts_center, int N, int rows_per_object, double T, double eps,
+                            double rtol, double atol, int denoise, double *x_out, double *stats, double *obj_stats,
+                            void *workspace, size_t workspace_bytes, int mode, gp_stream_t s);
+GP_API int gp_scorenet_ode_dense_objects(const void *packed, const float *proj, const double *x0,
+                                  const float *pts_center, int N, int rows_per_object, double T, double eps,
+                                  double rtol, double atol, int denoise, double *x_out, const double *t_eval,
+                                  int n_eval, double *dense, double *stats, double *obj_stats, void *workspace,
+                                  size_t workspace_bytes, int mode, gp_stream_t s);
+
 /* Post-processing of a recorded trajectory into the reference's `xs` (samplers.py:251-255):
  * traj [S,N,9] f64 raw -> xs [N,S,9] f64 with Gram-Schmidt on the rotation part and the centre
  * added. */
