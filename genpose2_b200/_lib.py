@@ -95,6 +95,10 @@ SIGNATURES = {
     "gp_scorenet_ode_dense_objects": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_double,
                                               c_double, c_double, c_double, c_int, c_void_p, c_void_p, c_int, c_void_p,
                                               c_void_p, c_void_p, c_void_p, c_size_t, c_int, c_void_p]),
+    "gp_scorenet_ode_objects_t0": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_double,
+                                           c_double, c_double, c_int, c_void_p, c_void_p, c_int, c_void_p, c_void_p,
+                                           c_void_p, c_void_p, c_size_t, c_int, c_void_p]),
+    "gp_object_noise": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "gp_traj_finalize": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "gp_scorenet_pc_workspace_bytes": (c_size_t, [c_int]),
     "gp_scorenet_pc": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,

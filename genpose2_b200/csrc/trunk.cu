@@ -1019,6 +1019,8 @@ struct OdeObjArgs {
     OdeArgs a;          // N = B * R, rpo = R; traj unused; y / K hold nobj * nsub padded tiles
     int nobj, nsub;
     double *obj_stats;  // [nobj][GP_STAT_COUNT]
+    const double *T_obj;    // [nobj] start time of each object (device), or nullptr: a.T for every object
+    size_t t_eval_stride;   // doubles between the dense-output grids of consecutive objects (0: one shared grid)
 };
 
 template <class EV>
@@ -1036,9 +1038,10 @@ __global__ void __launch_bounds__(EV::NT, 1) ode_rk45_obj_kernel(OdeObjArgs oa) 
     float *const tqtab = EV::tq(S);
     float *const xin = EV::xin(S);
     const float *const fo = EV::outp(S);
-    const double direction = (a.eps > a.T) ? 1.0 : ((a.eps < a.T) ? -1.0 : 1.0);
     const double t_bound = a.eps;
     const size_t roff = EV::replica_index(ctx) * a.replica;
+    __shared__ double s_T0;   // start time of the current object
+    auto direction_of = [&]() { const double T0 = s_T0; return (a.eps > T0) ? 1.0 : ((a.eps < T0) ? -1.0 : 1.0); };
     __shared__ double s_coef[8];
     __shared__ float s_std[8];
     __shared__ double s_part[3][OBJ_MAX_SUB];   // per-tile partial sums of the current object
@@ -1065,10 +1068,10 @@ __global__ void __launch_bounds__(EV::NT, 1) ode_rk45_obj_kernel(OdeObjArgs oa) 
         double nfev = 0, n_acc = 0, n_rej = 0;
         int next_eval = 0;
         int status = 0;
-
-        // ---- f0 = fun(T, y0), d0, d1 (select_initial_step, common.py:68-134) ----
-        double t = a.T;
-        if (tid == 0) S.times[0] = (float)t;
+        // The object's start time.  It is kept in shared memory and its direction is derived where it is used, rather
+        // than held in registers for the whole object: this kernel runs at its register cap.
+        double t = oa.T_obj != nullptr ? oa.T_obj[b] : a.T;
+        if (tid == 0) { S.times[0] = (float)t; s_T0 = t; }
         __syncthreads();
         EV::stage_tq(P, S, ctx, 1);
         for (int j = 0; j < nsub; ++j) {
@@ -1104,12 +1107,13 @@ __global__ void __launch_bounds__(EV::NT, 1) ode_rk45_obj_kernel(OdeObjArgs oa) 
         nfev += 1;
         const double d0 = sqrt(total(0) / n_total);
         const double d1 = sqrt(total(1) / n_total);
-        const double interval = fabs(t_bound - a.T);
+        const double interval = fabs(t_bound - s_T0);
         double h0 = (d0 < 1e-5 || d1 < 1e-5) ? 1e-6 : 0.01 * d0 / d1;
         h0 = fmin(h0, interval);
 
         // ---- f1 = fun(t0 + h0*dir, y0 + h0*dir*f0), d2 ----
         {
+            const double direction = direction_of();
             const double t1 = t + h0 * direction;
             if (tid == 0) S.times[0] = (float)t1;
             __syncthreads();
@@ -1153,7 +1157,8 @@ __global__ void __launch_bounds__(EV::NT, 1) ode_rk45_obj_kernel(OdeObjArgs oa) 
 
         // ---- main loop (ivp.py while status is None; rk.py _step_impl) ----
         long attempts = 0;
-        while (direction * (t - t_bound) < 0.0 && status == 0) {
+        while (direction_of() * (t - t_bound) < 0.0 && status == 0) {
+            const double direction = direction_of();
             const double min_step = 10.0 * fabs(nextafter(t, direction * INFINITY) - t);
             if (h_abs < min_step) h_abs = min_step;
             bool step_rejected = false;
@@ -1210,8 +1215,9 @@ __global__ void __launch_bounds__(EV::NT, 1) ode_rk45_obj_kernel(OdeObjArgs oa) 
                     if (step_rejected) factor = fmin(1.0, factor);
                     h_abs *= factor;
                     if (a.t_eval != nullptr) {
-                        while (next_eval < a.n_eval && direction * (a.t_eval[next_eval] - t_new) <= 0.0) {
-                            const double xe = (a.t_eval[next_eval] - t) / h;
+                        const double *const t_eval = a.t_eval + (size_t)b * oa.t_eval_stride;   // the object's grid
+                        while (next_eval < a.n_eval && direction * (t_eval[next_eval] - t_new) <= 0.0) {
+                            const double xe = (t_eval[next_eval] - t) / h;
                             for (int j = 0; j < nsub; ++j) {
                                 const int tile = b * nsub + j;
                                 if (EV::writer(ctx))
@@ -1725,11 +1731,13 @@ extern "C" size_t gp_scorenet_ode_objects_workspace_bytes(int B, int R) {
     return ode_obj_state_bytes(B) * 9 * tc::CL + 256;
 }
 
+// T_obj: [B] start times (device), or nullptr for T everywhere; with T_obj the dense-output grid is per object
+// ([B][n_eval]), without it one grid serves every object.
 static int scorenet_ode_objects_impl(const void *packed, const float *proj, const double *x0, const float *pts_center,
-                                     int N, int rows_per_object, double T, double eps, double rtol, double atol,
-                                     int denoise, double *x_out, const double *t_eval, int n_eval, double *dense,
-                                     double *stats, double *obj_stats, void *workspace, size_t workspace_bytes,
-                                     int mode, gp_stream_t s) {
+                                     int N, int rows_per_object, double T, const double *T_obj, double eps, double rtol,
+                                     double atol, int denoise, double *x_out, const double *t_eval, int n_eval,
+                                     double *dense, double *stats, double *obj_stats, void *workspace,
+                                     size_t workspace_bytes, int mode, gp_stream_t s) {
     GP_REQUIRE(packed && proj && x0 && pts_center && x_out && stats && obj_stats && workspace,
                "gp_scorenet_ode_objects: null pointer");
     GP_REQUIRE(N >= 1 && rows_per_object >= 1 && N % rows_per_object == 0,
@@ -1765,6 +1773,8 @@ static int scorenet_ode_objects_impl(const void *packed, const float *proj, cons
     a.part = nullptr; a.gbar = nullptr;
     oa.nobj = B;
     oa.obj_stats = obj_stats;
+    oa.T_obj = T_obj;
+    oa.t_eval_stride = (T_obj != nullptr && t_eval != nullptr) ? (size_t)n_eval : 0;
     cudaStream_t st = as_stream(s);
     // the evaluator shape follows the tile count B exactly as the batch rule follows its tile count
     const int solo_shape = use_solo(mode, B * tc::RT);
@@ -1791,8 +1801,9 @@ extern "C" int gp_scorenet_ode_objects(const void *packed, const float *proj, co
                                        int N, int rows_per_object, double T, double eps, double rtol, double atol,
                                        int denoise, double *x_out, double *stats, double *obj_stats, void *workspace,
                                        size_t workspace_bytes, int mode, gp_stream_t s) {
-    return scorenet_ode_objects_impl(packed, proj, x0, pts_center, N, rows_per_object, T, eps, rtol, atol, denoise,
-                                     x_out, nullptr, 0, nullptr, stats, obj_stats, workspace, workspace_bytes, mode, s);
+    return scorenet_ode_objects_impl(packed, proj, x0, pts_center, N, rows_per_object, T, nullptr, eps, rtol, atol,
+                                     denoise, x_out, nullptr, 0, nullptr, stats, obj_stats, workspace, workspace_bytes,
+                                     mode, s);
 }
 
 extern "C" int gp_scorenet_ode_dense_objects(const void *packed, const float *proj, const double *x0,
@@ -1801,8 +1812,24 @@ extern "C" int gp_scorenet_ode_dense_objects(const void *packed, const float *pr
                                              int n_eval, double *dense, double *stats, double *obj_stats,
                                              void *workspace, size_t workspace_bytes, int mode, gp_stream_t s) {
     GP_REQUIRE(t_eval && dense && n_eval >= 1, "gp_scorenet_ode_dense_objects: t_eval / dense missing");
-    return scorenet_ode_objects_impl(packed, proj, x0, pts_center, N, rows_per_object, T, eps, rtol, atol, denoise,
-                                     x_out, t_eval, n_eval, dense, stats, obj_stats, workspace, workspace_bytes, mode, s);
+    return scorenet_ode_objects_impl(packed, proj, x0, pts_center, N, rows_per_object, T, nullptr, eps, rtol, atol,
+                                     denoise, x_out, t_eval, n_eval, dense, stats, obj_stats, workspace, workspace_bytes,
+                                     mode, s);
+}
+
+// Per-object start times: T_obj[b] (device; the caller checks T_obj[b] > eps, this entry cannot read it).  t_eval is
+// optional and per object, [B][n_eval] in integration order (t_eval[b][0] = T_obj[b]); NULL (with dense NULL) means
+// no dense output.
+extern "C" int gp_scorenet_ode_objects_t0(const void *packed, const float *proj, const double *x0,
+                                          const float *pts_center, int N, int rows_per_object, const double *T_obj,
+                                          double eps, double rtol, double atol, int denoise, double *x_out,
+                                          const double *t_eval, int n_eval, double *dense, double *stats,
+                                          double *obj_stats, void *workspace, size_t workspace_bytes, int mode,
+                                          gp_stream_t s) {
+    GP_REQUIRE(T_obj, "gp_scorenet_ode_objects_t0: null pointer (T_obj)");
+    return scorenet_ode_objects_impl(packed, proj, x0, pts_center, N, rows_per_object, 0.0, T_obj, eps, rtol, atol,
+                                     denoise, x_out, t_eval, n_eval, dense, stats, obj_stats, workspace, workspace_bytes,
+                                     mode, s);
 }
 
 extern "C" int gp_traj_finalize(const double *traj, const float *pts_center, int S, int N, double *xs, gp_stream_t s) {

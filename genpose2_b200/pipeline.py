@@ -50,7 +50,8 @@ class PosePipeline:
     """score + energy + scale agents wired together; every stage runs on libgenpose_b200.so."""
 
     def __init__(self, cfg=None, device="cuda", mlp_mode="fp32", use_graph=False, step_control="batch"):
-        """use_graph: replay the whole step as ONE CUDA graph per input signature (batch size, points, hypotheses, T0):
+        """use_graph: replay the whole step as ONE CUDA graph per input signature (batch size, points, hypotheses, T0 --
+        or "per-object T0", whatever the values --, warm start and noise keys present or not):
         ~80 kernel launches, the two-stream fork / join and the cooperative sampler launch become one graph launch; the
         only host work left per step is drawing the prior noise with the CPU generator (exactly like the reference,
         sde.py:34) and one pinned upload.  The captured graph bakes in the packed weights: load_state_dicts() drops it.
@@ -108,26 +109,67 @@ class PosePipeline:
         return (feats[0] if len(feats) == 1 else torch.cat(feats, dim=0)), (geos if keep_geometry else None)
 
     @torch.no_grad()
-    def __call__(self, data, repeat_num=None, T0=None, init_x=None, return_all=False):
-        """data{'pts' [B,N,3] f32 cuda, 'pts_center' [B,3]} -> (aggregated_pose [B,4,4] f32, length [B,3] f32)."""
+    def __call__(self, data, repeat_num=None, T0=None, init_x=None, return_all=False, *, noise_keys=None):
+        """data{'pts' [B,N,3] f32 cuda, 'pts_center' [B,3]} -> (aggregated_pose [B,4,4] f32, length [B,3] f32).
+
+        T0: one start time for the step, or one per object (1-D host values; step_control="object" only), so that a
+        tracking frame of new objects (T0 = 0.55, no warm start) and tracked ones (T0 = 0.25 with their previous pose)
+        is one call.  init_x [B,9]: warm start added to the prior noise; a zero row means "no warm start" for that
+        object (0 + noise == noise).  noise_keys: int64 [B] (CPU or device), object b's prior noise drawn by
+        gp_object_noise from noise_keys[b] instead of the global CPU generator.  With step_control="object" and keys,
+        an object's aggregated pose and length depend only on its cloud, its key, its T0 and its warm start (for
+        results computed on the same evaluator shape, DESIGN.md section 6)."""
+        from . import samplers
         cfg = self.cfg
         R = cfg.eval_repeat_num if repeat_num is None else repeat_num
         T0 = cfg.T0 if T0 is None else T0
+        B = data["pts"].shape[0]
+        T_obj = samplers.object_start_times(T0, B, cfg.step_control, self.score_agent.sampling_eps)
+        noise_keys = samplers.check_noise_keys(noise_keys, B)
+        if T_obj is not None:
+            T0 = T_obj
         if self.use_graph and not return_all:
-            return self._graph_step(data, R, float(T0), init_x)
-        return self._step(data, R, T0, init_x, return_all)
+            return self._graph_step(data, R, float(T0) if T_obj is None else T0, init_x, noise_keys)
+        return self._step(data, R, T0, init_x, return_all, noise_keys)
 
-    def _graph_key(self, pts, R, T0, init_x):
-        """One captured graph per input signature and sampler step control."""
-        return (pts.shape[0], pts.shape[1], R, T0, init_x is not None, pts.device.index, self.score_agent.cfg.step_control)
+    def _graph_key(self, pts, R, T0, init_x, noise_keys=None):
+        """One captured graph per input signature and sampler step control.  Per-object start times and noise keys
+        live in static buffers refilled before every replay: the key records that they are used, not their values."""
+        per_object = isinstance(T0, (list, tuple)) or getattr(T0, "ndim", 0) > 0
+        return (pts.shape[0], pts.shape[1], R, "per-object" if per_object else T0, init_x is not None,
+                pts.device.index, noise_keys is not None, self.score_agent.cfg.step_control)
 
-    def _graph_step(self, data, R, T0, init_x):
-        """The step as a CUDA graph: copy the inputs into the graph's static buffers, draw + upload the prior noise,
-        replay.  Returns clones of the two small results (the static ones are overwritten by the next replay)."""
+    def _fill_object_inputs(self, st, T0, noise_keys, B):
+        """Per-object start times, grids, sigmas and keys -> the graph's static buffers (pinned staging, asynchronous
+        uploads).  Returns the host sigmas."""
+        from . import samplers
+        T_obj = T0 if "T" in st else None
+        sig = samplers.object_sigmas(T_obj, T0, B)
+        uploads = [("sigma", sig)]
+        if T_obj is not None:
+            uploads.append(("T", torch.from_numpy(T_obj)))
+            if "t_eval" in st:
+                grids = samplers.object_grids(T_obj, self.score_agent.sampling_eps, st["t_eval"].shape[1])
+                uploads.append(("t_eval", torch.from_numpy(grids)))
+        if noise_keys is not None:
+            if noise_keys.is_cuda:
+                st["keys"].copy_(noise_keys, non_blocking=True)
+            else:
+                uploads.append(("keys", noise_keys))
+        for name, host in uploads:
+            st[name + "_host"].copy_(host)
+            st[name].copy_(st[name + "_host"], non_blocking=True)
+        return sig
+
+    def _graph_step(self, data, R, T0, init_x, noise_keys=None):
+        """The step as a CUDA graph: copy the inputs into the graph's static buffers, draw + upload the prior noise
+        (or, with noise_keys, upload the keys: the noise is generated inside the graph), replay.  Returns clones of the
+        two small results (the static ones are overwritten by the next replay)."""
         from . import samplers
         pts, center = data["pts"], data["pts_center"]
         B, N = pts.shape[0], pts.shape[1]
-        key = self._graph_key(pts, R, T0, init_x)
+        key = self._graph_key(pts, R, T0, init_x, noise_keys)
+        per_object, keyed = key[3] == "per-object", noise_keys is not None
         ent = self._graphs.get(key)
         net = self.score_agent.net
         real_prior = net.prior_fn
@@ -137,6 +179,18 @@ class PosePipeline:
                       init=None if init_x is None else torch.empty_like(init_x),
                       noise=torch.empty((B * R, 9), dtype=torch.float32, device=dev),
                       noise_host=torch.empty((B * R, 9), dtype=torch.float32, pin_memory=True))
+            if per_object or keyed:
+                bufs = {"sigma": ((B,), torch.float32)}
+                if per_object:
+                    bufs["T"] = ((B,), torch.float64)
+                    if self.cfg.sampling_steps is not None:
+                        bufs["t_eval"] = ((B, int(self.cfg.sampling_steps)), torch.float64)
+                if keyed:
+                    bufs["keys"] = ((B,), torch.int64)
+                for name, (shape, dtype) in bufs.items():
+                    st[name] = torch.empty(shape, dtype=dtype, device=dev)
+                    st[name + "_host"] = torch.empty(shape, dtype=dtype, pin_memory=True)
+                self._fill_object_inputs(st, T0, noise_keys, B)   # no draw: the global generator is not touched
             st["pts"].copy_(pts); st["center"].copy_(center)
             if init_x is not None:
                 st["init"].copy_(init_x)
@@ -145,22 +199,25 @@ class PosePipeline:
             st["noise"].copy_(torch.randn((B * R, 9), generator=torch.Generator().manual_seed(0)))
             sdata = {"pts": st["pts"], "pts_center": st["center"]}
             net.prior_fn = lambda shape, T=1.0: st["noise"]    # device tensor: no host work inside the capture
+            if per_object or keyed:   # the sampler takes T, sigma, keys and the noise from the static buffers
+                net.static_object_inputs = {k: st.get(k) for k in ("noise", "sigma", "T", "t_eval", "keys")}
             try:
                 warm = torch.cuda.Stream(device=dev)
                 warm.wait_stream(torch.cuda.current_stream(dev))
                 with torch.cuda.stream(warm):
                     for _ in range(2):   # packs weights, sets kernel attributes, sizes the allocator pools
-                        self._step(sdata, R, T0, st["init"], False)
+                        self._step(sdata, R, T0, st["init"], False, st.get("keys"))
                 torch.cuda.current_stream(dev).wait_stream(warm)
                 torch.cuda.synchronize(dev)
                 graph = torch.cuda.CUDAGraph()
                 n0 = _lib.launch_count()
                 with torch.cuda.graph(graph):
-                    out = self._step(sdata, R, T0, st["init"], False)
+                    out = self._step(sdata, R, T0, st["init"], False, st.get("keys"))
                 self.graph_launches = _lib.launch_count() - n0   # kernels of this library inside one replay
                 stats = {k: v for k, v in samplers.last_ode_stats.items() if k in ("device_stats", "device_obj_stats")}
             finally:
                 net.prior_fn = real_prior
+                net.static_object_inputs = None
             ent = self._graphs[key] = (graph, st, out, stats)
         graph, st, out, stats = ent
         if pts.data_ptr() != st["pts"].data_ptr():
@@ -168,12 +225,15 @@ class PosePipeline:
         st["center"].copy_(center, non_blocking=True)
         if init_x is not None:
             st["init"].copy_(init_x, non_blocking=True)
-        # prior noise: drawn on the CPU from the global generator in the reference's call order (samplers.py:197-201)
         ev = st.get("noise_event")
         if ev is not None:
-            ev.synchronize()     # the previous upload out of the pinned buffer (long finished in practice)
-        st["noise_host"].copy_(real_prior((B * R, 9), T=T0))
-        st["noise"].copy_(st["noise_host"], non_blocking=True)
+            ev.synchronize()     # the previous uploads out of the pinned buffers (long finished in practice)
+        sig = self._fill_object_inputs(st, T0, noise_keys, B) if (per_object or keyed) else None
+        if not keyed:
+            # prior noise: drawn on the CPU from the global generator in the reference's call order (samplers.py:197-201)
+            st["noise_host"].copy_(real_prior((B * R, 9), T=T0) if not per_object
+                                   else samplers.object_prior_noise(sig, R))
+            st["noise"].copy_(st["noise_host"], non_blocking=True)
         st["noise_event"] = torch.cuda.Event()
         st["noise_event"].record()
         graph.replay()
@@ -182,7 +242,7 @@ class PosePipeline:
             samplers.last_ode_stats.update(stats)
         return out[0].clone(), out[1].clone()
 
-    def _step(self, data, R, T0, init_x, return_all):
+    def _step(self, data, R, T0, init_x, return_all, noise_keys=None):
         cfg = self.cfg
         capturing = torch.cuda.is_current_stream_capturing()
         # The sampler of a small batch is a cooperative launch of at most 33 four-CTA clusters (100 SMs at 64 x 50): the
@@ -193,7 +253,7 @@ class PosePipeline:
         fork = torch.cuda.Event()
         fork.record(main)
         pred_pose, pred_q = self.score_agent.pred_func(
-            data=data, repeat_num=R, T0=T0, init_x=init_x, save_path=None, pts_feat=score_feat)
+            data=data, repeat_num=R, T0=T0, init_x=init_x, save_path=None, pts_feat=score_feat, noise_keys=noise_keys)
         if self._side is None:
             self._side = torch.cuda.Stream(device=score_feat.device)
         self._side.wait_event(fork)

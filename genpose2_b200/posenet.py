@@ -47,20 +47,23 @@ class GFObjectPose(nn.Module):
         return self.pts_encoder(data["pts"], geometry=geometry, return_geometry=return_geometry)
 
     def sample(self, data, sampler, atol=1e-5, rtol=1e-5, snr=0.16, denoise=True, init_x=None, T0=None,
-               return_trajectory=True):
-        """posenet.py:230-276."""
+               return_trajectory=True, *, noise_keys=None):
+        """posenet.py:230-276.  T0 may be one start time per object and `noise_keys` (not in the reference) int64 [B]
+        keys of per-object noise, see samplers.cond_ode_sampler."""
         if sampler == "pc":
             return cond_pc_sampler(
                 score_model=self, data=data, prior=self.prior_fn, sde_coeff=self.sde_fn,
                 num_steps=self.cfg.sampling_steps, snr=snr, device=self.device, eps=self.sampling_eps,
-                pose_mode=self.cfg.pose_mode, init_x=init_x, step_control=getattr(self.cfg, "step_control", "batch"))
+                pose_mode=self.cfg.pose_mode, init_x=init_x, step_control=getattr(self.cfg, "step_control", "batch"),
+                noise_keys=noise_keys)
         if sampler == "ode":
             T0 = self.T if T0 is None else T0
             return cond_ode_sampler(
                 score_model=self, data=data, prior=self.prior_fn, sde_coeff=self.sde_fn, atol=atol, rtol=rtol,
                 device=self.device, eps=self.sampling_eps, T=T0, num_steps=self.cfg.sampling_steps,
                 pose_mode=self.cfg.pose_mode, denoise=denoise, init_x=init_x,
-                return_trajectory=return_trajectory, step_control=getattr(self.cfg, "step_control", "batch"))
+                return_trajectory=return_trajectory, step_control=getattr(self.cfg, "step_control", "batch"),
+                noise_keys=noise_keys)
         raise NotImplementedError
 
     def forward(self, data, mode="score", init_x=None, T0=None, **kw):
@@ -76,7 +79,7 @@ class GFObjectPose(nn.Module):
         if mode == "rgb_feature":
             return None  # cfg.dino != "global" (posenet.py:313-315)
         if mode == "pc_sample":
-            return self.sample(data, "pc", init_x=init_x)
+            return self.sample(data, "pc", init_x=init_x, noise_keys=kw.get("noise_keys"))
         if mode == "ode_sample":
             return self.sample(data, "ode", init_x=init_x, T0=T0, **kw)
         raise NotImplementedError

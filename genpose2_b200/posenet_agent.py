@@ -55,7 +55,9 @@ class PoseNet(nn.Module):
     # ------------------------------------------------------------------------------------------
     def pred_func(self, data, repeat_num, save_path="./visualization_results", return_average_res=False,
                   init_x: torch.Tensor = None, T0=None, return_process=False, geometry=None,
-                  return_geometry=False, pts_feat=None, want_quat=True):
+                  return_geometry=False, pts_feat=None, want_quat=True, *, noise_keys=None):
+        """T0: a scalar, or one start time per object (step_control="object"); noise_keys (not in the reference):
+        int64 [bs] keys of per-object noise.  See samplers.cond_ode_sampler."""
         self.is_testing = True
         if self.net.training:   # eval() walks every sub-module: only when the flag actually has to change
             self.net.eval()
@@ -84,6 +86,8 @@ class PoseNet(nn.Module):
                                else init_x.unsqueeze(1).repeat(1, repeat_num, 1).view(N, -1))
             mode = f"{self.cfg.sampler_mode[0]}_sample"
             kw = {"return_trajectory": bool(return_process)} if mode == "ode_sample" else {}
+            if noise_keys is not None:
+                kw["noise_keys"] = noise_keys
             in_process_sample, res = self.net(sampler_data, mode=mode, init_x=repeated_init_x, T0=T0, **kw)
             pred_pose = res.reshape(bs, repeat_num, -1)
             in_process_sample = in_process_sample.reshape(bs, repeat_num, in_process_sample.shape[1], -1)

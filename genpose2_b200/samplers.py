@@ -14,6 +14,7 @@ import torch
 
 from . import _lib
 from .scorenet import _object_features
+from .sde import prior_std
 
 POSE_DIM = 9  # get_pose_dim("rot_matrix"), utils/genpose_utils.py:34-35
 MAX_TRAJ = 512  # accepted-step slots recorded when the trajectory is requested (upper bound)
@@ -52,6 +53,87 @@ def check_step_control(step_control, sampler="ode", rows_per_object=1, num_steps
         raise NotImplementedError("step_control='object' records no trajectory of accepted steps (objects accept "
                                   "different numbers of steps): pass num_steps for dense output on a common grid, or "
                                   "return_trajectory=False")
+
+
+def object_start_times(T, num_objects, step_control, eps):
+    """Per-object start times of the ODE sampler.  A scalar T (a number, or a 0-d array / tensor) -> None: one start
+    time for the call, as before.  A 1-D host sequence, ndarray or CPU tensor of `num_objects` values -> float64
+    ndarray [B] (a float32 tensor's values are read as they are stored).  Raises, before any sampler work, for:
+    a CUDA tensor (reading it would hide a device synchronisation), step_control other than "object" (the batch
+    controller has one t for the whole batch), the wrong length, and a value that is not finite or not > eps."""
+    if isinstance(T, torch.Tensor):
+        if T.dim() == 0:
+            return None
+        if T.is_cuda:
+            raise TypeError("a per-object T must be a host sequence, ndarray or CPU tensor: reading a CUDA tensor "
+                            "would synchronise the device")
+        vals = T.detach().to(torch.float64).numpy()
+    elif isinstance(T, np.ndarray):
+        if T.ndim == 0:
+            return None
+        vals = T.astype(np.float64)
+    elif isinstance(T, (list, tuple)):
+        vals = np.asarray(T, dtype=np.float64)
+    else:
+        return None
+    if vals.ndim != 1:
+        raise ValueError(f"a per-object T must be 1-D, got shape {tuple(vals.shape)}")
+    if step_control != "object":
+        raise NotImplementedError("a per-object T needs step_control='object' (the batch controller integrates the "
+                                  "whole batch from one start time)")
+    if vals.shape[0] != num_objects:
+        raise ValueError(f"a per-object T needs one value per object: {num_objects} objects, got {vals.shape[0]} values")
+    if not np.isfinite(vals).all() or (vals <= eps).any():
+        raise ValueError(f"every per-object T must be finite and > eps={eps}, got {vals.tolist()}")
+    return np.ascontiguousarray(vals)
+
+
+def check_noise_keys(noise_keys, num_objects):
+    """noise_keys: int64 [B] (CPU or CUDA tensor, or ndarray) -> tensor; None -> None.  Raises for another dtype or
+    shape."""
+    if noise_keys is None:
+        return None
+    if isinstance(noise_keys, np.ndarray):
+        noise_keys = torch.from_numpy(noise_keys)
+    if not isinstance(noise_keys, torch.Tensor):
+        raise TypeError(f"noise_keys must be an int64 tensor of shape [{num_objects}], got {type(noise_keys).__name__}")
+    if noise_keys.dtype != torch.int64:
+        raise TypeError(f"noise_keys must be int64, got {noise_keys.dtype}")
+    if tuple(noise_keys.shape) != (num_objects,):
+        raise ValueError(f"noise_keys must have shape [{num_objects}] (one key per object), got {tuple(noise_keys.shape)}")
+    return noise_keys
+
+
+def object_sigmas(T_obj, T, num_objects):
+    """float32 [B] standard deviation of each object's prior noise: float32(sigma(T_b)), sigma as ve_marginal_prob
+    computes it (the factor ve_prior applies to its float32 normals)."""
+    times = T_obj if T_obj is not None else [float(T)] * num_objects
+    return torch.tensor([prior_std(float(t)) for t in times], dtype=torch.float32)
+
+
+def object_prior_noise(sigmas, rows_per_object):
+    """Unkeyed per-object prior: the draw ve_prior makes (torch.randn((N, 9)) from the global CPU generator), with the
+    rows of object b scaled by sigmas[b] in float32.  A vector of equal sigmas gives ve_prior's result bit for bit."""
+    z = torch.randn((sigmas.shape[0] * rows_per_object, POSE_DIM))
+    return z * sigmas.repeat_interleave(rows_per_object).unsqueeze(1)
+
+
+def object_grids(T_obj, eps, num_steps):
+    """Dense-output grids of per-object start times: float64 [B, num_steps], row b = linspace(T_obj[b], eps)."""
+    return np.stack([np.linspace(t, eps, int(num_steps)) for t in T_obj])
+
+
+def keyed_noise(keys, sigmas, rows_per_object, out=None):
+    """gp_object_noise: [B*R, 9] float32 noise on the keys' device, object b's block a function of keys[b] and
+    sigmas[b] only (both device tensors)."""
+    B = keys.shape[0]
+    keys = _lib.check_cuda(keys.contiguous(), "noise_keys", torch.int64)
+    sigmas = _lib.check_cuda(sigmas.contiguous(), "sigmas", torch.float32)
+    if out is None:
+        out = torch.empty((B * rows_per_object, POSE_DIM), dtype=torch.float32, device=keys.device)
+    _lib.call("gp_object_noise", _lib.ptr(keys), _lib.ptr(sigmas), B, rows_per_object, _lib.ptr(out), device=out.device)
+    return out
+
 
 # Failure of the device integrator (status -1: step size underflow, -2: attempt cap) must not pass silently, and
 # checking it must not stall the stream: every call copies its statistics to pinned host memory asynchronously; the
@@ -129,25 +211,57 @@ def _to_device_async(t, device):
 
 def cond_ode_sampler(score_model, data, prior, sde_coeff, atol=1e-5, rtol=1e-5, device="cuda", eps=1e-5,
                      T=1.0, num_steps=None, pose_mode="quat_wxyz", denoise=True, init_x=None,
-                     return_trajectory=True, *, step_control="batch"):
+                     return_trajectory=True, *, step_control="batch", noise_keys=None):
     """-> (xs [N, S, 9] f64, x [N, 9] f64).  num_steps=None: xs holds every accepted step (scipy's res.y);
     num_steps=n: scipy's dense output on t_eval = linspace(T, eps, n) (samplers.py:222-235).
     `return_trajectory=False` (not in the reference) skips recording and returns xs = x[:, None].
     `step_control` (not in the reference): "batch" or "object", see STEP_CONTROLS.  "object" needs
-    num_steps or return_trajectory=False, and at most MAX_ROWS_PER_OBJECT rows per object."""
+    num_steps or return_trajectory=False, and at most MAX_ROWS_PER_OBJECT rows per object.
+    Not in the reference either:
+      T           may be one start time per object (1-D host values, B = N / R; step_control="object" only, see
+                  object_start_times): object b is integrated from T[b], its prior noise is scaled by sigma(T[b]) and
+                  its dense grid is linspace(T[b], eps, num_steps).  Without keys the noise is object_prior_noise
+                  (the `prior` callable is not used).
+      noise_keys  int64 [B] (CPU or device): the prior draw is replaced by gp_object_noise, so that object b's noise
+                  depends on noise_keys[b] and its T only; the global CPU generator is not touched."""
     if pose_mode != "rot_matrix":
         raise NotImplementedError("accelerated sampler supports pose_mode='rot_matrix' only")
     net = _score_net(score_model)
     batch_size = data["pts"].shape[0]
     feat, rpo = _object_features(data, batch_size)
     check_step_control(step_control, "ode", rpo, num_steps, return_trajectory)
+    B = batch_size // rpo
+    T_obj = object_start_times(T, B, step_control, eps)
+    keys = check_noise_keys(noise_keys, B)
     check_pending()
-    noise = _to_device_async(prior((batch_size, POSE_DIM), T=T), device)  # CPU generator, like samplers.py:197-201
+    # PosePipeline's graph capture hands in device buffers it refills before every replay
+    static = getattr(score_model, "static_object_inputs", None)
+    if keys is None and T_obj is None:
+        noise = _to_device_async(prior((batch_size, POSE_DIM), T=T), device)  # CPU generator, like samplers.py:197-201
+    elif static is not None:
+        noise = static["noise"]
+        if keys is not None:
+            keyed_noise(static["keys"], static["sigma"], rpo, out=noise)
+    else:
+        sig = object_sigmas(T_obj, T, B)
+        if keys is not None:
+            kdev = keys.to(device) if keys.is_cuda else _to_device_async(keys, device)
+            noise = keyed_noise(kdev, _to_device_async(sig, kdev.device), rpo)
+        else:
+            noise = _to_device_async(object_prior_noise(sig, rpo), device)
     x0 = noise if init_x is None else init_x + noise
     dev = x0.device
     x0 = x0.to(torch.float64).contiguous()  # scipy casts y0 to float64
     proj = net.project(feat.to(dev))
     center = _lib.check_cuda(data["pts_center"].to(torch.float32).contiguous(), "pts_center", torch.float32)
+    if T_obj is not None:
+        if static is not None:
+            T_dev, grids = static["T"], static.get("t_eval")
+        else:
+            T_dev = _to_device_async(torch.from_numpy(T_obj), dev)
+            grids = None if num_steps is None else _to_device_async(torch.from_numpy(object_grids(T_obj, eps, num_steps)), dev)
+        return _ode_objects(net, score_model, proj, x0, center, batch_size, rpo, T, eps, rtol, atol, denoise, num_steps,
+                            T_obj=T_dev, t_eval=grids)
     if step_control == "object":
         return _ode_objects(net, score_model, proj, x0, center, batch_size, rpo, T, eps, rtol, atol, denoise, num_steps)
 
@@ -194,8 +308,10 @@ def cond_ode_sampler(score_model, data, prior, sde_coeff, atol=1e-5, rtol=1e-5, 
     return xs, x_out
 
 
-def _ode_objects(net, score_model, proj, x0, center, batch_size, rpo, T, eps, rtol, atol, denoise, num_steps):
-    """step_control="object": gp_scorenet_ode_objects / gp_scorenet_ode_dense_objects."""
+def _ode_objects(net, score_model, proj, x0, center, batch_size, rpo, T, eps, rtol, atol, denoise, num_steps,
+                 T_obj=None, t_eval=None):
+    """step_control="object": gp_scorenet_ode_objects / gp_scorenet_ode_dense_objects; with per-object start times
+    (T_obj [B] f64 device, t_eval [B, num_steps] f64 device or None) gp_scorenet_ode_objects_t0."""
     dev = x0.device
     B = batch_size // rpo
     x_out = torch.empty((batch_size, POSE_DIM), dtype=torch.float64, device=dev)
@@ -203,6 +319,23 @@ def _ode_objects(net, score_model, proj, x0, center, batch_size, rpo, T, eps, rt
     obj_stats = torch.zeros((B, _lib.GP_STAT_COUNT), dtype=torch.float64, device=dev)
     ws_bytes = _lib.load().gp_scorenet_ode_objects_workspace_bytes(B, rpo)
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    if T_obj is not None:
+        n_eval = 0 if num_steps is None else int(num_steps)
+        dense = None if num_steps is None else torch.empty((n_eval, batch_size, POSE_DIM), dtype=torch.float64, device=dev)
+        _lib.call("gp_scorenet_ode_objects_t0", _lib.ptr(net.packed()), _lib.ptr(proj), _lib.ptr(x0), _lib.ptr(center),
+                  batch_size, rpo, _lib.ptr(T_obj), float(eps), float(rtol), float(atol), 1 if denoise else 0,
+                  _lib.ptr(x_out), _lib.ptr(t_eval if dense is not None else None), n_eval, _lib.ptr(dense),
+                  _lib.ptr(stats), _lib.ptr(obj_stats), _lib.ptr(ws), ws_bytes, _mlp_mode(score_model), device=dev)
+        if dense is not None:
+            xs = torch.empty((batch_size, n_eval, POSE_DIM), dtype=torch.float64, device=dev)
+            _lib.call("gp_traj_finalize", _lib.ptr(dense), _lib.ptr(center), n_eval, batch_size, _lib.ptr(xs), device=dev)
+        else:
+            xs = x_out.unsqueeze(1)
+        last_ode_stats.clear()
+        last_ode_stats["device_stats"] = stats
+        last_ode_stats["device_obj_stats"] = obj_stats
+        _watch(stats)
+        return xs, x_out
     args = (_lib.ptr(net.packed()), _lib.ptr(proj), _lib.ptr(x0), _lib.ptr(center), batch_size, rpo, float(T),
             float(eps), float(rtol), float(atol), 1 if denoise else 0, _lib.ptr(x_out))
     if num_steps is not None:
@@ -252,13 +385,16 @@ def ode_stats():
 
 
 def cond_pc_sampler(score_model, data, prior, sde_coeff, num_steps=500, snr=0.16, device="cuda", eps=1e-5,
-                    pose_mode="quat_wxyz", init_x=None, noise=None, *, step_control="batch"):
+                    pose_mode="quat_wxyz", init_x=None, noise=None, *, step_control="batch", noise_keys=None):
     """-> (xs [N, num_steps, 9] f32, mean_x [N, 9] f32).  `noise` (not in the reference):
     [num_steps, 2, N, 9] tensor replacing the per-step `torch.randn_like` draws; by default they are
     drawn with torch on `device` in the reference's call order.  `step_control`: "batch" only (the
-    Langevin step size is one batch-wide reduction); "object" raises NotImplementedError."""
+    Langevin step size is one batch-wide reduction); "object" raises NotImplementedError.  `noise_keys`: keyed
+    per-object noise is offered by the ODE sampler only; anything but None raises NotImplementedError."""
     if pose_mode != "rot_matrix":
         raise NotImplementedError("accelerated sampler supports pose_mode='rot_matrix' only")
+    if noise_keys is not None:
+        raise NotImplementedError("noise_keys (keyed per-object noise) is implemented for the ODE sampler only")
     check_step_control(step_control, "pc")
     net = _score_net(score_model)
     batch_size = data["pts"].shape[0]

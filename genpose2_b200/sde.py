@@ -35,6 +35,11 @@ def ve_prior(shape, sigma_min=0.01, sigma_max=90, T=1.0):
     return torch.randn(*shape) * sigma_max_prior
 
 
+def prior_std(T):
+    """sigma(T) of the prior that init_sde's prior_fn draws from, as a Python float (ve_marginal_prob)."""
+    return ve_marginal_prob(None, T, sigma_min=SIGMA_MIN, sigma_max=SIGMA_MAX)[1]
+
+
 def init_sde(sde_mode):
     if sde_mode != "ve":
         raise NotImplementedError(

@@ -335,6 +335,29 @@ GP_API int gp_scorenet_ode_dense_objects(const void *packed, const float *proj, 
                                   double rtol, double atol, int denoise, double *x_out, const double *t_eval,
                                   int n_eval, double *dense, double *stats, double *obj_stats, void *workspace,
                                   size_t workspace_bytes, int mode, gp_stream_t s);
+/* Per-object start time: the arguments of gp_scorenet_ode_dense_objects, except that
+ *   T_obj   [B] f64 (device) replaces T: object b is integrated from T_obj[b] to eps.  The caller must ensure
+ *           T_obj[b] > eps (this entry cannot read device memory); NULL is rejected.
+ *   t_eval  optional, per object: [B, n_eval] f64 (device), row b in integration order (t_eval[b][0] = T_obj[b]);
+ *           NULL (with dense NULL) means no dense output.  dense is [n_eval, N, 9] as in the entries above.
+ * The denoise step is (1 - eps) / n_eval with dense output, (1 - eps) / 1000 without.  Workspace:
+ * gp_scorenet_ode_objects_workspace_bytes(B, R).  The entries above are this one with T_obj[b] = T for every object
+ * (bit for bit). */
+GP_API int gp_scorenet_ode_objects_t0(const void *packed, const float *proj, const double *x0,
+                               const float *pts_center, int N, int rows_per_object, const double *T_obj, double eps,
+                               double rtol, double atol, int denoise, double *x_out, const double *t_eval,
+                               int n_eval, double *dense, double *stats, double *obj_stats, void *workspace,
+                               size_t workspace_bytes, int mode, gp_stream_t s);
+
+/* Keyed per-object initial noise of the ODE sampler (DESIGN.md section 4.6f): noise [B*R, 9] f32 (device), where the
+ * block of object b (rows b*R .. b*R+R-1) depends only on keys[b] and sigma[b], never on b, B or the other keys.
+ *   keys    [B] int64 (device);  sigma [B] f32 (device): the standard deviation of object b's block.
+ * Definition: Philox4x32-10 keyed with (lo32, hi32) of keys[b].  Element e = r*9 + c of the block belongs to Box-Muller
+ * pair p = e / 2; pair p uses the words 2*(p % 2) and 2*(p % 2) + 1 of the Philox output for counter (p / 2, 0, 0, 0).
+ * The words give u_a, u_b = (w + 0.5) * 2^-32 (f64); n_2p = sqrt(-2 ln u_a) cos(2 pi u_b) and n_2p+1 = sqrt(-2 ln u_a)
+ * sin(2 pi u_b) in f64, rounded to f32.  The output is n * sigma[b], multiplied in f32 (as ve_prior scales its f32
+ * normals).  R*9 odd: the sine of the last pair is dropped. */
+GP_API int gp_object_noise(const int64_t *keys, const float *sigma, int B, int R, float *noise, gp_stream_t s);
 
 /* Post-processing of a recorded trajectory into the reference's `xs` (samplers.py:251-255):
  * traj [S,N,9] f64 raw -> xs [N,S,9] f64 with Gram-Schmidt on the rotation part and the centre
