@@ -79,6 +79,7 @@ SIGNATURES = {
                                  c_int, c_void_p]),
     "gp_trunk_packed_bytes": (c_size_t, []),
     "gp_trunk_pack": (c_int, [ctypes.POINTER(TrunkParams), c_void_p, c_void_p]),
+    "gp_trunk_pack_tf32": (c_int, [ctypes.POINTER(TrunkParams), c_void_p, c_void_p]),
     "gp_trunk_project": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
     "gp_scorenet_eval": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p]),
     "gp_scorenet_ode_workspace_bytes": (c_size_t, [c_int]),

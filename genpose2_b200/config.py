@@ -40,7 +40,7 @@ def build_parser():
     p.add_argument("--clustering_eps", type=float, default=0.05)
     p.add_argument("--clustering_minpts", type=float, default=0.1667)
     p.add_argument("--retain_ratio", type=float, default=0.4)
-    # not in the reference: numerical mode of the fused MLP kernels (fp32 | fp32_ffma | bf16), see scorenet.MLP_MODES
+    # not in the reference: numerical mode of the fused MLP kernels (fp32 | fp32_ffma | tf32 | bf16), see scorenet.MLP_MODES
     p.add_argument("--mlp_mode", type=str, default="fp32")
     # not in the reference: RK45 step-size control shared by the batch (batch) or per object (object), see
     # samplers.STEP_CONTROLS

@@ -84,6 +84,30 @@ __device__ __forceinline__ void umma_bf16_ts_w(uint32_t d_tmem, uint32_t a_tmem,
         "@q tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
         ::"r"(d_tmem), "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
 }
+// D[tmem] (+)= A[tmem] * B[smem]^T, tf32 x tf32 -> f32, K = 8: the A operand is 8 consecutive 32-bit TMEM columns
+// starting at a_tmem (column k = element k); a K = 8 step reads 32 bytes of a B row, as a K = 16 bf16 step does
+__device__ __forceinline__ void umma_tf32_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}"
+        ::"r"(d_tmem), "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
+}
+__device__ __forceinline__ void umma_tf32_ts_w(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p, q;\n\t"
+        "elect.sync _|q, 0xffffffff;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "@q tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}"
+        ::"r"(d_tmem), "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
+}
+// fp32 -> tf32 operand value: round to nearest on the 13 dropped significand bits, ties away from zero (the MMA itself
+// would truncate them)
+__device__ __forceinline__ float tf32_rna(float x) {
+    uint32_t r;
+    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
+    return __uint_as_float(r);
+}
 __device__ __forceinline__ void umma_commit_w(unsigned long long *bar) {
     asm volatile(
         "{\n\t.reg .pred q;\n\t"
@@ -101,6 +125,10 @@ __device__ __forceinline__ uint64_t make_desc(uint32_t smem_addr) {
 // N>>3 at bit 17, M>>4 at bit 24
 __host__ __device__ constexpr uint32_t make_idesc_bf16(uint32_t M, uint32_t N) {
     return (1u << 4) | (1u << 7) | (1u << 10) | ((N >> 3) << 17) | ((M >> 4) << 24);
+}
+// the same for kind::tf32: a = TF32 (2 << 7), b = TF32 (2 << 10)
+__host__ __device__ constexpr uint32_t make_idesc_tf32(uint32_t M, uint32_t N) {
+    return (1u << 4) | (2u << 7) | (2u << 10) | ((N >> 3) << 17) | ((M >> 4) << 24);
 }
 
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {

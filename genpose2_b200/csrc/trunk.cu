@@ -17,6 +17,29 @@ struct RawTrunk {
     gp_trunk_params p;
 };
 
+// One 32-bit slot of a tensor-core weight image.  `row` holds k 0..nk-1 of the image's 64-wide k-atom (nk <= 64; k >= nk
+// is zero), `which` the image of the pair, `wb` the slot's byte offset inside its 128-byte row and `logical16` its
+// 16-byte unit with the SWIZZLE_128B XOR undone.
+//   bf16 (TF32 = false): k = kl, kl + 1 of the atom as bf16 hi (which 0) or lo = bf16(w - hi) (which 1) parts;
+//   tf32: k = 32 which + 4 logical16 + (wb % 16) / 4, rounded to tf32 (cvt.rna, the rounding of the A operand).
+template <bool TF32>
+__device__ __forceinline__ float pack_tc_slot(const float *row, size_t nk, size_t which, size_t logical16, size_t wb) {
+    if (TF32) {
+        const size_t k = 32 * which + logical16 * 4 + (wb % 16) / 4;
+        return k < nk ? tc::tf32_rna(row[k]) : 0.f;
+    }
+    const size_t kl = logical16 * 8 + (wb % 16) / 2;    // k inside the 64-wide atom (even)
+    float e[2];
+    for (int t = 0; t < 2; ++t) {
+        const float src = kl + t < nk ? row[kl + t] : 0.f;
+        const float hi = __bfloat162float(__float2bfloat16_rn(src));
+        e[t] = which == 0 ? hi : src - hi;
+    }
+    __nv_bfloat162 h2 = __floats2bfloat162_rn(e[0], e[1]);
+    return *reinterpret_cast<float *>(&h2);
+}
+
+template <bool TF32>
 __global__ void pack_trunk_kernel(RawTrunk raw, float *__restrict__ P) {
     const gp_trunk_params &p = raw.p;
     const size_t stride = (size_t)gridDim.x * blockDim.x;
@@ -66,16 +89,8 @@ __global__ void pack_trunk_kernel(RawTrunk raw, float *__restrict__ P) {
             const size_t im = f / per_img, which = im % 2, kc = (im / 2) % 4, r = im / 8, o = (f % per_img) * 4;
             const size_t nl = o / 128, wb = o % 128;
             const size_t logical16 = (wb / 16) ^ (nl & 7);
-            const size_t kl = logical16 * 8 + (wb % 16) / 2;
-            const size_t hh = nl / 64, n = 64 * r + nl % 64, k = kc * 64 + kl;
-            float e[2];
-            for (int t = 0; t < 2; ++t) {
-                const float src = p.head_w0[hh][n * 1408 + 1152 + k + t];
-                const float hi = __bfloat162float(__float2bfloat16_rn(src));
-                e[t] = which == 0 ? hi : src - hi;
-            }
-            __nv_bfloat162 h2 = __floats2bfloat162_rn(e[0], e[1]);
-            v = *reinterpret_cast<float *>(&h2);
+            const size_t hh = nl / 64, n = 64 * r + nl % 64;
+            v = pack_tc_slot<TF32>(p.head_w0[hh] + n * 1408 + 1152 + kc * 64, 64, which, logical16, wb);
         } else {
             // destination float slot -> (chunk q, image hi/lo, row n, 16-byte unit, element pair)
             const size_t f = i - TrunkLayout::W_TC;
@@ -84,31 +99,24 @@ __global__ void pack_trunk_kernel(RawTrunk raw, float *__restrict__ P) {
             const size_t q = f / (2 * per_img), which = (f / per_img) % 2, o = (f % per_img) * 4;
             const size_t nl = o / 128, wb = o % 128;
             const size_t logical16 = (wb / 16) ^ (nl & 7);      // undo the SWIZZLE_128B XOR
-            const size_t kl = logical16 * 8 + (wb % 16) / 2;    // k inside the 64-wide atom (even)
-            float src[2] = {0.f, 0.f};
+            const float *row;                                   // k 0.. of the image's k-atom
+            size_t nk = 64;
             if (q < 2) {                 // pose_encoder.0: [256][9], zero-padded to k = 64
-                const size_t n = q * 128 + nl;
-                for (int t = 0; t < 2; ++t)
-                    if (kl + t < 9) src[t] = p.pose_w0[n * 9 + kl + t];
+                row = p.pose_w0 + (q * 128 + nl) * 9;
+                nk = 9;
             } else if (q < 10) {         // pose_encoder.2
-                const size_t kc = (q - 2) / 2, nh = (q - 2) % 2, n = nh * 128 + nl, k = kc * 64 + kl;
-                for (int t = 0; t < 2; ++t) src[t] = p.pose_w1[n * 256 + k + t];
+                const size_t kc = (q - 2) / 2, nh = (q - 2) % 2, n = nh * 128 + nl;
+                row = p.pose_w1 + n * 256 + kc * 64;
             } else if (q < TrunkLayout::TC_CHUNKS) {   // head columns of one cluster rank, two k-atoms per image
                 const size_t r = (q - 10) / 6, hh = ((q - 10) % 6) / 2, j = (q - 10) % 2;
-                const size_t kc = 2 * j + nl / 64, n = 64 * r + nl % 64, k = kc * 64 + kl;
-                for (int t = 0; t < 2; ++t) src[t] = p.head_w0[hh][n * 1408 + 1152 + k + t];
+                const size_t kc = 2 * j + nl / 64, n = 64 * r + nl % 64;
+                row = p.head_w0[hh] + n * 1408 + 1152 + kc * 64;
             } else {                     // whole heads: [h][kc][nh] images of [128 n][64 k]
                 const size_t qs = q - TrunkLayout::TC_CHUNKS;
-                const size_t hh = qs / 8, kc = (qs % 8) / 2, nh = qs % 2, n = nh * 128 + nl, k = kc * 64 + kl;
-                for (int t = 0; t < 2; ++t) src[t] = p.head_w0[hh][n * 1408 + 1152 + k + t];
+                const size_t hh = qs / 8, kc = (qs % 8) / 2, nh = qs % 2, n = nh * 128 + nl;
+                row = p.head_w0[hh] + n * 1408 + 1152 + kc * 64;
             }
-            float e[2];
-            for (int t = 0; t < 2; ++t) {
-                const float hi = __bfloat162float(__float2bfloat16_rn(src[t]));
-                e[t] = which == 0 ? hi : src[t] - hi;
-            }
-            __nv_bfloat162 h2 = __floats2bfloat162_rn(e[0], e[1]);
-            v = *reinterpret_cast<float *>(&h2);
+            v = pack_tc_slot<TF32>(row, nk, which, logical16, wb);
         }
         P[i] = v;
     }
@@ -343,6 +351,8 @@ static_assert(sizeof(solo::Smem<3>) + 1024 + 768 <= 227 * 1024, "solo evaluator 
 static_assert(sizeof(solo::Smem<1>) + 1024 + 768 <= 227 * 1024, "solo evaluator shared memory exceeds 227 KB");
 static_assert(sizeof(tc::Smem<3>) + 1024 <= 227 * 1024, "TC evaluator shared memory exceeds 227 KB");
 static_assert(sizeof(tc::Smem<1>) + 1024 <= 227 * 1024, "TC evaluator shared memory exceeds 227 KB");
+static_assert(sizeof(solot::Smem<2>) == sizeof(solot::Smem<3>) && sizeof(tc::Smem<2>) == sizeof(tc::Smem<3>),
+              "tf32 mode uses the split mode's ring");
 
 // ------------------------------------------------------------------------------------------
 // single evaluation / energy: one CTA per tile; rows may carry different t (handled by runs)
@@ -1542,7 +1552,7 @@ static int launch_ode_obj(OdeObjArgs &oa, cudaStream_t st) {
 
 static size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
 
-// `mode` of the public entries: bits 0..1 = arithmetic (0 FFMA, 1 bf16, 2 split-bf16), GP_MODE_SOLO / GP_MODE_CLUSTER
+// `mode` of the public entries: bits 0..1 = arithmetic (0 FFMA, 1 bf16, 2 split-bf16, 3 tf32), GP_MODE_SOLO / GP_MODE_CLUSTER
 // force the shape of the tensor-core evaluator; by default a batch of more 128-row tiles than the GPU holds 4-CTA
 // clusters at once (33 on a B200) runs one CTA per tile.
 // 0: cluster shape, 1: one CTA per tile (A operand in shared memory), 2: one CTA per tile, A operand in tensor memory
@@ -1552,10 +1562,20 @@ static int use_solo(int mode, int N) {
     return (N + tc::RT - 1) / tc::RT > 32 ? ((mode & GP_MODE_SMEM_A) ? 1 : 2) : 0;
 }
 static bool mode_ok(int mode) {
-    const int a = mode & 3;
-    return a <= 2 && (mode & ~(3 | GP_MODE_SOLO | GP_MODE_CLUSTER | GP_MODE_SMEM_A)) == 0 &&
+    return (mode & ~(3 | GP_MODE_SOLO | GP_MODE_CLUSTER | GP_MODE_SMEM_A)) == 0 &&
            (mode & (GP_MODE_SOLO | GP_MODE_CLUSTER)) != (GP_MODE_SOLO | GP_MODE_CLUSTER);
 }
+// Validation of `mode` shared by the trunk entries: a malformed value is a bad argument; tf32 (3) has evaluators with
+// the A operand in tensor memory only, so asking for the shared-memory-A shape is unsupported.
+#define GP_REQUIRE_MODE(mode, name)                                                                                    \
+    do {                                                                                                               \
+        GP_REQUIRE(mode_ok(mode), "%s: mode must be 0 (fp32 FFMA), 1 (bf16 tcgen05), 2 (split-bf16 x3 tcgen05) or 3 "  \
+                   "(tf32 tcgen05) [| GP_MODE_SOLO / GP_MODE_CLUSTER / GP_MODE_SMEM_A]", name);                         \
+        if (((mode) & 3) == 3 && ((mode) & GP_MODE_SMEM_A)) {                                                          \
+            gp::set_error("%s: tf32 mode (3) has no shared-memory-A evaluator (GP_MODE_SMEM_A)", name);                 \
+            return GP_ERR_UNSUPPORTED;                                                                                 \
+        }                                                                                                              \
+    } while (0)
 
 // Rows per compute thread of the FFMA evaluator (tile = 4x that many rows): the choice that minimises the
 // per-CTA critical path  waves(tiles / SMs) x rows-per-tile; ties go to the larger tile (fewer weight streams).
@@ -1576,18 +1596,27 @@ using namespace gp;
 
 extern "C" size_t gp_trunk_packed_bytes(void) { return TrunkLayout::END * sizeof(float); }
 
-extern "C" int gp_trunk_pack(const gp_trunk_params *raw, void *packed, gp_stream_t s) {
-    GP_REQUIRE(raw && packed, "gp_trunk_pack: null pointer");
+template <bool TF32>
+static int trunk_pack(const gp_trunk_params *raw, void *packed, gp_stream_t s, const char *name) {
+    GP_REQUIRE(raw && packed, "%s: null pointer", name);
     GP_REQUIRE(raw->pose_w0 && raw->pose_b0 && raw->pose_w1 && raw->pose_b1 && raw->fourier_w && raw->t_w && raw->t_b,
-               "gp_trunk_pack: null parameter");
+               "%s: null parameter", name);
     for (int h = 0; h < 3; ++h)
-        GP_REQUIRE(raw->head_w0[h] && raw->head_b0[h] && raw->head_w1[h] && raw->head_b1[h], "gp_trunk_pack: null head %d", h);
-    GP_REQUIRE(((uintptr_t)packed & 15) == 0, "gp_trunk_pack: packed must be 16-byte aligned");
+        GP_REQUIRE(raw->head_w0[h] && raw->head_b0[h] && raw->head_w1[h] && raw->head_b1[h], "%s: null head %d", name, h);
+    GP_REQUIRE(((uintptr_t)packed & 15) == 0, "%s: packed must be 16-byte aligned", name);
     RawTrunk r;
     r.p = *raw;
-    pack_trunk_kernel<<<num_sms() * 4, 256, 0, as_stream(s)>>>(r, (float *)packed);
-    GP_CHECK_LAUNCH("gp_trunk_pack");
+    pack_trunk_kernel<TF32><<<num_sms() * 4, 256, 0, as_stream(s)>>>(r, (float *)packed);
+    GP_CHECK_LAUNCH(name);
     return GP_OK;
+}
+
+extern "C" int gp_trunk_pack(const gp_trunk_params *raw, void *packed, gp_stream_t s) {
+    return trunk_pack<false>(raw, packed, s, "gp_trunk_pack");
+}
+
+extern "C" int gp_trunk_pack_tf32(const gp_trunk_params *raw, void *packed, gp_stream_t s) {
+    return trunk_pack<true>(raw, packed, s, "gp_trunk_pack_tf32");
 }
 
 extern "C" int gp_trunk_project(const void *packed, const float *pts_feat, int B, float *proj, gp_stream_t s) {
@@ -1618,7 +1647,9 @@ static int launch_eval(const void *packed, const float *proj, const float *x, co
     int rc;
     const int solo_shape = use_solo(mode, N);
     mode &= 3;
-    if (mode == 1 && solo_shape == 2) rc = launch_eval_ev<TcSoloT<1>, MODE>(packed, proj, x, poses, center, t, N, rpo, out, st);
+    if (mode == 3) rc = solo_shape == 2 ? launch_eval_ev<TcSoloT<2>, MODE>(packed, proj, x, poses, center, t, N, rpo, out, st)
+                                        : launch_eval_ev<TcEval<2>, MODE>(packed, proj, x, poses, center, t, N, rpo, out, st);
+    else if (mode == 1 && solo_shape == 2) rc = launch_eval_ev<TcSoloT<1>, MODE>(packed, proj, x, poses, center, t, N, rpo, out, st);
     else if (mode == 2 && solo_shape == 2) rc = launch_eval_ev<TcSoloT<3>, MODE>(packed, proj, x, poses, center, t, N, rpo, out, st);
     else if (mode == 1 && solo_shape) rc = launch_eval_ev<TcSolo<1>, MODE>(packed, proj, x, poses, center, t, N, rpo, out, st);
     else if (mode == 2 && solo_shape) rc = launch_eval_ev<TcSolo<3>, MODE>(packed, proj, x, poses, center, t, N, rpo, out, st);
@@ -1635,7 +1666,7 @@ extern "C" int gp_scorenet_eval(const void *packed, const float *proj, const flo
     GP_REQUIRE(N >= 0 && rows_per_object >= 1, "gp_scorenet_eval: bad sizes");
     if (N == 0) return GP_OK;
     GP_REQUIRE(packed && proj && x && t && score, "gp_scorenet_eval: null pointer");
-    GP_REQUIRE(mode_ok(mode), "gp_scorenet_eval: mode must be 0 (fp32 FFMA), 1 (bf16 tcgen05) or 2 (split-bf16 x3 tcgen05) [| GP_MODE_SOLO / GP_MODE_CLUSTER / GP_MODE_SMEM_A]");
+    GP_REQUIRE_MODE(mode, "gp_scorenet_eval");
     return launch_eval<0>(packed, proj, x, nullptr, nullptr, t, N, rows_per_object, score, mode, as_stream(s), "gp_scorenet_eval");
 }
 
@@ -1644,7 +1675,7 @@ extern "C" int gp_energy(const void *packed, const float *proj, const double *po
     GP_REQUIRE(N >= 0 && rows_per_object >= 1, "gp_energy: bad sizes");
     if (N == 0) return GP_OK;
     GP_REQUIRE(packed && proj && poses && pts_center && t_rows && energy, "gp_energy: null pointer");
-    GP_REQUIRE(mode_ok(mode), "gp_energy: mode must be 0 (fp32 FFMA), 1 (bf16 tcgen05) or 2 (split-bf16 x3 tcgen05) [| GP_MODE_SOLO / GP_MODE_CLUSTER / GP_MODE_SMEM_A]");
+    GP_REQUIRE_MODE(mode, "gp_energy");
     return launch_eval<1>(packed, proj, nullptr, poses, pts_center, t_rows, N, rows_per_object, energy, mode, as_stream(s), "gp_energy");
 }
 
@@ -1667,7 +1698,7 @@ static int scorenet_ode_impl(const void *packed, const float *proj, const double
     GP_REQUIRE(N >= 1 && rows_per_object >= 1, "gp_scorenet_ode: bad sizes N=%d rows_per_object=%d", N, rows_per_object);
     GP_REQUIRE(rtol > 0 && atol > 0, "gp_scorenet_ode: tolerances must be positive");
     GP_REQUIRE(traj == nullptr || max_traj >= 1, "gp_scorenet_ode: max_traj < 1");
-    GP_REQUIRE(mode_ok(mode), "gp_scorenet_ode: mode must be 0 (fp32 FFMA), 1 (bf16 tcgen05) or 2 (split-bf16 x3 tcgen05) [| GP_MODE_SOLO / GP_MODE_CLUSTER / GP_MODE_SMEM_A]");
+    GP_REQUIRE_MODE(mode, "gp_scorenet_ode");
     GP_REQUIRE((t_eval == nullptr) == (dense == nullptr) && (t_eval == nullptr || n_eval >= 1), "gp_scorenet_ode_dense: t_eval / dense / n_eval inconsistent");
     if (workspace_bytes < gp_scorenet_ode_workspace_bytes(N)) {
         set_error("gp_scorenet_ode: workspace too small (%zu < %zu)", workspace_bytes, gp_scorenet_ode_workspace_bytes(N));
@@ -1695,6 +1726,7 @@ static int scorenet_ode_impl(const void *packed, const float *proj, const double
     const int sms = num_sms();
     const int solo_shape = use_solo(mode, N);
     mode &= 3;
+    if (mode == 3) return solo_shape == 2 ? launch_ode<TcSoloT<2>>(a, st) : launch_ode<TcEval<2>>(a, st);
     if (mode == 1) return solo_shape == 2 ? launch_ode<TcSoloT<1>>(a, st) : solo_shape ? launch_ode<TcSolo<1>>(a, st) : launch_ode<TcEval<1>>(a, st);
     if (mode == 2) return solo_shape == 2 ? launch_ode<TcSoloT<3>>(a, st) : solo_shape ? launch_ode<TcSolo<3>>(a, st) : launch_ode<TcEval<3>>(a, st);
     switch (simt_rows_per_thread(N, sms)) {
@@ -1747,7 +1779,7 @@ static int scorenet_ode_objects_impl(const void *packed, const float *proj, cons
         return GP_ERR_UNSUPPORTED;
     }
     GP_REQUIRE(rtol > 0 && atol > 0, "gp_scorenet_ode_objects: tolerances must be positive");
-    GP_REQUIRE(mode_ok(mode), "gp_scorenet_ode_objects: mode must be 0 (fp32 FFMA), 1 (bf16 tcgen05) or 2 (split-bf16 x3 tcgen05) [| GP_MODE_SOLO / GP_MODE_CLUSTER / GP_MODE_SMEM_A]");
+    GP_REQUIRE_MODE(mode, "gp_scorenet_ode_objects");
     GP_REQUIRE((t_eval == nullptr) == (dense == nullptr) && (t_eval == nullptr || n_eval >= 1),
                "gp_scorenet_ode_dense_objects: t_eval / dense / n_eval inconsistent");
     const int B = N / rows_per_object;
@@ -1780,7 +1812,8 @@ static int scorenet_ode_objects_impl(const void *packed, const float *proj, cons
     const int solo_shape = use_solo(mode, B * tc::RT);
     mode &= 3;
     int rc;
-    if (mode == 1) rc = solo_shape == 2 ? launch_ode_obj<TcSoloT<1>>(oa, st) : solo_shape ? launch_ode_obj<TcSolo<1>>(oa, st) : launch_ode_obj<TcEval<1>>(oa, st);
+    if (mode == 3) rc = solo_shape == 2 ? launch_ode_obj<TcSoloT<2>>(oa, st) : launch_ode_obj<TcEval<2>>(oa, st);
+    else if (mode == 1) rc = solo_shape == 2 ? launch_ode_obj<TcSoloT<1>>(oa, st) : solo_shape ? launch_ode_obj<TcSolo<1>>(oa, st) : launch_ode_obj<TcEval<1>>(oa, st);
     else if (mode == 2) rc = solo_shape == 2 ? launch_ode_obj<TcSoloT<3>>(oa, st) : solo_shape ? launch_ode_obj<TcSolo<3>>(oa, st) : launch_ode_obj<TcEval<3>>(oa, st);
     else {
         // the FFMA tile height of a batch call with this one object, so that the two agree bit for bit
@@ -1859,7 +1892,7 @@ extern "C" int gp_scorenet_pc(const void *packed, const float *proj, const float
                               size_t workspace_bytes, int mode, gp_stream_t s) {
     GP_REQUIRE(packed && proj && x0 && noise && pts_center && time_steps && mean_x && workspace, "gp_scorenet_pc: null pointer");
     GP_REQUIRE(N >= 1 && rows_per_object >= 1 && num_steps >= 2, "gp_scorenet_pc: bad sizes");
-    GP_REQUIRE(mode_ok(mode), "gp_scorenet_pc: mode must be 0 (fp32 FFMA), 1 (bf16 tcgen05) or 2 (split-bf16 x3 tcgen05) [| GP_MODE_SOLO / GP_MODE_CLUSTER / GP_MODE_SMEM_A]");
+    GP_REQUIRE_MODE(mode, "gp_scorenet_pc");
     if (workspace_bytes < gp_scorenet_pc_workspace_bytes(N)) {
         set_error("gp_scorenet_pc: workspace too small");
         return GP_ERR_WORKSPACE;
@@ -1877,6 +1910,7 @@ extern "C" int gp_scorenet_pc(const void *packed, const float *proj, const float
     const int sms = num_sms();
     const int solo_shape = use_solo(mode, N);
     mode &= 3;
+    if (mode == 3) return solo_shape == 2 ? launch_pc<TcSoloT<2>>(a, st) : launch_pc<TcEval<2>>(a, st);
     if (mode == 1) return solo_shape == 2 ? launch_pc<TcSoloT<1>>(a, st) : solo_shape ? launch_pc<TcSolo<1>>(a, st) : launch_pc<TcEval<1>>(a, st);
     if (mode == 2) return solo_shape == 2 ? launch_pc<TcSoloT<3>>(a, st) : solo_shape ? launch_pc<TcSolo<3>>(a, st) : launch_pc<TcEval<3>>(a, st);
     switch (simt_rows_per_thread(N, sms)) {

@@ -11,6 +11,7 @@
 //
 // TMEM map (512 columns x 128 lanes, lane = row of the tile):
 //   [  0..127]  A hi : 256 k as packed bf16 pairs (column j = k 2j, 2j+1)      [128..255]  A lo (split mode)
+//   (tf32 mode: [0..255] = 256 k, column k = tf32 value of k; a weight chunk's two images hold k 0..31 and 32..63)
 //   [256..383]  accumulator slot 0                                            [384..511]  accumulator slot 1
 // Per evaluation:
 //   x (K = 16)  -> D0 = slots 0|1 (N = 256)  -> h1 = relu(D0 + b1) -> A
@@ -32,7 +33,7 @@ constexpr int NSTAGE = 8;            // ring depth (single 16 KB images)
 
 template <int NPASS>
 struct Smem {
-    static constexpr int IMAGES = NPASS == 3 ? 2 : 1;
+    static constexpr int IMAGES = NPASS == 1 ? 1 : 2;
     static constexpr int ENTRIES = NCHUNKS * IMAGES;   // ring entries (single images) per evaluation
     uint8_t ring[NSTAGE][IMG_BYTES];          // 128 KB; the struct sits on a 1024-byte boundary
     float4 wo[768];                           // output-layer weights per head column (3 used)
@@ -178,6 +179,21 @@ __device__ __noinline__ void forward(const float *__restrict__ P, const float *_
             // one weight chunk (hi image, then lo image in split mode) against k-atom `kc` of the A operand
             // (`nk` 16-wide k steps = 8 packed TMEM columns each) into accumulator columns d .. d + 127
             auto chunk = [&](uint32_t d, int kc, int nk, bool first) {
+                if constexpr (NPASS == 2) {
+                    // tf32: image w holds k 32 w .. 32 w + 31 of the k-atom; `nk` 16-wide k steps = 2 nk K = 8 MMAs
+                    for (int w = 0; w < 2; ++w) {
+                        const uint32_t g = st.consumed, s = g % NSTAGE;
+                        mbar_wait(&S.full[s], (g / NSTAGE) & 1);
+                        tc_fence_after();
+                        const uint32_t b = smem_u32(&S.ring[s][0]);
+                        for (int kk = 0; kk < 4 && 4 * w + kk < 2 * nk; ++kk)
+                            umma_tf32_ts(d, a_hi + (uint32_t)(kc * 64 + w * 32 + kk * 8), make_desc(b + kk * 32), kIdescT128,
+                                         (first && w == 0 && kk == 0) ? 0u : 1u);
+                        umma_commit(&S.empty[s]);
+                        st.consumed = g + 1;
+                    }
+                    return;
+                }
                 {
                     const uint32_t g = st.consumed, s = g % NSTAGE;
                     mbar_wait(&S.full[s], (g / NSTAGE) & 1);
@@ -244,23 +260,13 @@ __device__ __noinline__ void forward(const float *__restrict__ P, const float *_
         float *scratch = reinterpret_cast<float *>(gp_dyn_smem + (smem_u32(S.scratch) - dyn0));
 
         long long t0 = clock64();
-        // inputs -> A operand: k 0..8 (k 9..15 zero) as 8 packed columns, one row per thread of the first four epilogue warps
+        // inputs -> A operand: k 0..8 (k 9..15 zero), one row per thread of the first four epilogue warps
         if (half == 0) {
             float xv[9];
 #pragma unroll
             for (int c = 0; c < 9; ++c) xv[c] = sx[row * XS + c];
-            uint32_t hi[8], lo[8];
-#pragma unroll
-            for (int p = 0; p < 8; ++p) {
-                const float v0 = 2 * p < 9 ? xv[2 * p] : 0.f, v1 = 2 * p + 1 < 9 ? xv[2 * p + 1] : 0.f;
-                const __nv_bfloat162 h2 = __floats2bfloat162_rn(v0, v1);
-                const float2 hf = __bfloat1622float2(h2);
-                const __nv_bfloat162 l2 = __floats2bfloat162_rn(v0 - hf.x, v1 - hf.y);
-                hi[p] = *reinterpret_cast<const uint32_t *>(&h2);
-                lo[p] = *reinterpret_cast<const uint32_t *>(&l2);
-            }
-            tmem_st8(lane_addr + COL_A_HI, hi);
-            if (NPASS == 3) tmem_st8(lane_addr + COL_A_LO, lo);
+            if constexpr (NPASS == 2) store_x_tf32(lane_addr, xv);
+            else store_x_bf16<NPASS>(lane_addr, xv);
             tmem_st_wait();
         }
         tc_fence_before();

@@ -29,6 +29,10 @@
 //   hi*hi + lo*hi + hi*lo in fp32 (TMEM): 16 mantissa bits per operand.  On the reference's own fixtures this
 //   is indistinguishable from a plain fp32 evaluation (same size as changing the fp32 summation order),
 //   while plain bf16 costs 1e-3 rad / 3e-4.
+// NPASS = 2 ("tf32" mode): operands rounded to tf32 (cvt.rna, 11 significand bits), kind::tf32 MMAs of K = 8.  A tf32
+//   value is as wide as a hi + lo bf16 pair, so the layout is the split mode's: a chunk's two images hold k 0..31 and
+//   k 32..63 in the hi and lo slots of the ring, the A operand fills TMEM columns 0..255 (column = k), and a K = 8 step
+//   advances the descriptors by the bytes and columns of a K = 16 bf16 step: 2 MMAs per 16 k instead of 3.
 //
 // Per evaluation: D0 = x . W1^T ; h1 = relu(D0 + b1) ; D1 = h1 . W2^T ; h2 = relu(D1 + b2) ;
 // D2_h = h2 . Whp_h[64r..64r+63]^T (3 heads).  Operand layout: canonical K-major SWIZZLE_128B (8-row x
@@ -58,17 +62,21 @@ constexpr int MAX_SLOTS = 5;          // objects a tile may span for the shared-
 constexpr uint32_t kIdescN128 = make_idesc_bf16(128, 128);
 constexpr uint32_t kIdescN64 = make_idesc_bf16(128, 64);
 constexpr uint32_t kIdescN192 = make_idesc_bf16(128, NHC);
+constexpr uint32_t kIdescT128 = make_idesc_tf32(128, 128);
+constexpr uint32_t kIdescT192 = make_idesc_tf32(128, NHC);
 constexpr uint32_t COL_A_HI = 0, COL_A_LO = 128, COL_ACC = 256;   // TMEM columns: A operand (hi, lo), accumulators
 static_assert(TrunkLayout::TC_CHUNKS == NCOMMON + CL * NRANK, "packed chunk count");
 static_assert(TrunkLayout::WIDE_IMG_FLOATS * 4 == WIDE_BYTES, "wide head image size");
 
 template <int NPASS>
 struct Smem {
-    static constexpr int IMAGES = NPASS == 3 ? 2 : 1;
-    static constexpr int NSTAGE = NPASS == 3 ? 5 : 6;
-    // one ring slot holds a pose-encoder chunk ([128][64] image; hi + lo in split mode) or ONE wide head image (24 KB)
-    static constexpr int SLOT = NPASS == 3 ? 2 * IMG_BYTES : WIDE_BYTES;
-    // ring entries per evaluation: 10 pose-encoder chunks + 4 k-atoms of the wide head image (hi, lo separately)
+    static constexpr int IMAGES = NPASS == 1 ? 1 : 2;
+    static constexpr int NSTAGE = NPASS == 1 ? 6 : 5;
+    // one ring slot holds a pose-encoder chunk ([128][64] image; hi + lo in split mode, k 0..31 + k 32..63 in tf32
+    // mode) or ONE wide head image (24 KB)
+    static constexpr int SLOT = NPASS == 1 ? WIDE_BYTES : 2 * IMG_BYTES;
+    // ring entries per evaluation: 10 pose-encoder chunks (all images of a chunk in one slot) + 4 k-atoms of the wide
+    // head image (one slot per image)
     static constexpr int ENTRIES = NCOMMON + 4 * IMAGES;
     uint8_t ring[NSTAGE][SLOT];               // 160 / 144 KB; the struct sits on a 1024-byte boundary
     float stage[9 * RT];                      // this CTA's combined partial [c][row], source of the bulk copies to the peers
@@ -263,9 +271,32 @@ __device__ __forceinline__ void epi_hidden(uint32_t taddr, const float *sbias, i
 
 // accumulator columns [acc + c0, acc + c0 + 128) of this thread's row -> relu(. + bias) -> packed bf16 (hi / lo)
 // -> the A operand in TMEM (k = output column: 32 output columns = 16 packed 32-bit columns)
+// (tf32 mode: 32 output columns = 32 TMEM columns of tf32-rounded values)
 template <int NPASS>
 __device__ __forceinline__ void epi_hidden_t(uint32_t lane_addr, uint32_t acc, const float *sbias, int c0) {
     uint32_t r[2][32];
+    if constexpr (NPASS == 2) {
+        tmem_ld32_nowait(lane_addr + acc + c0, r[0]);
+#pragma unroll
+        for (int g = 0; g < 4; ++g) {
+            if (g + 1 < 4) tmem_ld32_nowait(lane_addr + acc + c0 + (g + 1) * 32, r[(g + 1) & 1]);
+            tmem_ld_wait();
+            uint32_t v[2][16];
+#pragma unroll
+            for (int j4 = 0; j4 < 8; ++j4) {
+                const float4 b = *reinterpret_cast<const float4 *>(sbias + c0 + g * 32 + j4 * 4);
+                const float bv[4] = {b.x, b.y, b.z, b.w};
+#pragma unroll
+                for (int j = 0; j < 4; ++j)
+                    v[j4 >> 2][(j4 & 3) * 4 + j] = __float_as_uint(tf32_rna(fmaxf(__uint_as_float(r[g & 1][j4 * 4 + j]) + bv[j], 0.f)));
+            }
+            const uint32_t kcol = (uint32_t)(c0 + g * 32);
+            tmem_st16(lane_addr + COL_A_HI + kcol, v[0]);
+            tmem_st16(lane_addr + COL_A_HI + kcol + 16, v[1]);
+        }
+        tmem_st_wait();
+        return;
+    }
     tmem_ld32_nowait(lane_addr + acc + c0, r[0]);
 #pragma unroll
     for (int g = 0; g < 4; ++g) {
@@ -293,6 +324,30 @@ __device__ __forceinline__ void epi_hidden_t(uint32_t lane_addr, uint32_t acc, c
         if (NPASS == 3) tmem_st16(lane_addr + COL_A_LO + kcol, lo);
     }
     tmem_st_wait();
+}
+
+// inputs (k 0..8, k 9..15 zero) of this thread's row -> the A operand in TMEM: 8 packed bf16 columns (hi, and lo in
+// split mode) or 16 tf32 columns
+template <int NPASS>
+__device__ __forceinline__ void store_x_bf16(uint32_t lane_addr, const float (&xv)[9]) {
+    uint32_t hi[8], lo[8];
+#pragma unroll
+    for (int p = 0; p < 8; ++p) {
+        const float v0 = 2 * p < 9 ? xv[2 * p] : 0.f, v1 = 2 * p + 1 < 9 ? xv[2 * p + 1] : 0.f;
+        const __nv_bfloat162 h2 = __floats2bfloat162_rn(v0, v1);
+        const float2 hf = __bfloat1622float2(h2);
+        const __nv_bfloat162 l2 = __floats2bfloat162_rn(v0 - hf.x, v1 - hf.y);
+        hi[p] = *reinterpret_cast<const uint32_t *>(&h2);
+        lo[p] = *reinterpret_cast<const uint32_t *>(&l2);
+    }
+    tmem_st8(lane_addr + COL_A_HI, hi);
+    if (NPASS == 3) tmem_st8(lane_addr + COL_A_LO, lo);
+}
+__device__ __forceinline__ void store_x_tf32(uint32_t lane_addr, const float (&xv)[9]) {
+    uint32_t v[16];
+#pragma unroll
+    for (int k = 0; k < 16; ++k) v[k] = k < 9 ? __float_as_uint(tf32_rna(xv[k])) : 0u;
+    tmem_st16(lane_addr + COL_A_HI, v);
 }
 
 // Head epilogue of one head for a warp's 32 rows x 32 accumulator columns: z = relu(D + e) and the 256 -> 3 output layer over
@@ -405,7 +460,7 @@ __device__ __noinline__ void forward(const float *__restrict__ P, const float *_
                 st.cyc_wfull += clock64() - w0;
                 tc_fence_after();
                 b_hi = smem_u32(&S.ring[stage][0]);
-                b_lo = b_hi + (NPASS == 3 ? IMG_BYTES : 0);
+                b_lo = b_hi + (NPASS != 1 ? IMG_BYTES : 0);
             };
             auto chunk_done = [&]() {
                 umma_commit(&S.empty[stage]);
@@ -424,7 +479,12 @@ __device__ __noinline__ void forward(const float *__restrict__ P, const float *_
             tc_fence_after();
             for (int nh = 0; nh < 2; ++nh) {
                 next_chunk();
-                mma(acc + nh * 128, 0, 0, kIdescN128, 0u);
+                if constexpr (NPASS == 2) {   // k 0..7, 8..15 of the first image
+                    umma_tf32_ts(acc + nh * 128, a_hi, make_desc(b_hi), kIdescT128, 0u);
+                    umma_tf32_ts(acc + nh * 128, a_hi + 8, make_desc(b_hi + 32), kIdescT128, 1u);
+                } else {
+                    mma(acc + nh * 128, 0, 0, kIdescN128, 0u);
+                }
                 chunk_done();
             }
             umma_commit(&S.dbar[0]);
@@ -442,16 +502,26 @@ __device__ __noinline__ void forward(const float *__restrict__ P, const float *_
                 tc_fence_after();
                 const uint32_t b0 = smem_u32(&S.ring[s0][0]), b1 = smem_u32(&S.ring[s1][0]);
                 const uint32_t bl0 = b0 + (NPASS == 3 ? IMG_BYTES : 0), bl1 = b1 + (NPASS == 3 ? IMG_BYTES : 0);
+                if constexpr (NPASS == 2) {
 #pragma unroll
-                for (int kk = 0; kk < 4; ++kk) {
-                    const uint32_t ac = kc * 32 + kk * 8, bo = kk * 32, accum = (kc | kk) ? 1u : 0u;
-                    umma_bf16_ts(acc, a_hi + ac, make_desc(b0 + bo), kIdescN128, accum);
-                    umma_bf16_ts(acc + 128, a_hi + ac, make_desc(b1 + bo), kIdescN128, accum);
-                    if (NPASS == 3) {
-                        umma_bf16_ts(acc, a_lo + ac, make_desc(b0 + bo), kIdescN128, 1u);
-                        umma_bf16_ts(acc + 128, a_lo + ac, make_desc(b1 + bo), kIdescN128, 1u);
-                        umma_bf16_ts(acc, a_hi + ac, make_desc(bl0 + bo), kIdescN128, 1u);
-                        umma_bf16_ts(acc + 128, a_hi + ac, make_desc(bl1 + bo), kIdescN128, 1u);
+                    for (int k8 = 0; k8 < 8; ++k8) {   // image k8 / 4 of the chunk, A columns = k
+                        const uint32_t ac = kc * 64 + k8 * 8, bo = (k8 >> 2) * IMG_BYTES + (k8 & 3) * 32;
+                        const uint32_t accum = (kc | k8) ? 1u : 0u;
+                        umma_tf32_ts(acc, a_hi + ac, make_desc(b0 + bo), kIdescT128, accum);
+                        umma_tf32_ts(acc + 128, a_hi + ac, make_desc(b1 + bo), kIdescT128, accum);
+                    }
+                } else {
+#pragma unroll
+                    for (int kk = 0; kk < 4; ++kk) {
+                        const uint32_t ac = kc * 32 + kk * 8, bo = kk * 32, accum = (kc | kk) ? 1u : 0u;
+                        umma_bf16_ts(acc, a_hi + ac, make_desc(b0 + bo), kIdescN128, accum);
+                        umma_bf16_ts(acc + 128, a_hi + ac, make_desc(b1 + bo), kIdescN128, accum);
+                        if (NPASS == 3) {
+                            umma_bf16_ts(acc, a_lo + ac, make_desc(b0 + bo), kIdescN128, 1u);
+                            umma_bf16_ts(acc + 128, a_lo + ac, make_desc(b1 + bo), kIdescN128, 1u);
+                            umma_bf16_ts(acc, a_hi + ac, make_desc(bl0 + bo), kIdescN128, 1u);
+                            umma_bf16_ts(acc + 128, a_hi + ac, make_desc(bl1 + bo), kIdescN128, 1u);
+                        }
                     }
                 }
                 umma_commit(&S.empty[s0]);
@@ -466,6 +536,17 @@ __device__ __noinline__ void forward(const float *__restrict__ P, const float *_
             mbar_wait(&S.a_ready, st.a_phase); st.a_phase ^= 1;
             tc_fence_after();
             for (int kc = 0; kc < 4; ++kc) {
+                if constexpr (NPASS == 2) {
+                    for (int w = 0; w < 2; ++w) {   // k 0..31, then k 32..63 of the k-atom
+                        next_chunk();
+#pragma unroll
+                        for (int kk = 0; kk < 4; ++kk)
+                            umma_tf32_ts(acc, a_hi + kc * 64 + w * 32 + kk * 8, make_desc(b_hi + kk * 32), kIdescT192,
+                                         (kc | w | kk) ? 1u : 0u);
+                        chunk_done();
+                    }
+                    continue;
+                }
                 next_chunk();   // hi image
 #pragma unroll
                 for (int kk = 0; kk < 4; ++kk) {
@@ -514,18 +595,8 @@ __device__ __noinline__ void forward(const float *__restrict__ P, const float *_
             float xv[9];
 #pragma unroll
             for (int c = 0; c < 9; ++c) xv[c] = sx[row * XS + c];
-            uint32_t hi[8], lo[8];
-#pragma unroll
-            for (int p = 0; p < 8; ++p) {
-                const float v0 = 2 * p < 9 ? xv[2 * p] : 0.f, v1 = 2 * p + 1 < 9 ? xv[2 * p + 1] : 0.f;
-                const __nv_bfloat162 h2 = __floats2bfloat162_rn(v0, v1);
-                const float2 hf = __bfloat1622float2(h2);
-                const __nv_bfloat162 l2 = __floats2bfloat162_rn(v0 - hf.x, v1 - hf.y);
-                hi[p] = *reinterpret_cast<const uint32_t *>(&h2);
-                lo[p] = *reinterpret_cast<const uint32_t *>(&l2);
-            }
-            tmem_st8(lane_addr + COL_A_HI, hi);
-            if (NPASS == 3) tmem_st8(lane_addr + COL_A_LO, lo);
+            if constexpr (NPASS == 2) store_x_tf32(lane_addr, xv);
+            else store_x_bf16<NPASS>(lane_addr, xv);
             tmem_st_wait();
         }
         tc_fence_before();

@@ -29,8 +29,10 @@ class GFObjectPose(nn.Module):
             raise NotImplementedError("pointnet2_params=%r: only 'light' (ClsMSG_CFG_Light)" % cfg.pointnet2_params)
         self.pts_encoder = Pointnet2ClsMSG(0)
         # SharedMLP operand precision: fp32 mode -> split-bf16 x3 on tcgen05 (fp32-class accuracy, 2e-5 of the
-        # reference's fp32 features), bf16 mode -> bf16 on tcgen05
-        self.pts_encoder.set_gemm_mode({"fp32": "bf16x3", "fp32_ffma": "bf16x3", "bf16": "bf16"}[getattr(cfg, "mlp_mode", "fp32")])
+        # reference's fp32 features), bf16 mode -> bf16 on tcgen05; tf32 mode keeps the encoder fp32-class (the trunk only
+        # runs in tf32)
+        self.pts_encoder.set_gemm_mode({"fp32": "bf16x3", "fp32_ffma": "bf16x3", "tf32": "bf16x3", "bf16": "bf16"}[
+            getattr(cfg, "mlp_mode", "fp32")])
         if cfg.agent_type == "score":
             self.pose_score_net = PoseScoreNet(self.marginal_prob_fn, 0, cfg.pose_mode, cfg.regression_head, False)
         elif cfg.agent_type == "energy":

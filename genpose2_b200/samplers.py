@@ -172,6 +172,8 @@ def _score_net(score_model):
     net = getattr(score_model, "pose_score_net", score_model)
     if not hasattr(net, "packed"):
         raise TypeError("score_model must be a genpose2_b200 GFObjectPose / PoseScoreNet (no fallback path)")
+    if hasattr(net, "mode_arg"):
+        net.mode_arg()   # an unsupported mlp_mode / eval_shape pair raises before the prior draw
     return net
 
 

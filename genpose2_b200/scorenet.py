@@ -20,8 +20,10 @@ from . import _lib
 #               as hi*hi + lo*hi + hi*lo in fp32): fp32-class results (same distance to the reference as a
 #               different fp32 summation order)
 #   "fp32_ffma" plain FP32 FFMA on the CUDA cores
+#   "tf32"      tf32 operands (round to nearest, 11 significand bits) on the tensor cores, fp32 accumulation: 2 MMAs
+#               per 16 k instead of 3 (DESIGN 4.6g); weights packed by gp_trunk_pack_tf32
 #   "bf16"      bf16 operands on the tensor cores, fp32 accumulation (stated looser bound)
-MLP_MODES = {"fp32_ffma": 0, "bf16": 1, "fp32": 2}
+MLP_MODES = {"fp32_ffma": 0, "bf16": 1, "fp32": 2, "tf32": 3}
 # shape of the tensor-core evaluator (include/genpose_b200.h, gp_mode_flag): "auto" = one CTA per 128-row tile for
 # batches of more than 32 tiles, a 4-CTA cluster per tile below; "solo" / "cluster" force one
 EVAL_SHAPES = {"auto": 0, "solo": 16, "cluster": 32, "solo_smem_a": 16 | 64}
@@ -76,10 +78,13 @@ class _Trunk(nn.Module):
                 heads)
 
     def packed(self):
-        """Device blob in the layout of csrc/trunk.cuh; rebuilt when any parameter was modified."""
+        """Device blob in the layout of csrc/trunk.cuh (gp_trunk_pack_tf32's for mlp_mode "tf32"); rebuilt when any
+        parameter or the kind of blob was modified."""
+        self.mode_arg()   # an unsupported mode / shape pair raises before any device work
         base, heads = self._raw_tensors()
         tensors = base + [t for h in heads for t in (h[0].weight, h[0].bias, h[2].weight, h[2].bias)]
-        key = tuple((t.data_ptr(), t._version) for t in tensors)
+        pack = "gp_trunk_pack_tf32" if self.mlp_mode == "tf32" else "gp_trunk_pack"
+        key = (pack,) + tuple((t.data_ptr(), t._version) for t in tensors)
         if self._packed is None or key != self._packed_key:
             dev = tensors[0].device
             if dev.type != "cuda":
@@ -93,13 +98,16 @@ class _Trunk(nn.Module):
                     w0.data_ptr(), b0.data_ptr(), w1.data_ptr(), b1.data_ptr())
             nbytes = _lib.load().gp_trunk_packed_bytes()
             blob = torch.empty(nbytes // 4, dtype=torch.float32, device=dev)
-            _lib.call("gp_trunk_pack", ctypes.byref(p), _lib.ptr(blob), device=dev)
+            _lib.call(pack, ctypes.byref(p), _lib.ptr(blob), device=dev)
             self._packed, self._packed_key = blob, key
         return self._packed
 
     def mode_arg(self):
         """the `mode` argument of the C entries: arithmetic | evaluator-shape flag"""
         m = MLP_MODES[self.mlp_mode]
+        if self.mlp_mode == "tf32" and self.eval_shape == "solo_smem_a":
+            raise ValueError("mlp_mode='tf32' runs with the A operand in tensor memory only: eval_shape='solo_smem_a' "
+                             "is not supported")
         return m | (EVAL_SHAPES[self.eval_shape] if m else 0)
 
     def project(self, pts_feat):

@@ -226,6 +226,13 @@ typedef struct gp_trunk_params {
 GP_API size_t gp_trunk_packed_bytes(void);
 /* Packs `raw` (device pointers) into `packed`.  Do once per checkpoint. */
 GP_API int gp_trunk_pack(const gp_trunk_params *raw, void *packed, gp_stream_t s);
+/* The blob of tf32 mode (mode 3 of the trunk entries): the same size and layout as gp_trunk_pack's, except that the
+ * tensor-core weight images hold tf32 values (cvt.rna: round to nearest on the 13 dropped bits, ties away from zero)
+ * with the two images of a 64-k chunk holding k 0..31 and k 32..63 instead of bf16 hi and lo parts.  The fp32
+ * matrices, biases and output layers are identical, so gp_trunk_project accepts either blob.
+ * Mode 3 needs a blob from gp_trunk_pack_tf32, modes 0..2 one from gp_trunk_pack.  The library cannot tell them
+ * apart without reading device memory: passing the wrong kind is the caller's error and gives wrong results. */
+GP_API int gp_trunk_pack_tf32(const gp_trunk_params *raw, void *packed, gp_stream_t s);
 
 /* Per-object hoisted head projection: proj[b, 0:768] = head_w0[:, :1024] @ pts_feat[b] + head_b0
  * (the pts_feat columns of scorenet.py:249,259-261, constant over hypotheses and ODE stages).
@@ -235,19 +242,21 @@ GP_API int gp_trunk_project(const void *packed, const float *pts_feat, int B, fl
 /* One PoseScoreNet.forward (scorenet.py:215-275): x [N,9] f32, t [N] f32 (one value per row),
  * proj [B,768] with row i belonging to object i / rows_per_object -> score [N,9] f32
  * (= f_theta / (std + 1e-7)).  Used by GFObjectPose.forward(mode="score") (posenet.py:305-307).
- * mode: 0 = fp32 FFMA, 1 = bf16 tcgen05, 2 = split-bf16 x3 tcgen05 (fp32-class), as for gp_scorenet_ode. */
+ * mode: 0 = fp32 FFMA, 1 = bf16 tcgen05, 2 = split-bf16 x3 tcgen05 (fp32-class), 3 = tf32 tcgen05, as for
+ * gp_scorenet_ode. */
 GP_API int gp_scorenet_eval(const void *packed, const float *proj, const float *x, const float *t, int N,
                      int rows_per_object, float *score, int mode, gp_stream_t s);
 
 /* Flags that may be OR-ed into the `mode` argument of gp_scorenet_eval / _ode / _ode_dense / _pc / gp_energy when it
- * selects a tensor-core arithmetic (1 or 2).  The tensor-core evaluator has two shapes: a 4-CTA cluster per 128-row
+ * selects a tensor-core arithmetic (1, 2 or 3).  The tensor-core evaluator has two shapes: a 4-CTA cluster per 128-row
  * tile (shortest critical path; every CTA re-evaluates the pose encoder and integrates a private copy of the state)
  * and one CTA per tile (no redundant work, one state copy: the throughput shape).  Default: one CTA per tile when the
  * batch has more than 32 tiles (more than the GPU holds clusters at once), clusters otherwise. */
 enum gp_mode_flag {
     GP_MODE_SOLO = 16,    /* force one CTA per tile */
     GP_MODE_CLUSTER = 32, /* force a 4-CTA cluster per tile */
-    GP_MODE_SMEM_A = 64   /* one-CTA-per-tile shape: keep the activations (A operand) in shared memory instead of tensor memory */
+    GP_MODE_SMEM_A = 64   /* one-CTA-per-tile shape: keep the activations (A operand) in shared memory instead of tensor memory
+                             (modes 1 and 2 only: with mode 3 the entries return GP_ERR_UNSUPPORTED) */
 };
 
 /* Integrator statistics written by gp_scorenet_ode (device, 16 doubles). */
@@ -282,8 +291,10 @@ GP_API size_t gp_scorenet_ode_workspace_bytes(int N);
  *   stats       [GP_STAT_COUNT] f64 (device)
  *   mode        arithmetic of the MLP contractions: 0 = fp32 FFMA on CUDA cores; 1 = bf16 operands on tcgen05;
  *               2 = tcgen05 with every operand split into two bf16 (hi*hi + lo*hi + hi*lo, fp32 accumulation in
- *               TMEM: 16 mantissa bits per operand, indistinguishable from fp32 on the reference's fixtures).
- *               Modes 1 and 2 run as 4-CTA clusters per 128-row tile (cooperative launch).
+ *               TMEM: 16 mantissa bits per operand, indistinguishable from fp32 on the reference's fixtures);
+ *               3 = tf32 operands on tcgen05 (kind::tf32, 11 significand bits, fp32 accumulation; `packed` from
+ *               gp_trunk_pack_tf32).
+ *               Modes 1..3 run as 4-CTA clusters per 128-row tile (cooperative launch) or one CTA per tile (gp_mode_flag).
  * The sampler kernels (this entry, gp_scorenet_ode_dense, gp_scorenet_pc) are persistent grids with a spin grid barrier,
  * launched cooperatively so that every CTA is resident.  The one process-wide switch this library reads is the
  * environment variable GP_NONCOOPERATIVE_LAUNCH=1 (read once): it drops the cooperative attribute for profilers that
