@@ -150,7 +150,8 @@ def test_tracking_sequence_matches_oracle():
 def test_config5_shard_size_properties():
     """BASELINE config 5: 8192 objects x 50 hypotheses sharded by object over 8 GPUs = 1024 objects
     (51 200 rows) per GPU.  One shard through the sampler + energy + aggregation + ScaleNet (features
-    injected: the encoder at this size is covered by the C3 sweep), size-independent properties."""
+    injected: the encoder at 1024 objects is covered by tests/test_gpu_encoder_scale.py, which checks its output against
+    float64 and its batch invariance), size-independent properties."""
     B, R = 1024, 50
     pipe = make_pipeline()
     g = torch.Generator().manual_seed(5)
