@@ -42,6 +42,9 @@ def build_parser():
     p.add_argument("--retain_ratio", type=float, default=0.4)
     # not in the reference: numerical mode of the fused MLP kernels (fp32 | fp32_ffma | tf32 | bf16), see scorenet.MLP_MODES
     p.add_argument("--mlp_mode", type=str, default="fp32")
+    # not in the reference: operand precision of the encoder's tensor-core SharedMLP GEMMs (auto | bf16x3 | bf16 | tf32);
+    # auto follows mlp_mode, see posenet.ENCODER_MODES
+    p.add_argument("--encoder_mode", type=str, default="auto")
     # not in the reference: RK45 step-size control shared by the batch (batch) or per object (object), see
     # samplers.STEP_CONTROLS
     p.add_argument("--step_control", type=str, default="batch")

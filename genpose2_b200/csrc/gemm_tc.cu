@@ -6,6 +6,8 @@
 // Operands are bf16 with fp32 accumulation in TMEM.  NPASS = 1: plain bf16 (bf16 mode).  NPASS = 3: every
 // fp32 value is split x = hi + lo (two bf16) and the product is accumulated as hi*hi + lo*hi + hi*lo:
 // 16 mantissa bits per operand, relative error ~2^-16 per product -- the fp32-mode encoder path.
+// NPASS = 2: tf32 operands rounded to nearest (11 significand bits; tc::tf32_rna_bits), tcgen05.mma.kind::tf32 K = 8.  A 64-k chunk is two
+// [rows][32 k] fp32 images (k 0..31, k 32..63) in the slots of the hi and lo images: same bytes, 8 MMAs instead of 12.
 //
 // CTA = 128 rows x BN (<= 256) columns, K streamed in chunks of 64 through NS shared-memory stages:
 //   warps 0-3  A loaders (one row per thread: 16-byte global loads, hi/lo split, swizzled 16-byte smem
@@ -52,19 +54,21 @@ __host__ __device__ inline int bn_of_tile(int N, int j) {  // columns of n-tile 
     return (rem + 15) & ~15;
 }
 __host__ __device__ inline size_t tile_image_bytes(int bn) { return (size_t)bn * 128; }
-// packed layout: for n-tile j, for chunk c: hi image [bn x 128 B] then (NPASS == 3) lo image
+// packed layout: for n-tile j, for chunk c: hi image [bn x 128 B] then (npass 3) lo image; npass 2: the tf32
+// images of k 0..31 and k 32..63
+__host__ __device__ inline int images_of(int npass) { return npass == 1 ? 1 : 2; }
 __host__ __device__ inline size_t packed_tile_offset(int N, int nchunks, int npass, int j) {
     size_t off = 0;
-    const int images = npass == 3 ? 2 : 1;
+    const int images = images_of(npass);
     for (int t = 0; t < j; ++t) off += (size_t)nchunks * images * tile_image_bytes(bn_of_tile(N, t));
     return off;
 }
 
 __global__ void pack_weights_kernel(const float *__restrict__ W, int N, int K, int npass, int nchunks,
                                     uint8_t *__restrict__ out, size_t total_bytes) {
-    // one thread per 4 bytes (two bf16) of the packed buffer
+    // one thread per 4 bytes (two bf16 or one tf32) of the packed buffer
     const size_t stride = (size_t)gridDim.x * blockDim.x;
-    const int images = npass == 3 ? 2 : 1;
+    const int images = images_of(npass);
     const int ntiles = (N + 255) / 256;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total_bytes / 4; i += stride) {
         size_t o = i * 4;
@@ -80,12 +84,18 @@ __global__ void pack_weights_kernel(const float *__restrict__ W, int N, int K, i
         const size_t rel = o - toff;
         const int c = (int)(rel / (images * img));
         const size_t in_c = rel % (images * img);
-        const int which = (int)(in_c / img);  // 0 hi, 1 lo
+        const int which = (int)(in_c / img);  // 0 hi, 1 lo (tf32: k 0..31, k 32..63)
         const size_t ob = in_c % img;
         const int nl = (int)(ob / 128), wb = (int)(ob % 128);
         const int logical16 = (wb / 16) ^ (nl & 7);
-        const int kk = logical16 * 8 + (wb % 16) / 2;
         const int n = 256 * j + nl;
+        if (npass == 2) {   // rounded as the activations are: the MMA would truncate the 13 dropped bits
+            const int k = c * KC + which * 32 + logical16 * 4 + (wb % 16) / 4;
+            const float w = (n < N && k < K) ? W[(size_t)n * K + k] : 0.f;
+            *reinterpret_cast<float *>(out + o) = tc::tf32_rna(w);
+            continue;
+        }
+        const int kk = logical16 * 8 + (wb % 16) / 2;
         float v[2];
         for (int e = 0; e < 2; ++e) {
             const int k = c * KC + kk + e;
@@ -131,7 +141,7 @@ __device__ __forceinline__ void pool_store(const float (&out)[32], int lane, boo
 // small grids run one CTA per SM with a deeper pipeline.
 template <int NPASS, int NS_>
 struct Cfg {
-    static constexpr int IMAGES = NPASS == 3 ? 2 : 1;
+    static constexpr int IMAGES = NPASS == 1 ? 1 : 2;
     static constexpr int NS = NS_;
     static constexpr int STAGE_BYTES = IMAGES * (A_TILE + B_TILE_MAX);
     static constexpr size_t SMEM = (size_t)NS * STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/;
@@ -226,6 +236,14 @@ __global__ void __launch_bounds__(NTHREADS, 2) gemm_bias_relu_kernel(Args a) {
                         p = make_float4(0.f, 0.f, 0.f, 0.f);
                     }
                 }
+                if (NPASS == 2) {
+                    // 16 bytes = k 4 jv .. 4 jv + 3: image jv / 8, 16-byte unit jv % 8 of its 128-byte row
+                    const int toff = rl * 128 + (((jv & 7) ^ (rl & 7)) << 4);
+                    const uint4 t = make_uint4(tc::tf32_rna_bits(p.x), tc::tf32_rna_bits(p.y), tc::tf32_rna_bits(p.z),
+                                               tc::tf32_rna_bits(p.w));
+                    *reinterpret_cast<uint4 *>((jv < 8 ? hi_img : lo_img) + toff) = t;
+                    continue;
+                }
                 const __nv_bfloat162 h0 = __floats2bfloat162_rn(p.x, p.y), h1 = __floats2bfloat162_rn(p.z, p.w);
                 uint2 pk;
                 pk.x = *reinterpret_cast<const uint32_t *>(&h0); pk.y = *reinterpret_cast<const uint32_t *>(&h1);
@@ -307,7 +325,7 @@ __global__ void __launch_bounds__(NTHREADS, 2) gemm_bias_relu_kernel(Args a) {
     } else {
         // ------------------------- MMA issuer -------------------------
         if (lane == 0) {
-            const uint32_t idesc = tc::make_idesc_bf16(128, (uint32_t)bn);
+            const uint32_t idesc = NPASS == 2 ? tc::make_idesc_tf32(128, (uint32_t)bn) : tc::make_idesc_bf16(128, (uint32_t)bn);
             for (int c = 0; c < a.nchunks; ++c) {
                 const int s = c % C::NS;
                 const uint32_t ph = (c / C::NS) & 1;
@@ -316,8 +334,15 @@ __global__ void __launch_bounds__(NTHREADS, 2) gemm_bias_relu_kernel(Args a) {
                 tc::tc_fence_after();
                 const uint32_t ahi = tc::smem_u32(a_img(s, 0)), alo = tc::smem_u32(a_img(s, 1));
                 const uint32_t bhi = tc::smem_u32(b_img(s, 0)), blo = tc::smem_u32(b_img(s, 1));
+                if (NPASS == 2) {
 #pragma unroll
-                for (int kk = 0; kk < 4; ++kk) {
+                    for (int kk = 0; kk < 8; ++kk) {   // K = 8 steps: 4 in the image of k 0..31, 4 in that of k 32..63
+                        const uint32_t ao = (kk < 4 ? ahi : alo) + (kk & 3) * 32, bo = (kk < 4 ? bhi : blo) + (kk & 3) * 32;
+                        tc::umma_tf32_ss(tmem, tc::make_desc(ao), tc::make_desc(bo), idesc, (c | kk) ? 1u : 0u);
+                    }
+                }
+#pragma unroll
+                for (int kk = 0; kk < (NPASS == 2 ? 0 : 4); ++kk) {
                     tc::umma_bf16(tmem, tc::make_desc(ahi + kk * 32), tc::make_desc(bhi + kk * 32), idesc, (c | kk) ? 1u : 0u);
                     if (NPASS == 3) {
                         tc::umma_bf16(tmem, tc::make_desc(alo + kk * 32), tc::make_desc(bhi + kk * 32), idesc, 1u);
@@ -348,9 +373,13 @@ template <int NPASS>
 static int launch(const Args &a, cudaStream_t st) {
     const long long ctas = ((a.R + BM - 1) / BM) * ((a.N + 255) / 256);
     const bool wide = ctas >= 2LL * num_sms();
-    // split-bf16: a stage is 96 KB (one per CTA when two CTAs share an SM, two otherwise); bf16: 48 KB (two / four)
-    if (NPASS == 3) return wide ? launch_ns<NPASS, 1>(a, st) : launch_ns<NPASS, 2>(a, st);
+    // split-bf16 and tf32: a stage is 96 KB (one per CTA when two CTAs share an SM, two otherwise); bf16: 48 KB (two / four)
+    if (NPASS != 1) return wide ? launch_ns<NPASS, 1>(a, st) : launch_ns<NPASS, 2>(a, st);
     return wide ? launch_ns<NPASS, 2>(a, st) : launch_ns<NPASS, 4>(a, st);
+}
+
+static int launch_npass(const Args &a, int npass, cudaStream_t st) {
+    return npass == 3 ? launch<3>(a, st) : npass == 2 ? launch<2>(a, st) : launch<1>(a, st);
 }
 
 }  // namespace gemm
@@ -359,14 +388,14 @@ static int launch(const Args &a, cudaStream_t st) {
 using namespace gp;
 
 extern "C" size_t gp_gemm_packed_bytes(int N, int K, int npass) {
-    if (N < 1 || K < 1 || (npass != 1 && npass != 3)) return 0;
+    if (N < 1 || K < 1 || npass < 1 || npass > 3) return 0;
     const int nchunks = (K + gemm::KC - 1) / gemm::KC;
     return gemm::packed_tile_offset(N, nchunks, npass, (N + 255) / 256);
 }
 
 extern "C" int gp_gemm_pack(const float *W, int N, int K, int npass, void *packed, gp_stream_t s) {
     GP_REQUIRE(W && packed, "gp_gemm_pack: null pointer");
-    GP_REQUIRE(N >= 1 && K >= 1 && (npass == 1 || npass == 3), "gp_gemm_pack: bad arguments");
+    GP_REQUIRE(N >= 1 && K >= 1 && npass >= 1 && npass <= 3, "gp_gemm_pack: bad arguments (npass must be 1, 2 or 3)");
     GP_REQUIRE(((uintptr_t)packed & 15) == 0, "gp_gemm_pack: packed must be 16-byte aligned");
     const int nchunks = (K + gemm::KC - 1) / gemm::KC;
     const size_t total = gp_gemm_packed_bytes(N, K, npass);
@@ -378,7 +407,7 @@ extern "C" int gp_gemm_pack(const float *W, int N, int K, int npass, void *packe
 extern "C" int gp_gemm_bias_relu(const float *X, long long R, int ldx, const void *packed, const float *bias, int N,
                                  int K, int npass, float *Y, int ldy, int pool_ns, float *pooled, int ld_pooled,
                                  gp_stream_t s) {
-    GP_REQUIRE(R >= 0 && N >= 1 && K >= 1 && (npass == 1 || npass == 3), "gp_gemm_bias_relu: bad arguments");
+    GP_REQUIRE(R >= 0 && N >= 1 && K >= 1 && npass >= 1 && npass <= 3, "gp_gemm_bias_relu: bad arguments (npass must be 1, 2 or 3)");
     if (R == 0) return GP_OK;
     GP_REQUIRE(X && packed && bias, "gp_gemm_bias_relu: null pointer");
     GP_REQUIRE(ldx >= 4 && (ldx & 3) == 0 && ((uintptr_t)X & 15) == 0, "gp_gemm_bias_relu: X rows must be 16-byte aligned (ldx %% 4 == 0)");
@@ -397,12 +426,12 @@ extern "C" int gp_gemm_bias_relu(const float *X, long long R, int ldx, const voi
     a.Y = Y; a.ldy = ldy; a.pool_ns = pool_ns; a.pooled = pooled; a.ld_pooled = ld_pooled;
     a.nchunks = (K + gemm::KC - 1) / gemm::KC;
     a.gidx = nullptr; a.rows_per_batch = 1; a.n_src = 0; a.Q = nullptr; a.ldq = 0; a.q_ns = 1; a.linear = 0;
-    return npass == 3 ? gemm::launch<3>(a, as_stream(s)) : gemm::launch<1>(a, as_stream(s));
+    return gemm::launch_npass(a, npass, as_stream(s));
 }
 
 extern "C" int gp_gemm_linear(const float *X, long long R, int ldx, const void *packed, int N, int K, int npass,
                               float *Y, int ldy, gp_stream_t s) {
-    GP_REQUIRE(R >= 0 && N >= 1 && K >= 1 && (npass == 1 || npass == 3), "gp_gemm_linear: bad arguments");
+    GP_REQUIRE(R >= 0 && N >= 1 && K >= 1 && npass >= 1 && npass <= 3, "gp_gemm_linear: bad arguments (npass must be 1, 2 or 3)");
     if (R == 0) return GP_OK;
     GP_REQUIRE(X && packed && Y, "gp_gemm_linear: null pointer");
     GP_REQUIRE(ldx >= 4 && (ldx & 3) == 0 && ((uintptr_t)X & 15) == 0, "gp_gemm_linear: X rows must be 16-byte aligned");
@@ -412,7 +441,7 @@ extern "C" int gp_gemm_linear(const float *X, long long R, int ldx, const void *
     a.Y = Y; a.ldy = ldy; a.pool_ns = 0; a.pooled = nullptr; a.ld_pooled = 0;
     a.nchunks = (K + gemm::KC - 1) / gemm::KC;
     a.gidx = nullptr; a.rows_per_batch = 1; a.n_src = 0; a.Q = nullptr; a.ldq = 0; a.q_ns = 1; a.linear = 1;
-    return npass == 3 ? gemm::launch<3>(a, as_stream(s)) : gemm::launch<1>(a, as_stream(s));
+    return gemm::launch_npass(a, npass, as_stream(s));
 }
 
 namespace gp {
@@ -466,7 +495,7 @@ extern "C" int gp_gemm_gather_bias_relu(const float *P, int n_src, int ldp, cons
                                         int rows_per_batch, const float *Q, int ldq, int q_ns, const void *packed,
                                         const float *bias, int N, int K, int npass, float *Y, int ldy, int pool_ns,
                                         float *pooled, int ld_pooled, gp_stream_t s) {
-    GP_REQUIRE(R >= 0 && N >= 1 && K >= 1 && (npass == 1 || npass == 3), "gp_gemm_gather_bias_relu: bad arguments");
+    GP_REQUIRE(R >= 0 && N >= 1 && K >= 1 && npass >= 1 && npass <= 3, "gp_gemm_gather_bias_relu: bad arguments (npass must be 1, 2 or 3)");
     if (R == 0) return GP_OK;
     GP_REQUIRE(P && gidx && Q && packed && bias, "gp_gemm_gather_bias_relu: null pointer");
     GP_REQUIRE(ldp >= 4 && (ldp & 3) == 0 && ((uintptr_t)P & 15) == 0 && ldq >= 4 && (ldq & 3) == 0 && ((uintptr_t)Q & 15) == 0,
@@ -486,5 +515,5 @@ extern "C" int gp_gemm_gather_bias_relu(const float *P, int n_src, int ldp, cons
     a.Y = Y; a.ldy = ldy; a.pool_ns = pool_ns; a.pooled = pooled; a.ld_pooled = ld_pooled;
     a.nchunks = (K + gemm::KC - 1) / gemm::KC;
     a.gidx = gidx; a.rows_per_batch = rows_per_batch; a.n_src = n_src; a.Q = Q; a.ldq = ldq; a.q_ns = q_ns; a.linear = 0;
-    return npass == 3 ? gemm::launch<3>(a, as_stream(s)) : gemm::launch<1>(a, as_stream(s));
+    return gemm::launch_npass(a, npass, as_stream(s));
 }

@@ -24,11 +24,15 @@
 // two 128-column chunks whose MMA chains are issued interleaved (a chain into one accumulator retires one MMA per ~90
 // cycles, an N = 128 MMA occupies the pipe for 64: two chains keep it busy).
 //
-// TMEM map: [0, hcols) H (hi: 32 columns per 64-wide k-atom, then lo in split mode) | [hcols, hcols + DN) accumulators.
+// TMEM map: [0, hcols) H (hi: 32 columns per 64-wide k-atom, then lo in split mode; tf32: one column per k, 64 per
+// k-atom) | [hcols, hcols + DN) accumulators.
 // CTA = NW worker warps + producer + MMA issuer, persistent over tiles: warp 0 streams the weight chunks
 // (cp.async.bulk, [<=128 n][64 k] images from the gp_gemm_pack layout) through a shared-memory ring and runs ahead
 // across tiles; warp 1 issues the MMAs; warps 2.. gather / convert / run both epilogues.
-// NPASS = 1: bf16 operands; NPASS = 3: split-bf16 (hi*hi + lo*hi + hi*lo), fp32-class.
+// NPASS = 1: bf16 operands; NPASS = 3: split-bf16 (hi*hi + lo*hi + hi*lo), fp32-class; NPASS = 2: tf32 operands
+// (rounded to nearest, tf32_rna_bits), kind::tf32 K = 8.  A tf32 64-k atom is two [rows][32 k] fp32 images (k 0..31, k 32..63) in the places of
+// the hi and lo images, so the ring, A buffer and TMEM plans are those of the split mode; an image whose k range is
+// beyond the layer's K (the second image of a K <= 32 layer) is neither streamed nor multiplied.
 #include "common.cuh"
 #include "tc_ptx.cuh"
 
@@ -81,8 +85,11 @@ struct Args {
 
 template <int NPASS>
 struct Cfg {
-    static constexpr int IMAGES = NPASS == 3 ? 2 : 1;
+    static constexpr int IMAGES = NPASS == 1 ? 1 : 2;
 };
+// whether image w of k-atom c of a layer with K = kdim takes part (the split mode's lo images always do)
+template <int NPASS>
+__host__ __device__ inline bool image_used(int kdim, int c, int w) { return NPASS != 2 || 64 * c + 32 * w < kdim; }
 
 __host__ __device__ inline int round16(int n) { return (n + 15) & ~15; }
 __host__ __device__ inline int atoms_of(int k) { return (k + 63) / 64; }
@@ -144,8 +151,8 @@ __device__ __forceinline__ void pool_block(const uint32_t (&r)[32], bool row_ok,
 }
 
 // First-level mode: one thread = one row.  x[k] = relu(W0[k] . d + b0[k]) for the thread's C1 / PARTS output channels
-// (weights from the parameter space: uniform operands), split to bf16 hi / lo and stored as 16-byte chunks of the
-// swizzled A operand atom.
+// (weights from the parameter space: uniform operands), split to bf16 hi / lo (or rounded to tf32) and stored as
+// 16-byte chunks of the swizzled A operand atom.
 template <int NPASS, int C1, int PARTS>
 __device__ __forceinline__ void xyz_first_layer(const Args &a, int part, float dx, float dy, float dz, bool valid, int rl,
                                                 uint32_t A_hi, uint32_t A_lo) {
@@ -160,6 +167,17 @@ __device__ __forceinline__ void xyz_first_layer(const Args &a, int part, float d
             // same operation order as the FP32 level-1 kernel (dense_relu_c): ((b + dx w0) + dy w1) + dz w2
             const float v = fmaf(dz, a.w0c[k * 3 + 2], fmaf(dy, a.w0c[k * 3 + 1], fmaf(dx, a.w0c[k * 3], a.b0c[k])));
             x[j] = valid ? fmaxf(v, 0.f) : 0.f;
+        }
+        if (NPASS == 2) {   // C1 <= 32: image 0 only, 4 k per 16 bytes
+#pragma unroll
+            for (int h = 0; h < 2; ++h) {
+                const int j16 = (part * NC + c8 * 8) / 4 + h;
+                const uint32_t off = rl * 128 + ((j16 ^ (rl & 7)) << 4);
+                asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(A_hi + off), "r"(tf32_rna_bits((x[4 * h]))),
+                             "r"(tf32_rna_bits((x[4 * h + 1]))), "r"(tf32_rna_bits((x[4 * h + 2]))),
+                             "r"(tf32_rna_bits((x[4 * h + 3]))));
+            }
+            continue;
         }
         const int j16 = (part * NC) / 8 + c8;
         const uint32_t off = rl * 128 + ((j16 ^ (rl & 7)) << 4);
@@ -260,7 +278,8 @@ __global__ void __launch_bounds__((NW + 2) * 32, NW == 4 ? 2 : 1) sa_mlp2_kernel
                     for (int p = 0; p < np; ++p) {
                         const int nch = pass_chunks(bn, p);
                         for (int c = 0; c < kat; ++c)
-                            for (int w = 0; w < IM; ++w)
+                            for (int w = 0; w < IM; ++w) {
+                                if (!image_used<NPASS>(gm ? a.c2 : a.c1, c, w)) continue;
                                 for (int nh = 0; nh < nch; ++nh) {
 #ifdef GP_SAF_PROBE
                                     const long long w0 = clock64();
@@ -282,6 +301,7 @@ __global__ void __launch_bounds__((NW + 2) * 32, NW == 4 ? 2 : 1) sa_mlp2_kernel
                                              rows * 128, &full[slot]);
                                     if (++slot == (uint32_t)NST) { slot = 0; ++wrap; }
                                 }
+                            }
                     }
                 }
             }
@@ -296,7 +316,7 @@ __global__ void __launch_bounds__((NW + 2) * 32, NW == 4 ? 2 : 1) sa_mlp2_kernel
         // ---------------- MMA issuer ----------------
         // The whole warp runs this code with identical state; one elected lane issues each MMA / commit (tc_ptx.cuh).
         {
-            const uint32_t a_hi = abuf_a, a_lo = abuf_a + (NPASS == 3 ? k1 * ATOM : 0);
+            const uint32_t a_hi = abuf_a, a_lo = abuf_a + (NPASS != 1 ? k1 * ATOM : 0);
             const uint32_t ring_a = smem_u32(ring);
             uint32_t slot = 0, fph = 0;     // ring position of the next entry to consume, parity of its `full` barrier
             uint32_t ph_a = 0, ph_e1 = 0, ph_p = 0;
@@ -314,12 +334,42 @@ __global__ void __launch_bounds__((NW + 2) * 32, NW == 4 ? 2 : 1) sa_mlp2_kernel
                 return ring_a + sl * SLOT;
             };
             // one accumulator pass: kat k-atoms, one or two chunks of <= 128 columns (two chunks = two interleaved chains)
-            // `kdim`: the populated K (c1 / c2 rounded up to 16): the last k-atom multiplies only its populated 16-wide steps
+            // `kdim`: the populated K (c1 / c2): the last k-atom multiplies only its populated 16-wide (tf32: 8-wide) steps
             auto pass = [&](const bool second, const int kat, const int kdim, const int bn, const int p) {
                 const bool two = pass_chunks(bn, p) == 2;
-                const uint32_t id0 = make_idesc_bf16(128, (uint32_t)chunk_rows(bn, p, 0));
-                const uint32_t id1 = two ? make_idesc_bf16(128, (uint32_t)chunk_rows(bn, p, 1)) : id0;
+                const uint32_t id0 = NPASS == 2 ? make_idesc_tf32(128, (uint32_t)chunk_rows(bn, p, 0))
+                                                : make_idesc_bf16(128, (uint32_t)chunk_rows(bn, p, 0));
+                const uint32_t id1 = two ? (NPASS == 2 ? make_idesc_tf32(128, (uint32_t)chunk_rows(bn, p, 1))
+                                                       : make_idesc_bf16(128, (uint32_t)chunk_rows(bn, p, 1))) : id0;
                 const uint32_t d0 = tmem + dcol, d1 = d0 + 128;
+                if (NPASS == 2) {
+                    // image w of atom c: k 64 c + 32 w .. +31; A from the A buffer's image or from H's columns k
+                    for (int c = 0; c < kat; ++c)
+                        for (int w = 0; w < 2; ++w) {
+                            if (!image_used<NPASS>(kdim, c, w)) break;
+                            uint32_t s0 = 0, s1 = 0, b0, b1 = 0;
+                            b0 = take(s0);
+                            if (two) b1 = take(s1);
+                            tc_fence_after();
+                            const int k0 = 64 * c + 32 * w;
+                            const int nk = min(4, (kdim - k0 + 7) >> 3);
+                            for (int kk = 0; kk < nk; ++kk) {
+                                const uint32_t accum = (c | w | kk) ? 1u : 0u;
+                                if (second) {
+                                    const uint32_t ah = h_hi + k0 + kk * 8;
+                                    umma_tf32_ts_w(d0, ah, make_desc(b0 + kk * 32), id0, accum);
+                                    if (two) umma_tf32_ts_w(d1, ah, make_desc(b1 + kk * 32), id1, accum);
+                                } else {
+                                    const uint64_t ad = make_desc((w ? a_lo : a_hi) + c * ATOM + kk * 32);
+                                    umma_tf32_ss_w(d0, ad, make_desc(b0 + kk * 32), id0, accum);
+                                    if (two) umma_tf32_ss_w(d1, ad, make_desc(b1 + kk * 32), id1, accum);
+                                }
+                            }
+                            umma_commit_w(&empty[s0]);
+                            if (two) umma_commit_w(&empty[s1]);
+                        }
+                    return;
+                }
                 for (int c = 0; c < kat; ++c) {
                     uint32_t s0 = 0, s1 = 0, b0, b1 = 0;
 #ifdef GP_SAF_PROBE
@@ -390,14 +440,14 @@ __global__ void __launch_bounds__((NW + 2) * 32, NW == 4 ? 2 : 1) sa_mlp2_kernel
 #endif
                 for (int p = 0; p < np1; ++p) {
                     if (p > 0) { mbar_wait(e1_done, ph_e1); ph_e1 ^= 1; tc_fence_after(); }   // accumulators read out
-                    pass(false, k1, round16(a.c1), bn1, p);
+                    pass(false, k1, a.c1, bn1, p);
                     umma_commit_w(d1bar);
                 }
                 mbar_wait(e1_done, ph_e1); ph_e1 ^= 1;     // H is complete in TMEM, accumulators free
                 tc_fence_after();
                 for (int q = 0; q < np2; ++q) {
                     if (q > 0) { mbar_wait(p_done, ph_p); ph_p ^= 1; tc_fence_after(); }
-                    pass(true, k2, bn1, bn2, q);
+                    pass(true, k2, a.c2, bn2, q);
                     umma_commit_w(d2bar);
                 }
                 mbar_wait(p_done, ph_p); ph_p ^= 1;        // last pass pooled: accumulators free for the next tile
@@ -418,7 +468,7 @@ __global__ void __launch_bounds__((NW + 2) * 32, NW == 4 ? 2 : 1) sa_mlp2_kernel
         const int half = e >> 2;                   // which 32-column groups (odd / even)
         const int row = 32 * quarter + lane;       // epilogue row
         const uint32_t lane_addr = tmem + ((uint32_t)(32 * quarter) << 16);
-        const uint32_t A_hi = abuf_a, A_lo = abuf_a + (NPASS == 3 ? k1 * ATOM : 0);
+        const uint32_t A_hi = abuf_a, A_lo = abuf_a + (NPASS != 1 ? k1 * ATOM : 0);
         const int jv = w & 15;                     // float4 inside a 64-float chunk
         const int rsub = w >> 4;                   // row inside a pass
         const int ns = a.pool_ns;
@@ -494,6 +544,17 @@ __global__ void __launch_bounds__((NW + 2) * 32, NW == 4 ? 2 : 1) sa_mlp2_kernel
                                     fmaxf(pv[c][0].z - qv[c][0].z, 0.f), fmaxf(pv[c][0].w - qv[c][0].w, 0.f),
                                     fmaxf(pv[c][1].x - qv[c][1].x, 0.f), fmaxf(pv[c][1].y - qv[c][1].y, 0.f),
                                     fmaxf(pv[c][1].z - qv[c][1].z, 0.f), fmaxf(pv[c][1].w - qv[c][1].w, 0.f)};
+                if (NPASS == 2) {   // column col = part NCH 8 + 8 c + 4 h: image col / 32, 16-byte unit (col % 32) / 4
+#pragma unroll
+                    for (int h = 0; h < 2; ++h) {
+                        const int col = (part * NCH + c) * 8 + 4 * h;
+                        const uint32_t off = (col >> 5) * (k1 * ATOM) + rl * 128 + ((((col & 31) >> 2) ^ (rl & 7)) << 4);
+                        asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(A_hi + off), "r"(tf32_rna_bits((x[4 * h]))),
+                                     "r"(tf32_rna_bits((x[4 * h + 1]))), "r"(tf32_rna_bits((x[4 * h + 2]))),
+                                     "r"(tf32_rna_bits((x[4 * h + 3]))));
+                    }
+                    continue;
+                }
                 const int j16 = part * NCH + c;
                 const uint32_t off = rl * 128 + ((j16 ^ (rl & 7)) << 4);
                 uint32_t hi[4], lo[4];
@@ -548,9 +609,15 @@ __global__ void __launch_bounds__((NW + 2) * 32, NW == 4 ? 2 : 1) sa_mlp2_kernel
 #pragma unroll
                     for (int p = 0; p < 8; ++p) {
                         const int rl = rsub + RSTEP * (pb + p);
-                        const uint32_t off = kc * ATOM + rl * 128 + (((jv >> 1) ^ (rl & 7)) << 4) + ((jv & 1) << 3);
                         const float x0 = fmaxf(pv[p].x - qv[p].x, 0.f), x1 = fmaxf(pv[p].y - qv[p].y, 0.f);
                         const float x2 = fmaxf(pv[p].z - qv[p].z, 0.f), x3 = fmaxf(pv[p].w - qv[p].w, 0.f);
+                        if (NPASS == 2) {   // k 4 jv .. 4 jv + 3 of the atom: image jv / 8, 16-byte unit jv % 8
+                            const uint32_t toff = (jv >> 3) * (k1 * ATOM) + kc * ATOM + rl * 128 + (((jv & 7) ^ (rl & 7)) << 4);
+                            asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(A_hi + toff), "r"(tf32_rna_bits((x0))),
+                                         "r"(tf32_rna_bits((x1))), "r"(tf32_rna_bits((x2))), "r"(tf32_rna_bits((x3))));
+                            continue;
+                        }
+                        const uint32_t off = kc * ATOM + rl * 128 + (((jv >> 1) ^ (rl & 7)) << 4) + ((jv & 1) << 3);
                         const __nv_bfloat162 h0 = __floats2bfloat162_rn(x0, x1), h1 = __floats2bfloat162_rn(x2, x3);
                         asm volatile("st.shared.v2.b32 [%0], {%1, %2};" ::"r"(A_hi + off), "r"(*reinterpret_cast<const uint32_t *>(&h0)),
                                      "r"(*reinterpret_cast<const uint32_t *>(&h1)));
@@ -591,6 +658,22 @@ __global__ void __launch_bounds__((NW + 2) * 32, NW == 4 ? 2 : 1) sa_mlp2_kernel
                 lap(2);
                 const int g_lo = p * DN / 32, g_hi = min(2 * k2, (p + 1) * DN / 32);
                 for (int g = g_lo + half; g < g_hi; g += HALVES) {
+                    if (NPASS == 2) {   // tf32: H column k = n, 32 columns per group
+                        uint32_t r[32];
+                        if (g * 32 < bn1) {
+                            tmem_ld32(lane_addr + dcol + (g * 32 - p * DN), r);
+#pragma unroll
+                            for (int j = 0; j < 32; ++j) {
+                                const int n = g * 32 + j;
+                                r[j] = n < a.c2 ? tf32_rna_bits((fmaxf(__uint_as_float(r[j]) + b1p[n], 0.f))) : 0u;
+                            }
+                        } else {
+#pragma unroll
+                            for (int j = 0; j < 32; ++j) r[j] = 0u;
+                        }
+                        tmem_st32(lane_addr + (uint32_t)(g * 32), r);
+                        continue;
+                    }
                     uint32_t hi[16], lo[16];
                     if (g * 32 < bn1) {
                         uint32_t r[32];
@@ -721,11 +804,15 @@ static int launch(Args a, cudaStream_t st) {
 
 using namespace gp;
 
+static int launch_npass(const saf::Args &a, int npass, cudaStream_t st) {
+    return npass == 3 ? saf::launch<3>(a, st) : npass == 2 ? saf::launch<2>(a, st) : saf::launch<1>(a, st);
+}
+
 extern "C" int gp_sa_mlp2_fused(const float *P, int n_src, int ldp, const int32_t *gidx, long long R, int rows_per_batch,
                                 const float *Q, int ldq, int q_ns, const void *packed1, const float *bias1, int c1, int c2,
                                 const void *packed2, const float *bias2, int c3, int npass, int pool_ns, float *pooled,
                                 int ld_pooled, gp_stream_t s) {
-    GP_REQUIRE(R >= 0 && (npass == 1 || npass == 3), "gp_sa_mlp2_fused: bad arguments");
+    GP_REQUIRE(R >= 0 && npass >= 1 && npass <= 3, "gp_sa_mlp2_fused: bad arguments (npass must be 1, 2 or 3)");
     if (R == 0) return GP_OK;
     GP_REQUIRE(P && gidx && Q && packed1 && bias1 && packed2 && bias2 && pooled, "gp_sa_mlp2_fused: null pointer");
     GP_REQUIRE(c1 >= 4 && c1 <= 256 && (c1 & 3) == 0 && c2 >= 1 && c2 <= 384 && c3 >= 1 && c3 <= 512,
@@ -745,14 +832,14 @@ extern "C" int gp_sa_mlp2_fused(const float *P, int n_src, int ldp, const int32_
     a.pool_ns = pool_ns; a.pooled = pooled; a.ld_pooled = ld_pooled;
     a.ntiles = (int)((R + saf::BM - 1) / saf::BM);
     a.xyz = nullptr; a.centres = nullptr;
-    return npass == 3 ? saf::launch<3>(a, as_stream(s)) : saf::launch<1>(a, as_stream(s));
+    return launch_npass(a, npass, as_stream(s));
 }
 
 extern "C" int gp_sa_mlp2_fused_xyz(const float *xyz, const float *centres, int n_src, const int32_t *gidx, long long R,
                                     int rows_per_batch, int q_ns, const float *host_W0, const float *host_b0, const void *packed1,
                                     const float *bias1, int c1, int c2, const void *packed2, const float *bias2, int c3, int npass,
                                     int pool_ns, float *pooled, int ld_pooled, gp_stream_t s) {
-    GP_REQUIRE(R >= 0 && (npass == 1 || npass == 3), "gp_sa_mlp2_fused_xyz: bad arguments");
+    GP_REQUIRE(R >= 0 && npass >= 1 && npass <= 3, "gp_sa_mlp2_fused_xyz: bad arguments (npass must be 1, 2 or 3)");
     if (R == 0) return GP_OK;
     GP_REQUIRE(xyz && centres && gidx && host_W0 && host_b0 && packed1 && bias1 && packed2 && bias2 && pooled, "gp_sa_mlp2_fused_xyz: null pointer");
     GP_REQUIRE((c1 == 16 || c1 == 32) && c2 >= 1 && c2 <= 384 && c3 >= 1 && c3 <= 512,
@@ -774,5 +861,5 @@ extern "C" int gp_sa_mlp2_fused_xyz(const float *xyz, const float *centres, int 
         a.b0c[k] = k < c1 ? host_b0[k] : 0.f;
         for (int d = 0; d < 3; ++d) a.w0c[k * 3 + d] = k < c1 ? host_W0[k * 3 + d] : 0.f;
     }
-    return npass == 3 ? saf::launch<3>(a, as_stream(s)) : saf::launch<1>(a, as_stream(s));
+    return launch_npass(a, npass, as_stream(s));
 }

@@ -101,6 +101,23 @@ __device__ __forceinline__ void umma_tf32_ts_w(uint32_t d_tmem, uint32_t a_tmem,
         "@q tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}"
         ::"r"(d_tmem), "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
 }
+// D[tmem] (+)= A[smem] * B[smem]^T, tf32 x tf32 -> f32, K = 8: both operands are [rows][32 k] fp32 images, K-major
+// SWIZZLE_128B; a K = 8 step advances both descriptors by 32 bytes, as a K = 16 bf16 step does
+__device__ __forceinline__ void umma_tf32_ss(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
+        ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
+}
+__device__ __forceinline__ void umma_tf32_ss_w(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p, q;\n\t"
+        "elect.sync _|q, 0xffffffff;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "@q tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
+        ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
+}
 // fp32 -> tf32 operand value: round to nearest on the 13 dropped significand bits, ties away from zero (the MMA itself
 // would truncate them)
 __device__ __forceinline__ float tf32_rna(float x) {
@@ -108,6 +125,12 @@ __device__ __forceinline__ float tf32_rna(float x) {
     asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
     return __uint_as_float(r);
 }
+// The same rounding as an MMA operand, in one integer add: kind::tf32 ignores the 13 low significand bits of an operand,
+// so adding half of their range to the magnitude bits before the MMA truncates them rounds to nearest, ties away from
+// zero -- what the MMA then reads equals cvt.rna.tf32.f32 for every finite x (a value that rounds past the largest
+// float becomes inf, as with cvt.rna).  cvt.rna has no packed form and costs several integer instructions per value;
+// the loaders and the hidden-layer epilogue of the encoder's GEMMs are issue bound.
+__device__ __forceinline__ uint32_t tf32_rna_bits(float x) { return __float_as_uint(x) + 0x1000u; }
 __device__ __forceinline__ void umma_commit_w(unsigned long long *bar) {
     asm volatile(
         "{\n\t.reg .pred q;\n\t"
@@ -172,7 +195,17 @@ __device__ __forceinline__ void tmem_ld_16x256b_x4_nowait(uint32_t taddr, uint32
         : "r"(taddr) : "memory");
 }
 
-// registers -> TMEM: this thread's lane, 16 / 8 consecutive 32-bit columns starting at taddr (warp-collective)
+// registers -> TMEM: this thread's lane, 32 / 16 / 8 consecutive 32-bit columns starting at taddr (warp-collective)
+__device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t (&v)[32]) {
+    asm volatile(
+        "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
+        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
+        "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
+        ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]),
+          "r"(v[8]), "r"(v[9]), "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15]),
+          "r"(v[16]), "r"(v[17]), "r"(v[18]), "r"(v[19]), "r"(v[20]), "r"(v[21]), "r"(v[22]), "r"(v[23]),
+          "r"(v[24]), "r"(v[25]), "r"(v[26]), "r"(v[27]), "r"(v[28]), "r"(v[29]), "r"(v[30]), "r"(v[31]) : "memory");
+}
 __device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&v)[16]) {
     asm volatile(
         "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "

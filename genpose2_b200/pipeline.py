@@ -49,20 +49,23 @@ def gather_results(pose, length, group=None):
 class PosePipeline:
     """score + energy + scale agents wired together; every stage runs on libgenpose_b200.so."""
 
-    def __init__(self, cfg=None, device="cuda", mlp_mode="fp32", use_graph=False, step_control="batch"):
+    def __init__(self, cfg=None, device="cuda", mlp_mode="fp32", use_graph=False, step_control="batch", encoder_mode="auto"):
         """use_graph: replay the whole step as ONE CUDA graph per input signature (batch size, points, hypotheses, T0 --
         or "per-object T0", whatever the values --, warm start and noise keys present or not):
         ~80 kernel launches, the two-stream fork / join and the cooperative sampler launch become one graph launch; the
         only host work left per step is drawing the prior noise with the CPU generator (exactly like the reference,
         sde.py:34) and one pinned upload.  The captured graph bakes in the packed weights: load_state_dicts() drops it.
         step_control: "batch" (the reference's RK45 controller over the whole batch) or "object" (every object integrated
-        as if it were alone: its poses do not depend on the other objects of the step), see samplers.STEP_CONTROLS."""
+        as if it were alone: its poses do not depend on the other objects of the step), see samplers.STEP_CONTROLS.
+        encoder_mode: operand precision of both point-cloud encoders' SharedMLP GEMMs, "auto" (follows mlp_mode),
+        "bf16x3", "tf32" or "bf16", see posenet.ENCODER_MODES."""
         from .samplers import check_step_control
         check_step_control(step_control)
         cfg = copy.copy(cfg) if cfg is not None else get_config()
         cfg.device = device
         cfg.mlp_mode = mlp_mode
         cfg.step_control = step_control
+        cfg.encoder_mode = encoder_mode
         if not getattr(cfg, "sampler_mode", None):
             cfg.sampler_mode = ["ode"]
         self.cfg = cfg

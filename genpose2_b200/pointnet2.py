@@ -16,7 +16,7 @@ The per-scale SharedMLP (conv1x1 + BatchNorm(eval) + ReLU, pytorch_utils.py:5-33
 section 8: BatchNorm is folded into the weights once per checkpoint, activations are channels-last (one GEMM
 row per sample) and every layer runs on the tcgen05 kernels of libgenpose_b200.so (csrc/gemm_tc.cu,
 csrc/sa_fused.cu; level 1 on the FP32 kernel of csrc/pointnet2.cu).  There is no library-GEMM backend:
-`gemm_mode` only selects the operand precision ("bf16x3" = split-bf16 x3, fp32-class; "bf16").
+`gemm_mode` only selects the operand precision, see GEMM_NPASS.
 """
 from typing import List, Optional
 
@@ -24,6 +24,10 @@ import torch
 import torch.nn as nn
 
 from . import pointnet2_utils as pu
+
+# operand precision of the tensor-core SharedMLP GEMMs -> the kernels' npass: "bf16x3" = split-bf16 x3 (fp32-class),
+# "tf32" = tcgen05 kind::tf32 with operands rounded to nearest tf32, "bf16" = bf16 operands
+GEMM_NPASS = {"bf16x3": 3, "tf32": 2, "bf16": 1}
 
 ClsMSG_CFG_Light = {
     "NPOINTS": [512, 256, 128, 64, None],
@@ -84,7 +88,7 @@ class SharedMLP(nn.Module):
         self.forward_rows_pooled(rows.contiguous(), B * M, ns, out, self.gemm_mode)
         return out.view(B, M, -1).permute(0, 2, 1).contiguous()
 
-    gemm_mode = "bf16x3"   # operand precision of the tensor-core GEMMs: "bf16x3" (fp32-class) | "bf16"
+    gemm_mode = "bf16x3"   # operand precision of the tensor-core GEMMs: a key of GEMM_NPASS
 
     _trusted = False  # set by Pointnet2ClsMSG.forward for the duration of one pass, after it has checked the cache
 
@@ -157,7 +161,7 @@ class SharedMLP(nn.Module):
         (centre, sample) activation matrix of the reference (pointnet2_utils.py:279-296) never exists in HBM --
         the second layer's operand loader gathers the per-point rows by ball-query index, subtracts the per-centre
         term and applies the ReLU on the fly.  pts_rows = [feat | xyz | 0-pad] per point, [B*n_src, ld]."""
-        npass = {"bf16x3": 3, "bf16": 1}[gemm_mode]
+        npass = GEMM_NPASS[gemm_mode]
         t = self._tc_hoisted(npass)
         B, M, ns = bq_idx.shape
         P = pu.gemm_linear(pts_rows, t["p0"], t["c1"], t["k0"], npass)                 # [B*n_src, ldp]
@@ -167,7 +171,7 @@ class SharedMLP(nn.Module):
     def hoisted_tail(self, P, Q, n_src, bq_idx, out, gemm_mode):
         """Layers 2, 3 and the max-pool of forward_hoisted, given the per-point table P and the per-centre term Q
         (both may be column slices of tables shared by the scales of a level)."""
-        npass = {"bf16x3": 3, "bf16": 1}[gemm_mode]
+        npass = GEMM_NPASS[gemm_mode]
         t = self._tc_hoisted(npass)
         B, M, ns = bq_idx.shape
         if pu.sa_mlp2_fused_fits(t["c1"], t["c2"], t["c3"], npass, ns):
@@ -182,9 +186,9 @@ class SharedMLP(nn.Module):
 
     def forward_rows_pooled(self, rows, groups, nsample, out, gemm_mode, feat_first=False, zeroed=False):
         """rows (R, ld) -> SharedMLP -> max over `nsample` rows per group, written into `out` (groups, Cout).
-        gemm_mode: "bf16x3" (tcgen05, split-bf16, fp32-class) or "bf16" (tcgen05).
+        gemm_mode: a key of GEMM_NPASS (tcgen05 operand precision).
         feat_first: the rows are [feat | xyz | 0] (the encoder's level buffers) instead of [xyz | feat]."""
-        npass = {"bf16x3": 3, "bf16": 1}[gemm_mode]
+        npass = GEMM_NPASS[gemm_mode]
         layers = self._tc_layers_featfirst(npass) if feat_first else self._tc_layers(npass)
         h = rows
         for i, (packed, b, N, K) in enumerate(layers):
@@ -203,7 +207,7 @@ class PointnetSAModuleMSG(nn.Module):
     def __init__(self, *, npoint, radii, nsamples, mlps):
         super().__init__()
         self.npoint, self.radii, self.nsamples = npoint, radii, nsamples
-        self.gemm_mode = "bf16x3"  # "bf16x3" | "bf16" (see SharedMLP.forward_rows_pooled)
+        self.gemm_mode = "bf16x3"  # a key of GEMM_NPASS (see SharedMLP.forward_rows_pooled)
         # feature-less scales (first level) that take the fused tensor-core kernel instead of the FP32 kernel
         self.level1_tc_specs = ((32, 32, 64),)
         self.groupers = nn.ModuleList(
@@ -293,7 +297,7 @@ class PointnetSAModuleMSG(nn.Module):
                                           torch.zeros((B, N, 1), dtype=torch.float32, device=xyz.device)],
                                          dim=-1).reshape(B * N, -1)
                 if all(m.n_layers == 3 for m in self.mlps):
-                    npass = {"bf16x3": 3, "bf16": 1}[self.gemm_mode]
+                    npass = GEMM_NPASS[self.gemm_mode]
                     mf = self._merged_first_layer(npass)
                     if mf is not None:
                         P_all = pu.gemm_linear(pts_rows, mf["p0"], mf["n"], mf["k0"], npass)
@@ -315,10 +319,10 @@ class PointnetSAModuleMSG(nn.Module):
                     continue
                 spec = tuple(getattr(mlp, f"layer{j}").conv.out_channels for j in range(mlp.n_layers))
                 if (feat_cl is None and tc and self.nsamples[i] in (16, 32) and spec in self.level1_tc_specs
-                        and pu.sa_mlp2_fused_fits(*spec, {"bf16x3": 3, "bf16": 1}[self.gemm_mode], self.nsamples[i])):
+                        and pu.sa_mlp2_fused_fits(*spec, GEMM_NPASS[self.gemm_mode], self.nsamples[i])):
                     # first level, wide scale: layers 2, 3 and the max-pool on the tensor cores, the K = 3 first layer
                     # evaluated in the fused kernel's operand loader
-                    npass = {"bf16x3": 3, "bf16": 1}[self.gemm_mode]
+                    npass = GEMM_NPASS[self.gemm_mode]
                     t = mlp._tc_hoisted(npass)
                     w0, b0 = mlp._folded_layers_host()[0]
                     pu.sa_mlp2_fused_xyz(xyz, new_xyz, bq[i], w0, b0, t["p1"], t["b1"], t["c1"], t["c2"], t["p2"], t["b2"],
@@ -359,7 +363,7 @@ class PointnetSAModuleMSG(nn.Module):
             gm = self.gemm_mode
         out = pu.zeros((B, 1, C), xyz.device)   # the pooled GEMMs take the max into a zero-initialised output
         off = 0
-        npass = {"bf16x3": 3, "bf16": 1}[gm]
+        npass = GEMM_NPASS[gm]
         mg = self._merged_groupall_first(npass, feat_first)
         if mg is not None:
             # the scales read the same rows: their first layers are ONE GEMM (weights stacked along the output channels,
@@ -396,8 +400,8 @@ class Pointnet2ClsMSG(nn.Module):
 
     def set_gemm_mode(self, mode):
         """Operand precision of the tensor-core SharedMLP GEMMs for every level: "bf16x3" (split-bf16 x3,
-        fp32-class accuracy) or "bf16"."""
-        if mode not in ("bf16x3", "bf16"):
+        fp32-class accuracy), "tf32" (tf32 operands, rounded to nearest) or "bf16"."""
+        if mode not in GEMM_NPASS:
             raise ValueError(mode)
         for sa in self.SA_modules:
             sa.gemm_mode = mode

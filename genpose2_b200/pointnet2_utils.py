@@ -238,8 +238,9 @@ def zeros(shape, device):
 
 
 def gemm_pack(weight: torch.Tensor, npass: int) -> torch.Tensor:
-    """Pack W [N, K] fp32 into the pre-swizzled bf16 (npass=1) / bf16 hi+lo (npass=3) chunk images the
-    tcgen05 GEMM streams with TMA (gp_gemm_pack).  Do once per checkpoint."""
+    """Pack W [N, K] fp32 into the pre-swizzled bf16 (npass=1) / bf16 hi+lo (npass=3) / tf32 k 0..31 + k 32..63
+    (npass=2, rounded to nearest tf32) chunk images the tcgen05 GEMM streams with TMA (gp_gemm_pack).  Do once per
+    checkpoint."""
     w = _lib.check_cuda(weight.detach().to(torch.float32).contiguous(), "weight", torch.float32)
     N, K = w.shape
     nbytes = _lib.load().gp_gemm_packed_bytes(N, K, npass)
@@ -351,11 +352,12 @@ def sa_mlp2_fused_xyz(xyz, new_xyz, bq_idx, w0, b0, packed1, bias1, c1, c2, pack
 
 def sa_mlp2_fused_fits(c1, c2, c3, npass, pool_ns):
     """Shapes the fused kernel takes (the plan of csrc/sa_fused.cu): H = relu(layer 2) lives in tensor memory as packed
-    bf16 (32 columns per 64-wide k-atom, hi + lo in split mode) next to at least 128 accumulator columns, and the
-    gathered A operand plus a ring of at least two weight chunks (hi + lo) must fit in shared memory."""
+    bf16 (32 columns per 64-wide k-atom, hi + lo in split mode; tf32: 64 columns per k-atom) next to at least 128
+    accumulator columns, and the gathered A operand plus a ring of at least two weight chunks (hi + lo, or the two tf32
+    images) must fit in shared memory."""
     if c1 % 4 or c1 > 256 or c2 > 384 or c3 > 512 or pool_ns not in (8, 16, 32):
         return False
-    images = 2 if npass == 3 else 1
+    images = 1 if npass == 1 else 2
     if 512 - ((c2 + 63) // 64) * 32 * images < 128:
         return False
     return images * ((c1 + 63) // 64) * 16384 + 2 * images * 16384 + 2048 + 1536 <= 227 * 1024

@@ -6,15 +6,30 @@ raises NotImplementedError (no fallback / multi-backend dispatch)."""
 import torch
 import torch.nn as nn
 
-from .pointnet2 import Pointnet2ClsMSG
+from .pointnet2 import GEMM_NPASS, Pointnet2ClsMSG
 from .samplers import cond_ode_sampler, cond_pc_sampler
 from .scorenet import PoseEnergyNet, PoseScoreNet
+
+# cfg.encoder_mode: "auto" or a SharedMLP operand precision (pointnet2.GEMM_NPASS).  "auto" follows mlp_mode: fp32,
+# fp32_ffma and tf32 -> split-bf16 x3 (fp32-class, 2e-5 of the reference's fp32 features; mlp_mode tf32 runs only the
+# trunk in tf32), bf16 -> bf16
+ENCODER_MODES = ("auto",) + tuple(GEMM_NPASS)
+_AUTO_ENCODER_MODE = {"fp32": "bf16x3", "fp32_ffma": "bf16x3", "tf32": "bf16x3", "bf16": "bf16"}
+
+
+def encoder_gemm_mode(cfg):
+    """The encoder's SharedMLP operand precision for cfg (ValueError for an unknown encoder_mode)."""
+    mode = getattr(cfg, "encoder_mode", "auto")
+    if mode not in ENCODER_MODES:
+        raise ValueError(f"encoder_mode={mode!r}: expected one of {ENCODER_MODES}")
+    return _AUTO_ENCODER_MODE[getattr(cfg, "mlp_mode", "fp32")] if mode == "auto" else mode
 
 
 class GFObjectPose(nn.Module):
     def __init__(self, cfg, prior_fn, marginal_prob_fn, sde_fn, sampling_eps, T):
         super().__init__()
         self.cfg = cfg
+        encoder_mode = encoder_gemm_mode(cfg)
         self.device = cfg.device
         self.is_testing = False
         self.prior_fn, self.marginal_prob_fn, self.sde_fn = prior_fn, marginal_prob_fn, sde_fn
@@ -28,11 +43,7 @@ class GFObjectPose(nn.Module):
         if getattr(cfg, "pointnet2_params", "light") != "light":
             raise NotImplementedError("pointnet2_params=%r: only 'light' (ClsMSG_CFG_Light)" % cfg.pointnet2_params)
         self.pts_encoder = Pointnet2ClsMSG(0)
-        # SharedMLP operand precision: fp32 mode -> split-bf16 x3 on tcgen05 (fp32-class accuracy, 2e-5 of the
-        # reference's fp32 features), bf16 mode -> bf16 on tcgen05; tf32 mode keeps the encoder fp32-class (the trunk only
-        # runs in tf32)
-        self.pts_encoder.set_gemm_mode({"fp32": "bf16x3", "fp32_ffma": "bf16x3", "tf32": "bf16x3", "bf16": "bf16"}[
-            getattr(cfg, "mlp_mode", "fp32")])
+        self.pts_encoder.set_gemm_mode(encoder_mode)
         if cfg.agent_type == "score":
             self.pose_score_net = PoseScoreNet(self.marginal_prob_fn, 0, cfg.pose_mode, cfg.regression_head, False)
         elif cfg.agent_type == "energy":

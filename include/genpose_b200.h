@@ -145,7 +145,10 @@ GP_API int gp_zero(void *dst, size_t bytes, gp_stream_t s);
  * rows, on the tcgen05 tensor cores: Y = relu(X . W^T + bias), optionally fused with the max-pool over
  * `pool_ns` consecutive rows (P2/pointnet2_modules.py:59-61).
  *   npass = 1: bf16 operands (bf16 mode);  npass = 3: fp32 values split into hi + lo bf16 and accumulated
- *   as hi*hi + lo*hi + hi*lo (16 mantissa bits per operand, fp32 accumulation) -- the fp32-mode path.
+ *   as hi*hi + lo*hi + hi*lo (16 mantissa bits per operand, fp32 accumulation) -- the fp32-mode path;
+ *   npass = 2: tf32 operands (both rounded to nearest tf32, 11 significand bits; tcgen05 kind::tf32, fp32
+ *   accumulation), packed to the same size as npass = 3.  Other values: GP_ERR_BAD_ARG (gp_gemm_packed_bytes
+ *   returns 0).  The same npass values hold for gp_gemm_linear, gp_gemm_gather_bias_relu and gp_sa_mlp2_fused(_xyz).
  *   W [N,K] fp32 row-major is packed once per checkpoint with gp_gemm_pack (gp_gemm_packed_bytes bytes).
  *   X [R, ldx] fp32, ldx %% 4 == 0, columns K..ldx-1 must be finite (they meet zero weights).
  *   pool_ns == 0: Y [R, ldy] with ldy = round_up(N, 32); columns N..ldy-1 are written as zeros.
