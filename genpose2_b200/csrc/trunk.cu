@@ -1,7 +1,8 @@
 // ScoreNet / EnergyNet trunk kernels: weight packing, per-object head projection, single evaluation, energy
 // scoring, the device-resident Dormand-Prince (scipy-RK45-faithful) integrator fused with the ScoreNet RHS (with
 // scipy's dense output), and the fixed-step predictor-corrector sampler.  The MLP evaluation itself is a policy:
-// SimtEval (FP32 FFMA, trunk.cuh) or TcEval (tcgen05, 4-CTA clusters, trunk_tc.cuh).
+// SimtEval (FP32 FFMA, trunk.cuh), TcEval (tcgen05, 4-CTA clusters, trunk_tc.cuh), or TcSoloT / TcSolo (tcgen05, one
+// CTA per tile, trunk_solo_t.cuh / trunk_solo.cuh); with_evaluator() picks one from an entry's `mode`.
 #include <cuda_bf16.h>
 
 #include <cstdlib>
@@ -184,17 +185,32 @@ project_kernel(const float *__restrict__ P, const float *__restrict__ feat, int 
 }
 
 // ------------------------------------------------------------------------------------------
-// Evaluator policies: how one tile of rows gets its f_theta.  SimtEval<RPT>: FP32 FFMA, 4*RPT rows,
-// 256 threads.  TcEval: bf16 tcgen05, 128 rows, 320 threads (trunk_tc.cuh).  Both expose the same
-// shared-memory members (x, out, obj, tq, four, tfeat, times, red) to the integrator code.
+// Evaluator policies: how one tile of rows gets its f_theta.  Every kernel below is a template over one of them, and
+// they all expose the same shared-memory members (x, out, obj, tq, four, tfeat, times, red) to the integrator code.
+//   SimtEval<RPT>    FP32 FFMA, 4*RPT rows, 256 threads, one CTA per tile (trunk.cuh)
+//   TcEval<NPASS>    tcgen05, 128 rows, 320 threads, a 4-CTA cluster per tile (trunk_tc.cuh)
+//   TcSoloT<NPASS>   tcgen05, 128 rows, 320 threads, one CTA per tile, A operand in tensor memory (trunk_solo_t.cuh)
+//   TcSolo<NPASS>    the same with the A operand in shared memory (trunk_solo.cuh)
+// NPASS is the number of MMAs per product: 1 bf16, 2 tf32, 3 split-bf16.  with_evaluator() picks one for an entry.
 // ------------------------------------------------------------------------------------------
+// Tile loop of the evaluators without a cluster: CTA b takes tiles b, b + gridDim.x, ... and stores its own results.
+struct OneCtaPerTile {
+    static constexpr int CLUSTER = 1;     // CTAs that share a tile
+    static __device__ __forceinline__ int tile_first() { return blockIdx.x; }
+    static __device__ __forceinline__ int tile_step() { return gridDim.x; }
+    template <class Ctx>
+    static __device__ __forceinline__ bool writer(const Ctx &) { return true; }
+    template <class Ctx>
+    static __device__ __forceinline__ size_t replica_index(const Ctx &) { return 0; }
+    static __device__ __forceinline__ void tile_sync() {}
+};
+
 template <int RPT>
-struct SimtEval {
+struct SimtEval : OneCtaPerTile {
     static constexpr int RT = 4 * RPT;
     static constexpr int NT = SIMT_THREADS;
     static constexpr int XS = 12;         // row stride of the input / output tile
     static constexpr int TQW = 768;       // t-branch columns held per stage
-    static constexpr int CLUSTER = 1;     // CTAs that share a tile
     using Smem = TileSmem<RPT>;
     using Ctx = SimtCtx;
     static constexpr size_t smem_bytes() { return sizeof(Smem) + 16; }
@@ -202,11 +218,6 @@ struct SimtEval {
         // pointer arithmetic on the __shared__ array keeps the shared address space (LDS/STS, not generic LD/ST)
         return *reinterpret_cast<Smem *>(raw + ((16u - (tc::smem_u32(raw) & 15u)) & 15u));
     }
-    static __device__ __forceinline__ int tile_first() { return blockIdx.x; }
-    static __device__ __forceinline__ int tile_step() { return gridDim.x; }
-    static __device__ __forceinline__ bool writer(const Ctx &) { return true; }
-    static __device__ __forceinline__ size_t replica_index(const Ctx &) { return 0; }
-    static __device__ __forceinline__ void tile_sync() {}
     static __device__ __forceinline__ float *xin(Smem &S) { return S.x; }
     static __device__ __forceinline__ float *outp(Smem &S) { return S.out[0]; }
     static __device__ __forceinline__ float *tq(Smem &S) { return S.tq; }
@@ -266,38 +277,24 @@ struct TcEval {
         if (blockIdx.x == 0 && threadIdx.x == 32) stats[15] = (double)c.cyc_wfull;   // the MMA issuer's own counter
     }
 };
-// One CTA per 128-row tile, no cluster: the throughput shape for batches of more tiles than the GPU has clusters
-// (trunk_solo.cuh).  Same interface; one copy of the integrator state.
-template <int NPASS>
-struct TcSolo {
+
+// One CTA per 128-row tile, no cluster: the throughput shape for batches of more tiles than the GPU has clusters.
+// One copy of the integrator state.  TcSoloT and TcSolo share everything here and differ in where A lives.
+template <class SmemT, class CtxT>
+struct TcSoloTile : OneCtaPerTile {
     static constexpr int RT = tc::RT;
     static constexpr int NT = tc::NTHREADS;
     static constexpr int XS = tc::XS;
     static constexpr int TQW = 768;
-    static constexpr int CLUSTER = 1;
-    using Smem = solo::Smem<NPASS>;
-    using Ctx = solo::State;
+    using Smem = SmemT;
+    using Ctx = CtxT;
     static constexpr size_t smem_bytes() { return sizeof(Smem) + 1024; }
     static __device__ __forceinline__ Smem &smem(unsigned char *raw) {
         return *reinterpret_cast<Smem *>(((uintptr_t)raw + 1023) & ~(uintptr_t)1023);
     }
-    static __device__ __forceinline__ int tile_first() { return blockIdx.x; }
-    static __device__ __forceinline__ int tile_step() { return gridDim.x; }
-    static __device__ __forceinline__ bool writer(const Ctx &) { return true; }
-    static __device__ __forceinline__ size_t replica_index(const Ctx &) { return 0; }
-    static __device__ __forceinline__ void tile_sync() {}
     static __device__ __forceinline__ float *xin(Smem &S) { return S.x; }
     static __device__ __forceinline__ float *outp(Smem &S) { return S.x; }   // forward() overwrites its inputs
     static __device__ __forceinline__ float *tq(Smem &S) { return S.tq; }
-    static __device__ __forceinline__ void setup(Smem &S, Ctx &c, const float *P) { solo::setup<NPASS>(S, c, P); }
-    static __device__ __forceinline__ void teardown(Smem &S, Ctx &c) { solo::teardown<NPASS>(S, c); }
-    static __device__ __forceinline__ void stage_tq(const float *P, Smem &S, Ctx &, int ns) { solo::compute_tq_all<NPASS>(P, S, ns); }
-    static __device__ __forceinline__ void begin_tile(Smem &S, Ctx &c, const float *proj, int r0, int N, int rpo) {
-        solo::begin_tile<NPASS>(S, c, proj, r0, N, rpo);
-    }
-    static __device__ __forceinline__ void forward(const float *P, const float *proj, Smem &S, Ctx &c, const float *tq) {
-        solo::forward<NPASS>(P, proj, S, c, tq);
-    }
     static __device__ __forceinline__ void report(Ctx &c, double *stats) {
         if (blockIdx.x == 0 && threadIdx.x == 64) {
             stats[8] = (double)c.cyc_fwd; stats[9] = (double)c.cyc_l1; stats[10] = (double)c.cyc_wait1;
@@ -306,28 +303,11 @@ struct TcSolo {
         }
     }
 };
-// The same shape with the A operand in tensor memory (trunk_solo_t.cuh).
+// A operand in tensor memory (trunk_solo_t.cuh).
 template <int NPASS>
-struct TcSoloT {
-    static constexpr int RT = tc::RT;
-    static constexpr int NT = tc::NTHREADS;
-    static constexpr int XS = tc::XS;
-    static constexpr int TQW = 768;
-    static constexpr int CLUSTER = 1;
+struct TcSoloT : TcSoloTile<solot::Smem<NPASS>, solot::State> {
     using Smem = solot::Smem<NPASS>;
     using Ctx = solot::State;
-    static constexpr size_t smem_bytes() { return sizeof(Smem) + 1024; }
-    static __device__ __forceinline__ Smem &smem(unsigned char *raw) {
-        return *reinterpret_cast<Smem *>(((uintptr_t)raw + 1023) & ~(uintptr_t)1023);
-    }
-    static __device__ __forceinline__ int tile_first() { return blockIdx.x; }
-    static __device__ __forceinline__ int tile_step() { return gridDim.x; }
-    static __device__ __forceinline__ bool writer(const Ctx &) { return true; }
-    static __device__ __forceinline__ size_t replica_index(const Ctx &) { return 0; }
-    static __device__ __forceinline__ void tile_sync() {}
-    static __device__ __forceinline__ float *xin(Smem &S) { return S.x; }
-    static __device__ __forceinline__ float *outp(Smem &S) { return S.x; }
-    static __device__ __forceinline__ float *tq(Smem &S) { return S.tq; }
     static __device__ __forceinline__ void setup(Smem &S, Ctx &c, const float *P) { solot::setup<NPASS>(S, c, P); }
     static __device__ __forceinline__ void teardown(Smem &S, Ctx &c) { solot::teardown<NPASS>(S, c); }
     static __device__ __forceinline__ void stage_tq(const float *P, Smem &S, Ctx &, int ns) { solot::compute_tq_all<NPASS>(P, S, ns); }
@@ -337,20 +317,30 @@ struct TcSoloT {
     static __device__ __forceinline__ void forward(const float *P, const float *proj, Smem &S, Ctx &c, const float *tq) {
         solot::forward<NPASS>(P, proj, S, c, tq);
     }
-    static __device__ __forceinline__ void report(Ctx &c, double *stats) {
-        if (blockIdx.x == 0 && threadIdx.x == 64) {
-            stats[8] = (double)c.cyc_fwd; stats[9] = (double)c.cyc_l1; stats[10] = (double)c.cyc_wait1;
-            stats[11] = (double)c.cyc_epi1; stats[12] = (double)c.cyc_waith; stats[13] = (double)c.cyc_epi2;
-            stats[20] = (double)c.cyc_tail;
-        }
+};
+// A operand in shared memory (trunk_solo.cuh).
+template <int NPASS>
+struct TcSolo : TcSoloTile<solo::Smem<NPASS>, solo::State> {
+    using Smem = solo::Smem<NPASS>;
+    using Ctx = solo::State;
+    static __device__ __forceinline__ void setup(Smem &S, Ctx &c, const float *P) { solo::setup<NPASS>(S, c, P); }
+    static __device__ __forceinline__ void teardown(Smem &S, Ctx &c) { solo::teardown<NPASS>(S, c); }
+    static __device__ __forceinline__ void stage_tq(const float *P, Smem &S, Ctx &, int ns) { solo::compute_tq_all<NPASS>(P, S, ns); }
+    static __device__ __forceinline__ void begin_tile(Smem &S, Ctx &c, const float *proj, int r0, int N, int rpo) {
+        solo::begin_tile<NPASS>(S, c, proj, r0, N, rpo);
+    }
+    static __device__ __forceinline__ void forward(const float *P, const float *proj, Smem &S, Ctx &c, const float *tq) {
+        solo::forward<NPASS>(P, proj, S, c, tq);
     }
 };
-static_assert(sizeof(solot::Smem<3>) + 1024 + 768 <= 227 * 1024, "solo (TMEM A) evaluator shared memory exceeds 227 KB");
-// static shared memory of the kernels built on the evaluators (stage constants, per-row t) must fit beside it
-static_assert(sizeof(solo::Smem<3>) + 1024 + 768 <= 227 * 1024, "solo evaluator shared memory exceeds 227 KB");
-static_assert(sizeof(solo::Smem<1>) + 1024 + 768 <= 227 * 1024, "solo evaluator shared memory exceeds 227 KB");
-static_assert(sizeof(tc::Smem<3>) + 1024 <= 227 * 1024, "TC evaluator shared memory exceeds 227 KB");
-static_assert(sizeof(tc::Smem<1>) + 1024 <= 227 * 1024, "TC evaluator shared memory exceeds 227 KB");
+
+// Each evaluator's dynamic shared memory leaves room for the static shared memory of the kernels built on it (stage
+// constants, per-row t) in the 227 KB of a CTA.
+template <class... EV>
+constexpr bool smem_fits() { return ((EV::smem_bytes() + 768 <= 227 * 1024) && ...); }
+static_assert(smem_fits<SimtEval<2>, SimtEval<4>, SimtEval<6>, SimtEval<8>, TcEval<1>, TcEval<2>, TcEval<3>, TcSoloT<1>,
+                        TcSoloT<2>, TcSoloT<3>, TcSolo<1>, TcSolo<3>>(),
+              "evaluator shared memory exceeds 227 KB");
 static_assert(sizeof(solot::Smem<2>) == sizeof(solot::Smem<3>) && sizeof(tc::Smem<2>) == sizeof(tc::Smem<3>),
               "tf32 mode uses the split mode's ring");
 
@@ -1488,7 +1478,7 @@ __global__ void __launch_bounds__(EV::NT, 1) pc_kernel(PcArgs a) {
 // Launch `kern` over tiles: `tiles` CTAs (evaluators without clusters) or `tiles` clusters of EV::CLUSTER CTAs.
 // Cooperative launches are clamped to what can be co-resident (tiles are then strided); returns the error code.
 template <class EV, class Kern, class Args>
-static int launch_tiles(Kern kern, int tiles, bool cooperative, Args &args, cudaStream_t st, const char *name) {
+static int launch_tiles(Kern kern, int tiles, bool cooperative, const Args &args, cudaStream_t st, const char *name) {
     const size_t smem = EV::smem_bytes();
     GP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     cudaLaunchConfig_t cfg = {};
@@ -1531,51 +1521,57 @@ static int launch_tiles(Kern kern, int tiles, bool cooperative, Args &args, cuda
     return GP_OK;
 }
 
-template <class EV>
-static int launch_ode(OdeArgs &a, cudaStream_t st) {
-    a.ntiles = (a.N + EV::RT - 1) / EV::RT;
-    return launch_tiles<EV>(ode_rk45_kernel<EV>, a.ntiles, true, a, st, "gp_scorenet_ode");
-}
-
-// One CTA (or cluster) per object, no grid barrier: an ordinary launch whose CTAs the hardware hands out as SMs free
-// up, which balances objects that finish at different step counts.
-template <class EV>
-static int launch_ode_obj(OdeObjArgs &oa, cudaStream_t st) {
-    oa.nsub = (oa.a.rpo + EV::RT - 1) / EV::RT;
-    if (oa.nsub * EV::RT > 128 || oa.nsub > OBJ_MAX_SUB) {
-        set_error("gp_scorenet_ode_objects: %d rows per object do not fit whole %d-row tiles in 128 rows", oa.a.rpo, EV::RT);
-        return GP_ERR_UNSUPPORTED;
-    }
-    oa.a.ntiles = oa.nobj * oa.nsub;
-    return launch_tiles<EV>(ode_rk45_obj_kernel<EV>, oa.nobj, false, oa, st, "gp_scorenet_ode_objects");
-}
-
 static size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
 
-// `mode` of the public entries: bits 0..1 = arithmetic (0 FFMA, 1 bf16, 2 split-bf16, 3 tf32), GP_MODE_SOLO / GP_MODE_CLUSTER
-// force the shape of the tensor-core evaluator; by default a batch of more 128-row tiles than the GPU holds 4-CTA
-// clusters at once (33 on a B200) runs one CTA per tile.
-// 0: cluster shape, 1: one CTA per tile (A operand in shared memory), 2: one CTA per tile, A operand in tensor memory
-static int use_solo(int mode, int N) {
-    if (mode & GP_MODE_SOLO) return (mode & GP_MODE_SMEM_A) ? 1 : 2;
-    if (mode & GP_MODE_CLUSTER) return 0;
-    return (N + tc::RT - 1) / tc::RT > 32 ? ((mode & GP_MODE_SMEM_A) ? 1 : 2) : 0;
+// Carries an evaluator type to a generic lambda: [&](auto use) { using EV = typename decltype(use)::type; ... }
+template <class EV>
+struct Use {
+    using type = EV;
+};
+
+// f(Use<SimtEval<rpt>>{}) for rpt among the FFMA tile heights RPT... the caller instantiates (the last one otherwise)
+template <int RPT, int... MORE, class F>
+static int with_simt_eval(int rpt, F &f) {
+    if constexpr (sizeof...(MORE) == 0) {
+        return f(Use<SimtEval<RPT>>{});
+    } else {
+        return rpt == RPT ? f(Use<SimtEval<RPT>>{}) : with_simt_eval<MORE...>(rpt, f);
+    }
 }
-static bool mode_ok(int mode) {
-    return (mode & ~(3 | GP_MODE_SOLO | GP_MODE_CLUSTER | GP_MODE_SMEM_A)) == 0 &&
-           (mode & (GP_MODE_SOLO | GP_MODE_CLUSTER)) != (GP_MODE_SOLO | GP_MODE_CLUSTER);
+
+// The trunk's evaluator for the `mode` of the public entries: calls f(Use<EV>{}) and returns its result.
+//   mode & 3       | cluster    | one CTA, A in tensor memory | one CTA, A in shared memory (GP_MODE_SMEM_A)
+//   0 fp32 FFMA    | SimtEval<rpt>: the caller's tile rule, one of RPT...; no shapes
+//   1 bf16         | TcEval<1>  | TcSoloT<1>                  | TcSolo<1>
+//   2 split-bf16   | TcEval<3>  | TcSoloT<3>                  | TcSolo<3>
+//   3 tf32         | TcEval<2>  | TcSoloT<2>                  | none: check_mode() refuses it
+// GP_MODE_SOLO / GP_MODE_CLUSTER force the shape; by default `shape_rows` that make more 128-row tiles than the GPU
+// holds 4-CTA clusters at once (33 on a B200) run one CTA per tile.  `mode` must have passed check_mode().
+template <int... RPT, class F>
+static int with_evaluator(int mode, int shape_rows, int rpt, F &&f) {
+    const bool solo = (mode & GP_MODE_SOLO) || (!(mode & GP_MODE_CLUSTER) && (shape_rows + tc::RT - 1) / tc::RT > 32);
+    const bool smem_a = (mode & GP_MODE_SMEM_A) != 0;
+    switch (mode & 3) {
+        case 1: return !solo ? f(Use<TcEval<1>>{}) : smem_a ? f(Use<TcSolo<1>>{}) : f(Use<TcSoloT<1>>{});
+        case 2: return !solo ? f(Use<TcEval<3>>{}) : smem_a ? f(Use<TcSolo<3>>{}) : f(Use<TcSoloT<3>>{});
+        case 3: return !solo ? f(Use<TcEval<2>>{}) : f(Use<TcSoloT<2>>{});
+        default: return with_simt_eval<RPT...>(rpt, f);
+    }
 }
+
 // Validation of `mode` shared by the trunk entries: a malformed value is a bad argument; tf32 (3) has evaluators with
-// the A operand in tensor memory only, so asking for the shared-memory-A shape is unsupported.
-#define GP_REQUIRE_MODE(mode, name)                                                                                    \
-    do {                                                                                                               \
-        GP_REQUIRE(mode_ok(mode), "%s: mode must be 0 (fp32 FFMA), 1 (bf16 tcgen05), 2 (split-bf16 x3 tcgen05) or 3 "  \
-                   "(tf32 tcgen05) [| GP_MODE_SOLO / GP_MODE_CLUSTER / GP_MODE_SMEM_A]", name);                         \
-        if (((mode) & 3) == 3 && ((mode) & GP_MODE_SMEM_A)) {                                                          \
-            gp::set_error("%s: tf32 mode (3) has no shared-memory-A evaluator (GP_MODE_SMEM_A)", name);                 \
-            return GP_ERR_UNSUPPORTED;                                                                                 \
-        }                                                                                                              \
-    } while (0)
+// the A operand in tensor memory only, so asking for the shared-memory-A shape is unsupported.  Returns the error code.
+static int check_mode(int mode, const char *name) {
+    GP_REQUIRE((mode & ~(3 | GP_MODE_SOLO | GP_MODE_CLUSTER | GP_MODE_SMEM_A)) == 0 &&
+                   (mode & (GP_MODE_SOLO | GP_MODE_CLUSTER)) != (GP_MODE_SOLO | GP_MODE_CLUSTER),
+               "%s: mode must be 0 (fp32 FFMA), 1 (bf16 tcgen05), 2 (split-bf16 x3 tcgen05) or 3 (tf32 tcgen05) "
+               "[| GP_MODE_SOLO / GP_MODE_CLUSTER / GP_MODE_SMEM_A]", name);
+    if ((mode & 3) == 3 && (mode & GP_MODE_SMEM_A)) {
+        set_error("%s: tf32 mode (3) has no shared-memory-A evaluator (GP_MODE_SMEM_A)", name);
+        return GP_ERR_UNSUPPORTED;
+    }
+    return GP_OK;
+}
 
 // Rows per compute thread of the FFMA evaluator (tile = 4x that many rows): the choice that minimises the
 // per-CTA critical path  waves(tiles / SMs) x rows-per-tile; ties go to the larger tile (fewer weight streams).
@@ -1630,35 +1626,13 @@ extern "C" int gp_trunk_project(const void *packed, const float *pts_feat, int B
     return GP_OK;
 }
 
-template <class EV, int MODE>
-static int launch_eval_ev(const void *packed, const float *proj, const float *x, const double *poses,
-                          const float *center, const float *t, int N, int rpo, float *out, cudaStream_t st) {
-    EvalArgs a;
-    a.P = (const float *)packed; a.proj = proj; a.x = x; a.poses = poses; a.center = center; a.t = t;
-    a.N = N; a.rpo = rpo; a.out = out;
-    return launch_tiles<EV>(eval_kernel<EV, MODE>, (N + EV::RT - 1) / EV::RT, false, a, st, "gp_scorenet_eval");
-}
-
+// Single evaluation (MODE 0) or energy (MODE 1): FFMA tiles of 16 rows up to 16 rows per SM, 32 above.
 template <int MODE>
-static int launch_eval(const void *packed, const float *proj, const float *x, const double *poses,
-                       const float *center, const float *t, int N, int rpo, float *out, int mode,
-                       cudaStream_t st, const char *name) {
-    if (N == 0) return GP_OK;
-    int rc;
-    const int solo_shape = use_solo(mode, N);
-    mode &= 3;
-    if (mode == 3) rc = solo_shape == 2 ? launch_eval_ev<TcSoloT<2>, MODE>(packed, proj, x, poses, center, t, N, rpo, out, st)
-                                        : launch_eval_ev<TcEval<2>, MODE>(packed, proj, x, poses, center, t, N, rpo, out, st);
-    else if (mode == 1 && solo_shape == 2) rc = launch_eval_ev<TcSoloT<1>, MODE>(packed, proj, x, poses, center, t, N, rpo, out, st);
-    else if (mode == 2 && solo_shape == 2) rc = launch_eval_ev<TcSoloT<3>, MODE>(packed, proj, x, poses, center, t, N, rpo, out, st);
-    else if (mode == 1 && solo_shape) rc = launch_eval_ev<TcSolo<1>, MODE>(packed, proj, x, poses, center, t, N, rpo, out, st);
-    else if (mode == 2 && solo_shape) rc = launch_eval_ev<TcSolo<3>, MODE>(packed, proj, x, poses, center, t, N, rpo, out, st);
-    else if (mode == 1) rc = launch_eval_ev<TcEval<1>, MODE>(packed, proj, x, poses, center, t, N, rpo, out, st);
-    else if (mode == 2) rc = launch_eval_ev<TcEval<3>, MODE>(packed, proj, x, poses, center, t, N, rpo, out, st);
-    else if (N <= 16 * num_sms()) rc = launch_eval_ev<SimtEval<4>, MODE>(packed, proj, x, poses, center, t, N, rpo, out, st);
-    else rc = launch_eval_ev<SimtEval<8>, MODE>(packed, proj, x, poses, center, t, N, rpo, out, st);
-    (void)name;
-    return rc;
+static int launch_eval(const EvalArgs &a, int mode, cudaStream_t st, const char *name) {
+    return with_evaluator<4, 8>(mode, a.N, a.N <= 16 * num_sms() ? 4 : 8, [&](auto use) {
+        using EV = typename decltype(use)::type;
+        return launch_tiles<EV>(eval_kernel<EV, MODE>, (a.N + EV::RT - 1) / EV::RT, false, a, st, name);
+    });
 }
 
 extern "C" int gp_scorenet_eval(const void *packed, const float *proj, const float *x, const float *t,
@@ -1666,8 +1640,9 @@ extern "C" int gp_scorenet_eval(const void *packed, const float *proj, const flo
     GP_REQUIRE(N >= 0 && rows_per_object >= 1, "gp_scorenet_eval: bad sizes");
     if (N == 0) return GP_OK;
     GP_REQUIRE(packed && proj && x && t && score, "gp_scorenet_eval: null pointer");
-    GP_REQUIRE_MODE(mode, "gp_scorenet_eval");
-    return launch_eval<0>(packed, proj, x, nullptr, nullptr, t, N, rows_per_object, score, mode, as_stream(s), "gp_scorenet_eval");
+    if (const int rc = check_mode(mode, "gp_scorenet_eval")) return rc;
+    const EvalArgs a = {(const float *)packed, proj, x, nullptr, nullptr, t, N, rows_per_object, score};
+    return launch_eval<0>(a, mode, as_stream(s), "gp_scorenet_eval");
 }
 
 extern "C" int gp_energy(const void *packed, const float *proj, const double *poses, const float *pts_center,
@@ -1675,8 +1650,9 @@ extern "C" int gp_energy(const void *packed, const float *proj, const double *po
     GP_REQUIRE(N >= 0 && rows_per_object >= 1, "gp_energy: bad sizes");
     if (N == 0) return GP_OK;
     GP_REQUIRE(packed && proj && poses && pts_center && t_rows && energy, "gp_energy: null pointer");
-    GP_REQUIRE_MODE(mode, "gp_energy");
-    return launch_eval<1>(packed, proj, nullptr, poses, pts_center, t_rows, N, rows_per_object, energy, mode, as_stream(s), "gp_energy");
+    if (const int rc = check_mode(mode, "gp_energy")) return rc;
+    const EvalArgs a = {(const float *)packed, proj, nullptr, poses, pts_center, t_rows, N, rows_per_object, energy};
+    return launch_eval<1>(a, mode, as_stream(s), "gp_energy");
 }
 
 // one [N][9] float64 array, padded to whole 128-row tiles (the per-tile vector loads are unconditional)
@@ -1689,6 +1665,33 @@ extern "C" size_t gp_scorenet_ode_workspace_bytes(int N) {
     return state * 9 * tc::CL + align256(2 * 3 * ntiles_max * sizeof(double)) + 256 /*barrier*/ + 256;
 }
 
+// The OdeArgs fields the batch and per-object entries share.  With t_eval (dense output) the denoise step is
+// (1 - eps) / n_eval, otherwise (1 - eps) / 1000 (samplers.py:238-249).
+static OdeArgs ode_args(const void *packed, const float *proj, const double *x0, const float *pts_center, int N,
+                        int rows_per_object, double T, double eps, double rtol, double atol, int denoise,
+                        double *x_out, const double *t_eval, int n_eval, double *dense, double *stats) {
+    // scipy validate_tol: rtol is clamped to 100 * EPS
+    if (rtol < 100 * 2.220446049250313e-16) rtol = 100 * 2.220446049250313e-16;
+    OdeArgs a = {};
+    a.P = (const float *)packed; a.proj = proj; a.x0 = x0; a.center = pts_center;
+    a.N = N; a.rpo = rows_per_object; a.T = T; a.eps = eps; a.rtol = rtol; a.atol = atol;
+    a.denoise = denoise; a.x_out = x_out; a.stats = stats;
+    a.t_eval = t_eval; a.n_eval = t_eval ? n_eval : 0; a.dense = dense;
+    a.denoise_steps = t_eval ? (double)n_eval : 1000.0;
+    return a;
+}
+
+// y[0..1] and K[0..6], `state` bytes each, from the 256-byte aligned start of the workspace, followed by the copies
+// of the other cluster ranks (a.replica doubles apart).  Returns the first byte after them.
+static unsigned char *carve_ode_state(OdeArgs &a, void *workspace, size_t state) {
+    unsigned char *w = (unsigned char *)(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
+    a.y[0] = (double *)w;
+    a.y[1] = (double *)(w + state);
+    for (int k = 0; k < 7; ++k) a.K[k] = (double *)(w + (2 + k) * state);
+    a.replica = 9 * state / sizeof(double);
+    return w + tc::CL * 9 * state;
+}
+
 static int scorenet_ode_impl(const void *packed, const float *proj, const double *x0, const float *pts_center,
                              int N, int rows_per_object, double T, double eps, double rtol, double atol,
                              int denoise, double *x_out, double *traj, int max_traj, const double *t_eval, int n_eval,
@@ -1698,43 +1701,25 @@ static int scorenet_ode_impl(const void *packed, const float *proj, const double
     GP_REQUIRE(N >= 1 && rows_per_object >= 1, "gp_scorenet_ode: bad sizes N=%d rows_per_object=%d", N, rows_per_object);
     GP_REQUIRE(rtol > 0 && atol > 0, "gp_scorenet_ode: tolerances must be positive");
     GP_REQUIRE(traj == nullptr || max_traj >= 1, "gp_scorenet_ode: max_traj < 1");
-    GP_REQUIRE_MODE(mode, "gp_scorenet_ode");
+    if (const int rc = check_mode(mode, "gp_scorenet_ode")) return rc;
     GP_REQUIRE((t_eval == nullptr) == (dense == nullptr) && (t_eval == nullptr || n_eval >= 1), "gp_scorenet_ode_dense: t_eval / dense / n_eval inconsistent");
     if (workspace_bytes < gp_scorenet_ode_workspace_bytes(N)) {
         set_error("gp_scorenet_ode: workspace too small (%zu < %zu)", workspace_bytes, gp_scorenet_ode_workspace_bytes(N));
         return GP_ERR_WORKSPACE;
     }
-    // scipy validate_tol: rtol is clamped to 100 * EPS
-    if (rtol < 100 * 2.220446049250313e-16) rtol = 100 * 2.220446049250313e-16;
-    OdeArgs a;
-    a.P = (const float *)packed; a.proj = proj; a.x0 = x0; a.center = pts_center;
-    a.N = N; a.rpo = rows_per_object; a.T = T; a.eps = eps; a.rtol = rtol; a.atol = atol;
-    a.denoise = denoise; a.x_out = x_out; a.traj = traj; a.max_traj = max_traj; a.stats = stats;
-    a.t_eval = t_eval; a.n_eval = t_eval ? n_eval : 0; a.dense = dense;
-    a.denoise_steps = t_eval ? (double)n_eval : 1000.0;   // samplers.py:238-249
-    unsigned char *w = (unsigned char *)(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
-    const size_t state = ode_state_bytes(N);
-    a.y[0] = (double *)w; w += state;
-    a.y[1] = (double *)w; w += state;
-    for (int k = 0; k < 7; ++k) { a.K[k] = (double *)w; w += state; }
-    a.replica = 9 * state / sizeof(double);
-    w += (tc::CL - 1) * 9 * state;
+    OdeArgs a = ode_args(packed, proj, x0, pts_center, N, rows_per_object, T, eps, rtol, atol, denoise, x_out, t_eval,
+                         n_eval, dense, stats);
+    a.traj = traj; a.max_traj = max_traj;
+    unsigned char *w = carve_ode_state(a, workspace, ode_state_bytes(N));
     a.part = (double *)w; w += align256(2 * 3 * ((size_t)(N + 7) / 8 + 1) * sizeof(double));
     a.gbar = (unsigned int *)w;
     cudaStream_t st = as_stream(s);
     GP_CUDA(cudaMemsetAsync(a.gbar, 0, 256, st));
-    const int sms = num_sms();
-    const int solo_shape = use_solo(mode, N);
-    mode &= 3;
-    if (mode == 3) return solo_shape == 2 ? launch_ode<TcSoloT<2>>(a, st) : launch_ode<TcEval<2>>(a, st);
-    if (mode == 1) return solo_shape == 2 ? launch_ode<TcSoloT<1>>(a, st) : solo_shape ? launch_ode<TcSolo<1>>(a, st) : launch_ode<TcEval<1>>(a, st);
-    if (mode == 2) return solo_shape == 2 ? launch_ode<TcSoloT<3>>(a, st) : solo_shape ? launch_ode<TcSolo<3>>(a, st) : launch_ode<TcEval<3>>(a, st);
-    switch (simt_rows_per_thread(N, sms)) {
-        case 2: return launch_ode<SimtEval<2>>(a, st);
-        case 4: return launch_ode<SimtEval<4>>(a, st);
-        case 6: return launch_ode<SimtEval<6>>(a, st);
-        default: return launch_ode<SimtEval<8>>(a, st);
-    }
+    return with_evaluator<2, 4, 6, 8>(mode, N, simt_rows_per_thread(N, num_sms()), [&](auto use) {
+        using EV = typename decltype(use)::type;
+        a.ntiles = (N + EV::RT - 1) / EV::RT;
+        return launch_tiles<EV>(ode_rk45_kernel<EV>, a.ntiles, true, a, st, "gp_scorenet_ode");
+    });
 }
 
 extern "C" int gp_scorenet_ode(const void *packed, const float *proj, const double *x0, const float *pts_center,
@@ -1779,7 +1764,7 @@ static int scorenet_ode_objects_impl(const void *packed, const float *proj, cons
         return GP_ERR_UNSUPPORTED;
     }
     GP_REQUIRE(rtol > 0 && atol > 0, "gp_scorenet_ode_objects: tolerances must be positive");
-    GP_REQUIRE_MODE(mode, "gp_scorenet_ode_objects");
+    if (const int rc = check_mode(mode, "gp_scorenet_ode_objects")) return rc;
     GP_REQUIRE((t_eval == nullptr) == (dense == nullptr) && (t_eval == nullptr || n_eval >= 1),
                "gp_scorenet_ode_dense_objects: t_eval / dense / n_eval inconsistent");
     const int B = N / rows_per_object;
@@ -1788,42 +1773,31 @@ static int scorenet_ode_objects_impl(const void *packed, const float *proj, cons
                   gp_scorenet_ode_objects_workspace_bytes(B, rows_per_object));
         return GP_ERR_WORKSPACE;
     }
-    if (rtol < 100 * 2.220446049250313e-16) rtol = 100 * 2.220446049250313e-16;
     OdeObjArgs oa = {};
-    OdeArgs &a = oa.a;
-    a.P = (const float *)packed; a.proj = proj; a.x0 = x0; a.center = pts_center;
-    a.N = N; a.rpo = rows_per_object; a.T = T; a.eps = eps; a.rtol = rtol; a.atol = atol;
-    a.denoise = denoise; a.x_out = x_out; a.traj = nullptr; a.max_traj = 0; a.stats = stats;
-    a.t_eval = t_eval; a.n_eval = t_eval ? n_eval : 0; a.dense = dense;
-    a.denoise_steps = t_eval ? (double)n_eval : 1000.0;
-    unsigned char *w = (unsigned char *)(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
-    const size_t state = ode_obj_state_bytes(B);
-    a.y[0] = (double *)w; w += state;
-    a.y[1] = (double *)w; w += state;
-    for (int k = 0; k < 7; ++k) { a.K[k] = (double *)w; w += state; }
-    a.replica = 9 * state / sizeof(double);
-    a.part = nullptr; a.gbar = nullptr;
+    oa.a = ode_args(packed, proj, x0, pts_center, N, rows_per_object, T, eps, rtol, atol, denoise, x_out, t_eval, n_eval,
+                    dense, stats);
+    carve_ode_state(oa.a, workspace, ode_obj_state_bytes(B));
     oa.nobj = B;
     oa.obj_stats = obj_stats;
     oa.T_obj = T_obj;
     oa.t_eval_stride = (T_obj != nullptr && t_eval != nullptr) ? (size_t)n_eval : 0;
     cudaStream_t st = as_stream(s);
-    // the evaluator shape follows the tile count B exactly as the batch rule follows its tile count
-    const int solo_shape = use_solo(mode, B * tc::RT);
-    mode &= 3;
-    int rc;
-    if (mode == 3) rc = solo_shape == 2 ? launch_ode_obj<TcSoloT<2>>(oa, st) : launch_ode_obj<TcEval<2>>(oa, st);
-    else if (mode == 1) rc = solo_shape == 2 ? launch_ode_obj<TcSoloT<1>>(oa, st) : solo_shape ? launch_ode_obj<TcSolo<1>>(oa, st) : launch_ode_obj<TcEval<1>>(oa, st);
-    else if (mode == 2) rc = solo_shape == 2 ? launch_ode_obj<TcSoloT<3>>(oa, st) : solo_shape ? launch_ode_obj<TcSolo<3>>(oa, st) : launch_ode_obj<TcEval<3>>(oa, st);
-    else {
-        // the FFMA tile height of a batch call with this one object, so that the two agree bit for bit
-        switch (simt_rows_per_thread(rows_per_object, num_sms())) {
-            case 2: rc = launch_ode_obj<SimtEval<2>>(oa, st); break;
-            case 4: rc = launch_ode_obj<SimtEval<4>>(oa, st); break;
-            case 6: rc = launch_ode_obj<SimtEval<6>>(oa, st); break;
-            default: rc = launch_ode_obj<SimtEval<8>>(oa, st); break;
+    // The evaluator shape follows the tile count B exactly as the batch rule follows its tile count; the FFMA tile
+    // height is that of a batch call with this one object, so that the two agree bit for bit.
+    const int rpt = simt_rows_per_thread(rows_per_object, num_sms());
+    const int rc = with_evaluator<2, 4, 6, 8>(mode, B * tc::RT, rpt, [&](auto use) {
+        using EV = typename decltype(use)::type;
+        oa.nsub = (rows_per_object + EV::RT - 1) / EV::RT;
+        if (oa.nsub * EV::RT > 128 || oa.nsub > OBJ_MAX_SUB) {
+            set_error("gp_scorenet_ode_objects: %d rows per object do not fit whole %d-row tiles in 128 rows",
+                      rows_per_object, EV::RT);
+            return (int)GP_ERR_UNSUPPORTED;
         }
-    }
+        oa.a.ntiles = B * oa.nsub;
+        // One CTA (or cluster) per object, no grid barrier: an ordinary launch whose CTAs the hardware hands out as
+        // SMs free up, which balances objects that finish at different step counts.
+        return launch_tiles<EV>(ode_rk45_obj_kernel<EV>, B, false, oa, st, "gp_scorenet_ode_objects");
+    });
     if (rc != GP_OK) return rc;
     ode_obj_summary_kernel<<<1, 32, 0, st>>>(obj_stats, B, stats);
     GP_CHECK_LAUNCH("gp_scorenet_ode_objects");
@@ -1880,19 +1854,13 @@ extern "C" size_t gp_scorenet_pc_workspace_bytes(int N) {
     return align256((size_t)N * 9 * sizeof(float)) + align256(2 * ((size_t)(N + 7) / 8 + 1) * sizeof(double)) + 256 /*barrier*/ + 256;
 }
 
-template <class EV>
-static int launch_pc(PcArgs &a, cudaStream_t st) {
-    a.ntiles = (a.N + EV::RT - 1) / EV::RT;
-    return launch_tiles<EV>(pc_kernel<EV>, a.ntiles, true, a, st, "gp_scorenet_pc");
-}
-
 extern "C" int gp_scorenet_pc(const void *packed, const float *proj, const float *x0, const float *noise,
                               const float *pts_center, const float *time_steps, int N, int rows_per_object,
                               int num_steps, double snr, float *xs, float *mean_x, void *workspace,
                               size_t workspace_bytes, int mode, gp_stream_t s) {
     GP_REQUIRE(packed && proj && x0 && noise && pts_center && time_steps && mean_x && workspace, "gp_scorenet_pc: null pointer");
     GP_REQUIRE(N >= 1 && rows_per_object >= 1 && num_steps >= 2, "gp_scorenet_pc: bad sizes");
-    GP_REQUIRE_MODE(mode, "gp_scorenet_pc");
+    if (const int rc = check_mode(mode, "gp_scorenet_pc")) return rc;
     if (workspace_bytes < gp_scorenet_pc_workspace_bytes(N)) {
         set_error("gp_scorenet_pc: workspace too small");
         return GP_ERR_WORKSPACE;
@@ -1907,16 +1875,9 @@ extern "C" int gp_scorenet_pc(const void *packed, const float *proj, const float
     a.gbar = (unsigned int *)w;
     cudaStream_t st = as_stream(s);
     GP_CUDA(cudaMemsetAsync(a.gbar, 0, 256, st));
-    const int sms = num_sms();
-    const int solo_shape = use_solo(mode, N);
-    mode &= 3;
-    if (mode == 3) return solo_shape == 2 ? launch_pc<TcSoloT<2>>(a, st) : launch_pc<TcEval<2>>(a, st);
-    if (mode == 1) return solo_shape == 2 ? launch_pc<TcSoloT<1>>(a, st) : solo_shape ? launch_pc<TcSolo<1>>(a, st) : launch_pc<TcEval<1>>(a, st);
-    if (mode == 2) return solo_shape == 2 ? launch_pc<TcSoloT<3>>(a, st) : solo_shape ? launch_pc<TcSolo<3>>(a, st) : launch_pc<TcEval<3>>(a, st);
-    switch (simt_rows_per_thread(N, sms)) {
-        case 2: return launch_pc<SimtEval<2>>(a, st);
-        case 4: return launch_pc<SimtEval<4>>(a, st);
-        case 6: return launch_pc<SimtEval<6>>(a, st);
-        default: return launch_pc<SimtEval<8>>(a, st);
-    }
+    return with_evaluator<2, 4, 6, 8>(mode, N, simt_rows_per_thread(N, num_sms()), [&](auto use) {
+        using EV = typename decltype(use)::type;
+        a.ntiles = (N + EV::RT - 1) / EV::RT;
+        return launch_tiles<EV>(pc_kernel<EV>, a.ntiles, true, a, st, "gp_scorenet_pc");
+    });
 }
