@@ -5,21 +5,9 @@
 // object's [R,9] block belongs to Box-Muller pair p = e / 2; pair p takes words 2*(p % 2), 2*(p % 2) + 1 of the
 // Philox output for counter (p / 2, 0, 0, 0).  One thread makes one Philox call: pairs 2q, 2q+1, elements 4q .. 4q+3.
 #include "common.cuh"
+#include "philox.cuh"
 
 namespace gp {
-
-__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint32_t k0, uint32_t k1) {
-    constexpr uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        const uint32_t hi0 = __umulhi(M0, c.x), lo0 = M0 * c.x;
-        const uint32_t hi1 = __umulhi(M1, c.z), lo1 = M1 * c.z;
-        c = make_uint4(hi1 ^ c.y ^ k0, lo1, hi0 ^ c.w ^ k1, lo0);
-        k0 += W0;
-        k1 += W1;
-    }
-    return c;
-}
 
 // u = (w + 0.5) * 2^-32 in (0, 1), float64
 __device__ __forceinline__ double philox_uniform(uint32_t w) { return ((double)w + 0.5) * 0x1p-32; }

@@ -187,3 +187,30 @@ def make_cluster_quaternion_poses(num_objects, repeat_num=50, seed=0, outlier_fr
             out[b, r, 3:6] = Rm[:, 1]
             out[b, r, 6:] = rng.normal(0, 0.01, 3) + np.array([0.0, 0.0, 0.8])
     return torch.from_numpy(out)
+
+
+def make_instance_frame(H, W, num_objects, seed=0, bad_depth=0.0, stray_labels=0.0):
+    """A depth frame and its instance-label image (the input of clouds.object_clouds): a slanted background 1.5-2.5 m
+    away and B rectangles (labels 1..B, drawn in order, so a later one may cover an earlier one) 0.4-1.2 m away, 1 mm
+    depth noise.  Rectangle sides scale with sqrt(H * W / B).  `bad_depth` of the pixels get a depth of 0, -0.5, NaN,
+    +inf or -inf; `stray_labels` of them a label outside 1..B (0, -1, B + 1, 2^30).
+    Returns (depth float32 [H,W], labels int32 [H,W]) as numpy arrays."""
+    rng = np.random.default_rng(seed)
+    B = num_objects
+    v, u = np.mgrid[0:H, 0:W]
+    depth = 1.5 + u / W * 0.5 + v / H * 0.5
+    labels = np.zeros((H, W), dtype=np.int32)
+    side = np.sqrt(H * W / B)
+    for b in range(B):
+        h = int(np.clip(side * rng.uniform(0.3, 1.5), 1, H))
+        w = int(np.clip(side * rng.uniform(0.3, 1.5), 1, W))
+        v0, u0 = int(rng.integers(0, H - h + 1)), int(rng.integers(0, W - w + 1))
+        labels[v0:v0 + h, u0:u0 + w] = b + 1
+        depth[v0:v0 + h, u0:u0 + w] = rng.uniform(0.4, 1.2) + 0.1 * (u[v0:v0 + h, u0:u0 + w] - u0) / max(w, 1)
+    depth = (depth + rng.normal(0.0, 1e-3, size=(H, W))).astype(np.float32)
+    pick = rng.random((H, W))
+    bad = pick < bad_depth
+    depth[bad] = rng.choice(np.array([0.0, -0.5, np.nan, np.inf, -np.inf], dtype=np.float32), int(bad.sum()))
+    stray = rng.random((H, W)) < stray_labels
+    labels[stray] = rng.choice(np.array([0, -1, B + 1, 1 << 30], dtype=np.int32), int(stray.sum()))
+    return depth, labels

@@ -373,6 +373,47 @@ GP_API int gp_scorenet_ode_objects_t0(const void *packed, const float *proj, con
  * normals).  R*9 odd: the sine of the last pair is dropped. */
 GP_API int gp_object_noise(const int64_t *keys, const float *sigma, int B, int R, float *noise, gp_stream_t s);
 
+/* ---------------------------------------------------------------------------------------------
+ * Per-object point clouds from a depth frame and an instance-label image (DESIGN.md section 4.13): the `pts` /
+ * `pts_center` inputs the pipeline takes, built on the device instead of the datasets' numpy loop
+ * (datasets/datasets_omni6dpose.py:459-473).
+ * ------------------------------------------------------------------------------------------ */
+
+/* Most objects and pixels one gp_backproject_instances call takes (2^30 pixels keeps every pixel index of the
+ * 1024-pixel tiles inside int). */
+enum { GP_MAX_FRAME_OBJECTS = 1024, GP_MAX_FRAME_PIXELS = 1 << 30 };
+
+/* Stage A, back-projection and stable per-object compaction.
+ *   depth  [H,W] f32 metres;  labels [H,W] i32: value b+1 is object b, values outside 1..B are background.
+ *   Pixel (u = column, v = row) is kept iff its label is in 1..B and z = depth > 0 and finite; its point is
+ *   (x, y, z) with x = ((float)u - cx) * z / fx and y = ((float)v - cy) * z / fy, IEEE float32 in that order
+ *   (no pixel-centre offset).
+ *   xyz     [H*W, 3] f32 (capacity-sized): object b's points are rows offsets[b] .. offsets[b+1]-1 in row-major
+ *           pixel order (numpy's xyz[labels == b+1]); rows from offsets[B] on are not written.
+ *   offsets [B+1] i32 (device).
+ * B > GP_MAX_FRAME_OBJECTS returns GP_ERR_UNSUPPORTED, H * W > GP_MAX_FRAME_PIXELS GP_ERR_BAD_ARG (the workspace
+ * query returns 0 for both, as for bad sizes).  Intrinsics
+ * must be finite with fx, fy != 0.  Three kernel launches, no host synchronisation. */
+GP_API size_t gp_backproject_instances_workspace_bytes(int H, int W, int B);
+GP_API int gp_backproject_instances(const float *depth, const int32_t *labels, int H, int W, float fx, float fy,
+                                    float cx, float cy, int B, float *xyz, int32_t *offsets, void *workspace,
+                                    size_t workspace_bytes, gp_stream_t s);
+
+/* Stage B, sample_points (datasets_omni6dpose.py:459-473) with a keyed random choice.  Object b has the K points
+ * xyz[offsets[b] .. offsets[b+1]-1] (offsets clamped into [0, rows] first; K = 0 when they cross); pts [B,N,3] f32:
+ *   K < N: row r < (N / K) * K is point r % K (np.tile), the last N % K rows are points pi_b(0) .. pi_b(N % K - 1);
+ *   K == N: the cloud unchanged;  K > N: row j is point pi_b(j) (permutation(K)[:N]);
+ *   K == 0: zero rows and a zero centre.
+ * pi_b, a permutation of [0, K): a 4-round balanced Feistel network on k = max(2, ceil(log2 K)) bits, k rounded up
+ * to even, halves of k/2 bits (x = L << k/2 | R); round r = 0..3 maps (L, R) to (R, L ^ F_r(R)) with
+ * F_r(R) = Philox4x32-10(counter (R, r, 1, 0), key (lo32, hi32) of keys[b]).x & (2^(k/2) - 1); values >= K are
+ * encrypted again (cycle walking).  Counter word 2 = 1 keeps this stream apart from gp_object_noise's (q, 0, 0, 0).
+ *   pts_center [B,3] f32: the mean of the N rows, summed in float64 and rounded to float32 (within 1 float32 ulp of
+ *   the float64 mean of pts);  counts [B] i32: K.
+ *   keys [B] int64 (device).  xyz may be NULL when rows == 0. */
+GP_API int gp_sample_points(const float *xyz, long long rows, const int32_t *offsets, const int64_t *keys, int B,
+                            int N, float *pts, float *pts_center, int32_t *counts, gp_stream_t s);
+
 /* Post-processing of a recorded trajectory into the reference's `xs` (samplers.py:251-255):
  * traj [S,N,9] f64 raw -> xs [N,S,9] f64 with Gram-Schmidt on the rotation part and the centre
  * added. */
