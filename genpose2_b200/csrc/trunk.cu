@@ -260,7 +260,14 @@ struct TcEval {
     static __device__ __forceinline__ float *tq(Smem &S) { return S.tq; }
     static __device__ __forceinline__ void setup(Smem &S, Ctx &c, const float *P) { tc::setup<NPASS>(S, c, P); }
     static __device__ __forceinline__ void teardown(Smem &S, Ctx &c) { tc::teardown<NPASS>(S, c); }
-    static __device__ __forceinline__ void stage_tq(const float *P, Smem &S, Ctx &c, int ns) { tc::compute_tq_rank<NPASS>(P, S, c, ns); }
+    // The t-branch uses S.part as scratch, and S.part is where the peers deposit their partials of the next forward()
+    // as soon as this CTA has consumed the previous ones.  A peer runs ahead whenever rank 0 has extra work between two
+    // evaluations (it alone stores outputs and dense-output points), so no peer may start the next forward() before
+    // every CTA of the cluster is done with its scratch: one cluster barrier per t-branch.
+    static __device__ __forceinline__ void stage_tq(const float *P, Smem &S, Ctx &c, int ns) {
+        tc::compute_tq_rank<NPASS>(P, S, c, ns);
+        tile_sync();
+    }
     static __device__ __forceinline__ void begin_tile(Smem &S, Ctx &c, const float *proj, int r0, int N, int rpo) {
         tc::begin_tile<NPASS>(S, c, proj, r0, N, rpo);
     }
