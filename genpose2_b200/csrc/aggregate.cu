@@ -2,6 +2,8 @@
 // object, and the ScaleNet bbox head.  Replaces the Python / sklearn / cuSOLVER host loop of
 // runners/evaluation_single.py:179-215 (one D2H + sklearn call per object) with segmented
 // reductions that never leave the device.
+// Energies are ranked like torch.sort(descending=True, stable=True) (NaN above +inf, ties by index), so an object whose
+// retained set holds a NaN pose comes out NaN in rows 0-2 with labels -1, and no other object changes.
 #include "common.cuh"
 
 namespace gp {
@@ -11,7 +13,7 @@ constexpr int AG_MAXR = 64;     // hypotheses per object
 constexpr int AG_MAXK = 32;     // retained hypotheses (DBSCAN neighbourhoods are 32-bit masks)
 
 struct AggSmem {
-    float e[AG_MAXR][2];
+    unsigned e[AG_MAXR][2];      // rank_key of the energies
     int order[2][AG_MAXR];       // rank -> hypothesis, per energy channel
     double q[AG_MAXR][4];        // retained quaternions (wxyz); more than AG_MAXK only without clustering
     double D[AG_MAXK][AG_MAXK];  // 1 - <qi,qj>^2
@@ -109,6 +111,14 @@ __device__ void average_quat(const double (*q)[4], unsigned long long mask, doub
     top_eigvec4(A, out);
 }
 
+// rank key of an energy: descending unsigned order of the keys is torch.sort(descending=True)'s order -- every NaN
+// (any payload) one key above +inf, -0 the key of +0 -- so with ties broken by index the ranks are a permutation
+// whatever the energies are.  Keys are made once per energy; the rank loop compares integers.
+__device__ __forceinline__ unsigned rank_key(float e) {
+    const unsigned u = e != e ? 0x7fc00000u : (e == 0.f ? 0u : __float_as_uint(e));
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+
 __global__ void __launch_bounds__(AG_WARPS * 32)
 aggregate_kernel(const double *__restrict__ poses, const float *__restrict__ energy, int B, int R, int retain,
                  int clustering, double eps, int min_samples, float *__restrict__ pose_out,
@@ -120,15 +130,15 @@ aggregate_kernel(const double *__restrict__ poses, const float *__restrict__ ene
     AggSmem &S = sm[warp];
     const double *P = poses + (size_t)b * R * 9;
 
-    for (int i = lane; i < R * 2; i += 32) S.e[i >> 1][i & 1] = energy[(size_t)b * R * 2 + i];
+    for (int i = lane; i < R * 2; i += 32) S.e[i >> 1][i & 1] = rank_key(energy[(size_t)b * R * 2 + i]);
     __syncwarp();
     // descending stable rank per channel (torch.sort(energy, descending=True, dim=1), reward.py:145)
     for (int i = lane; i < R; i += 32) {
         for (int ch = 0; ch < 2; ++ch) {
-            const float ei = S.e[i][ch];
+            const unsigned ei = S.e[i][ch];
             int rank = 0;
             for (int j = 0; j < R; ++j) {
-                const float ej = S.e[j][ch];
+                const unsigned ej = S.e[j][ch];
                 rank += (ej > ei) || (ej == ei && j < i);
             }
             S.order[ch][rank] = i;
@@ -286,7 +296,7 @@ __device__ __forceinline__ void dense_rows(const float *__restrict__ W, const fl
 #pragma unroll
                 for (int s = 16; s > 0; s >>= 1) v += __shfl_xor_sync(0xffffffffu, v, s);
                 v += bv;
-                if (lane == 0) out[o * out_ld + n] = RELU ? fmaxf(v, 0.f) : v;
+                if (lane == 0) out[o * out_ld + n] = RELU && v == v ? fmaxf(v, 0.f) : v;   // NaN passes, like torch.relu
             }
         }
     }
