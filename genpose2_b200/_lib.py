@@ -103,6 +103,9 @@ SIGNATURES = {
     "gp_backproject_instances_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "gp_backproject_instances": (c_int, [c_void_p, c_void_p, c_int, c_int, c_float, c_float, c_float, c_float, c_int,
                                          c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "gp_backproject_frames_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int]),
+    "gp_backproject_frames": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p,
+                                      c_void_p, c_void_p, c_size_t, c_void_p]),
     "gp_sample_points": (c_int, [c_void_p, ctypes.c_longlong, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p,
                                  c_void_p, c_void_p]),
     "gp_traj_finalize": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),

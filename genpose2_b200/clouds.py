@@ -7,6 +7,9 @@ datasets/datasets_omni6dpose.py:459-473).  Here both stages run on libgenpose_b2
   backproject_instances   depth + labels -> ragged per-object clouds (xyz, offsets)         gp_backproject_instances
   sample_points           ragged clouds -> fixed-size clouds with a keyed random choice     gp_sample_points
   object_clouds           both: the data dict PosePipeline(...)(data, ...) takes
+  backproject_frames      stage A over F frames of one size in one pass, objects numbered frame-major
+                                                                                    gp_backproject_frames
+  object_clouds_frames    both stages over F frames
 
 Object b's sampled cloud depends only on its pixels (or its K points) and keys[b]; the permutation uses the key's
 Philox stream with counter word 2 = 1, apart from the prior noise of gp_object_noise, so one key per object can feed
@@ -20,7 +23,8 @@ from . import _lib
 from .samplers import check_noise_keys
 
 MAX_OBJECTS = 1024   # GP_MAX_FRAME_OBJECTS: objects per frame of backproject_instances / object_clouds
-MAX_PIXELS = 1 << 30   # GP_MAX_FRAME_PIXELS: pixels per frame
+MAX_PIXELS = 1 << 30   # GP_MAX_FRAME_PIXELS: pixels per frame (per call of backproject_frames / object_clouds_frames)
+MAX_FRAMES = 1024   # GP_MAX_FRAMES: frames per call of backproject_frames / object_clouds_frames
 
 
 def _device_tensor(t, name, dtype, ndim):
@@ -162,5 +166,141 @@ def object_clouds(depth, labels, intrinsics, keys, num_points=1024):
     N = _check_num_points(num_points)
     keys = _check_keys(keys, B, depth)
     xyz, offsets = _backproject(depth, labels, H, W, B, intr)
+    pts, center, counts = _sample(xyz, offsets, keys, N)
+    return {"pts": pts, "pts_center": center, "counts": counts}
+
+
+def _check_frames(depth, labels, intrinsics, objects_per_frame, num_objects):
+    """-> (F, H, W, B, intrinsics, frame offsets): each either a CUDA tensor given by the caller or a host array to
+    upload (float32 [F,4], int32 [F+1])."""
+    _device_tensor(depth, "depth", torch.float32, 3)
+    _device_tensor(labels, "labels", torch.int32, 3)
+    if tuple(labels.shape) != tuple(depth.shape):
+        raise ValueError(f"labels {tuple(labels.shape)} and depth {tuple(depth.shape)} must have the same shape")
+    _same_device(depth, labels=labels)
+    F, H, W = depth.shape
+    if F * H * W == 0:
+        raise ValueError(f"depth must hold at least one frame of at least one pixel, got {tuple(depth.shape)}")
+    if F * H * W > MAX_PIXELS:
+        raise NotImplementedError(f"at most 2^30 pixels per call are supported, got {F} frames of {H} x {W}")
+    if F > MAX_FRAMES:
+        raise NotImplementedError(f"at most {MAX_FRAMES} frames per call are supported, got {F}")
+    capturing = torch.cuda.is_initialized() and torch.cuda.is_current_stream_capturing()
+    if isinstance(intrinsics, torch.Tensor) and intrinsics.is_cuda:
+        _device_tensor(intrinsics, "intrinsics", torch.float32, 2)
+        if tuple(intrinsics.shape) != (F, 4):
+            raise ValueError(f"intrinsics must be [F, 4] = [{F}, 4], got {tuple(intrinsics.shape)}")
+        _same_device(depth, intrinsics=intrinsics)
+        intr = intrinsics
+    else:
+        if capturing:
+            raise RuntimeError("host intrinsics cannot be used in a CUDA graph capture: pass a CUDA float32 [F, 4] "
+                               "tensor")
+        try:
+            vals = np.asarray(intrinsics, dtype=np.float64)
+        except (TypeError, ValueError):
+            raise TypeError(f"intrinsics must be F rows of four numbers (fx, fy, cx, cy), got {intrinsics!r}") from None
+        if vals.shape != (F, 4):
+            raise ValueError(f"intrinsics must be F rows of four numbers (fx, fy, cx, cy): [{F}, 4], got shape "
+                             f"{vals.shape}")
+        with np.errstate(over="ignore"):
+            intr = vals.astype(np.float32)
+        bad = ~np.isfinite(intr).all(1) | (intr[:, 0] == 0) | (intr[:, 1] == 0)
+        if bad.any():
+            f = int(np.nonzero(bad)[0][0])
+            raise ValueError(f"intrinsics must be finite float32 values with fx, fy != 0, got {vals[f].tolist()} "
+                             f"for frame {f}")
+    if num_objects is not None:
+        if isinstance(num_objects, bool) or not isinstance(num_objects, (int, np.integer)):
+            raise TypeError(f"num_objects must be an int, got {type(num_objects).__name__}")
+        num_objects = int(num_objects)
+    if isinstance(objects_per_frame, torch.Tensor) and objects_per_frame.is_cuda:
+        _device_tensor(objects_per_frame, "objects_per_frame", torch.int32, 1)
+        if objects_per_frame.shape[0] != F + 1:
+            raise ValueError(f"objects_per_frame as a CUDA tensor holds the frame offsets [F + 1] = [{F + 1}], got "
+                             f"{tuple(objects_per_frame.shape)}")
+        _same_device(depth, objects_per_frame=objects_per_frame)
+        if num_objects is None:
+            raise TypeError("the number of objects must be given with CUDA frame offsets (they are not read on the "
+                            "host)")
+        B, offsets = num_objects, objects_per_frame
+    else:
+        if capturing:
+            raise RuntimeError("host objects_per_frame cannot be used in a CUDA graph capture: pass the frame offsets "
+                               "as a CUDA int32 [F + 1] tensor")
+        if isinstance(objects_per_frame, torch.Tensor):
+            objects_per_frame = objects_per_frame.tolist()
+        try:
+            counts = list(objects_per_frame)
+        except TypeError:
+            raise TypeError(f"objects_per_frame must be a sequence of F ints, got {objects_per_frame!r}") from None
+        if len(counts) != F:
+            raise ValueError(f"objects_per_frame must hold one count per frame: {F} frames, got {len(counts)}")
+        for n in counts:
+            if isinstance(n, bool) or not isinstance(n, (int, np.integer)):
+                raise TypeError(f"objects_per_frame must hold ints, got {n!r}")
+            if n < 0:
+                raise ValueError(f"objects_per_frame must hold counts >= 0, got {counts}")
+        B = int(sum(int(n) for n in counts))
+        if num_objects is not None and num_objects != B:
+            raise ValueError(f"objects_per_frame sums to {B} objects, expected {num_objects}")
+        offsets = counts
+    if B < 1:
+        raise ValueError(f"the frames must hold at least one object, got {B}")
+    if B > MAX_OBJECTS:
+        raise NotImplementedError(f"at most {MAX_OBJECTS} objects per call are supported, got {B}")
+    if not isinstance(offsets, torch.Tensor):
+        offsets = np.concatenate([[0], np.cumsum(offsets)]).astype(np.int32)
+    return F, H, W, B, intr, offsets
+
+
+def _upload(a, dev):
+    """Host array -> device through pinned staging, without a synchronisation (torch's pinned-memory cache reuses the
+    staging block only after the copy's event)."""
+    if isinstance(a, torch.Tensor):
+        return a
+    return torch.from_numpy(a).pin_memory().to(dev, non_blocking=True)
+
+
+def _backproject_frames(depth, labels, F, H, W, B, intr, frame_offsets):
+    dev = depth.device
+    intr, frame_offsets = _upload(intr, dev), _upload(frame_offsets, dev)
+    xyz = torch.empty((F * H * W, 3), dtype=torch.float32, device=dev)
+    offsets = torch.empty((B + 1,), dtype=torch.int32, device=dev)
+    ws_bytes = _lib.load().gp_backproject_frames_workspace_bytes(F, H, W, B)
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+    _lib.call("gp_backproject_frames", _lib.ptr(depth), _lib.ptr(labels), F, H, W, _lib.ptr(intr),
+              _lib.ptr(frame_offsets), B, _lib.ptr(xyz), _lib.ptr(offsets), _lib.ptr(ws), ws_bytes, device=dev)
+    return xyz, offsets
+
+
+def backproject_frames(depth, labels, intrinsics, objects_per_frame, *, num_objects=None):
+    """Stage A over F frames of one size in one pass (one frame per tracked video, or per camera of a rig).
+    depth float32 [F,H,W], labels int32 [F,H,W], intrinsics one (fx, fy, cx, cy) per frame: host values [F][4] or a
+    CUDA float32 [F,4] tensor.  objects_per_frame: the host counts n_f of the F frames, or a CUDA int32 [F+1] tensor of
+    frame offsets (0, n_0, n_0 + n_1, ..., B), which needs num_objects = B.  At most MAX_FRAMES frames, MAX_OBJECTS
+    objects and MAX_PIXELS pixels in all.
+
+    Objects are numbered frame-major: label l with 1 <= l <= n_f in frame f is object n_0 + ... + n_(f-1) + l - 1, any
+    other label (one above n_f too) is background; each frame is back-projected with its own intrinsics by the rules of
+    backproject_instances.  Returns (xyz float32 [F*H*W, 3], offsets int32 [B+1]): bit for bit the concatenation, in
+    frame order, of backproject_instances on each frame.  Host forms are validated (finite, fx, fy != 0, counts >= 0)
+    and uploaded without a synchronisation; CUDA forms are not read on the host, so a graph captured with them replays
+    new intrinsics and new per-frame counts (same F, H, W and B).  Malformed CUDA offsets are clamped on the device
+    (include/genpose_b200.h, gp_backproject_frames): wrong clouds, never an out-of-bounds access."""
+    F, H, W, B, intr, offs = _check_frames(depth, labels, intrinsics, objects_per_frame, num_objects)
+    return _backproject_frames(depth, labels, F, H, W, B, intr, offs)
+
+
+def object_clouds_frames(depth, labels, intrinsics, objects_per_frame, keys, num_points=1024):
+    """Both stages over F frames: backproject_frames, then sample_points with keys[b] for object b (B = len(keys),
+    objects numbered frame-major) -> {"pts" [B,N,3], "pts_center" [B,3], "counts" [B]}, bit for bit the per-frame
+    object_clouds results concatenated.  Host counts must sum to len(keys)."""
+    if not isinstance(keys, torch.Tensor) or keys.dim() != 1:
+        raise TypeError("keys must be a 1-D int64 tensor, one key per object")
+    F, H, W, B, intr, offs = _check_frames(depth, labels, intrinsics, objects_per_frame, keys.shape[0])
+    N = _check_num_points(num_points)
+    keys = _check_keys(keys, B, depth)
+    xyz, offsets = _backproject_frames(depth, labels, F, H, W, B, intr, offs)
     pts, center, counts = _sample(xyz, offsets, keys, N)
     return {"pts": pts, "pts_center": center, "counts": counts}

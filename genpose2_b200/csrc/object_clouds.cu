@@ -1,14 +1,15 @@
-// Per-object point clouds built on the device from a depth frame and an instance-label image (DESIGN.md section 4.13).
+// Per-object point clouds built on the device from depth frames and instance-label images (DESIGN.md section 4.13).
 //
-// Stage A, gp_backproject_instances: back-projection and a stable segmented compaction, three launches.
-//   count    one warp per tile of 1024 consecutive pixels (32 rounds of 32): per-tile object counts into
-//            hist[object][tile] (__match_any_sync groups the lanes of one object, the lowest lane adds the group)
+// Stage A, gp_backproject_instances (one frame) and gp_backproject_frames (F frames of one size, objects numbered
+// frame-major): back-projection and a stable segmented compaction, three launches.  The count and scatter grids are
+// (tile groups of a frame, frame); one frame is the case F = 1 with objects [0, B) and the intrinsics as arguments.
+//   count    one warp per tile of 1024 consecutive pixels (32 rounds of 32): per-tile object counts of the block's
+//            frame into hist[object][tile of its frame] (__match_any_sync groups the lanes of one object, the lowest
+//            lane adds the group); with F frames the block also clamps its frame's object range from frame_offsets
 //   scan     one block per object: exclusive scan of its row of hist over the tiles, the row total into totals[object]
 //   scatter  the count kernel's walk again: every block scans totals into the object offsets, a kept pixel lands at
 //            offsets[object] + hist[object][tile] + (pixels of the object earlier in the tile) -- row-major pixel order
-//            within each object, whatever the scheduling, without atomics
-// Stage B, gp_sample_points: one block per object, one thread per output row (block-strided), the centre as a float64
-// block reduction.  The keyed permutation pi_b is a 4-round balanced Feistel network on Philox4x32-10 with cycle walking.
+//            within each object, frames in order, whatever the scheduling, without atomics
 #include <climits>
 #include <cmath>
 
@@ -52,21 +53,56 @@ __device__ __forceinline__ int block_exclusive_scan(int v, int &total) {
     return before + inc - v;
 }
 
-// object of pixel p (label b + 1 -> b) when the pixel is kept, else -1
-__device__ __forceinline__ int kept_object(int label, float z, int B) {
-    return (label >= 1 && label <= B && z > 0.0f && isfinite(z)) ? label - 1 : -1;
+// object of pixel p (label b + 1 -> b) when the pixel is kept, else -1; n = objects of the pixel's frame
+__device__ __forceinline__ int kept_object(int label, float z, int n) {
+    return (label >= 1 && label <= n && z > 0.0f && isfinite(z)) ? label - 1 : -1;
 }
 
-struct Frame {
+// One stage-A call: F = gridDim.y frames of HW pixels, frame f at depth + f * HW.  frame_offsets == nullptr: one frame
+// holding objects [0, B) (gp_backproject_instances); otherwise frame f holds the objects ranges[f] .. ranges[f+1]-1,
+// which the count kernel derives from frame_offsets (clamp_range) and the scatter kernel reads back.
+struct Frames {
     const float *depth;
     const int32_t *labels;
-    int HW, B, n_tiles;
+    int HW, B, n_tiles;               // n_tiles: tiles of one frame
+    const float *intrinsics;          // [F][4] (fx, fy, cx, cy), or nullptr: the scatter kernel's arguments
+    const int32_t *frame_offsets;     // [F+1] as given, or nullptr
+    int *ranges;                      // [F+1] workspace: the clamped offsets
 };
 
+// The block's frame: its pixels and its objects lo .. lo + n - 1 (object label l of the frame is lo + l - 1).
+struct FrameView {
+    const float *depth;
+    const int32_t *labels;
+    int HW, n_tiles, lo, n;
+};
+
+__device__ __forceinline__ FrameView frame_view(const Frames &fr, int lo, int n) {
+    const size_t first = (size_t)blockIdx.y * fr.HW;
+    return FrameView{fr.depth + first, fr.labels + first, fr.HW, fr.n_tiles, lo, n};
+}
+
+// Frame f's object range [lo, hi) from frame_offsets, whatever it holds: offsets[0] is read as 0 and offsets[F] as B;
+// in between offsets[g] is raised to the largest of offsets[1..g] and clamped into [0, B].  The ranges are then
+// monotone, disjoint and cover [0, B), so every row of hist is written once and every output row is in bounds.
+__device__ __forceinline__ void clamp_range(const Frames &fr, int f, int &lo, int &hi) {
+    __shared__ int warp_max[WARPS];
+    int m = INT_MIN;
+    for (int g = 1 + threadIdx.x; g <= f; g += blockDim.x) m = max(m, __ldg(fr.frame_offsets + g));
+    m = __reduce_max_sync(0xffffffffu, m);
+    if ((threadIdx.x & 31) == 0) warp_max[threadIdx.x >> 5] = m;
+    __syncthreads();
+#pragma unroll
+    for (int w = 0; w < WARPS; ++w) m = max(m, warp_max[w]);
+    lo = min(max(m, 0), fr.B);
+    hi = f == (int)gridDim.y - 1 ? fr.B : max(lo, min(max(__ldg(fr.frame_offsets + f + 1), 0), fr.B));
+}
+
 // Walk warp `warp`'s tile of block blockIdx.x in pixel order, calling f(pixel, z, object, peers) once per round for
-// every lane (object -1 for a dropped pixel or one past the frame); peers = the lanes of the round with the same object.
+// every lane (object: frame-local, -1 for a dropped pixel or one past the frame); peers = the lanes of the round with
+// the same object.
 template <typename F>
-__device__ __forceinline__ void walk_tile(const Frame &fr, F &&f) {
+__device__ __forceinline__ void walk_tile(const FrameView &fr, F &&f) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int tile = blockIdx.x * WARPS + warp;
     if (tile >= fr.n_tiles) return;
@@ -82,7 +118,7 @@ __device__ __forceinline__ void walk_tile(const Frame &fr, F &&f) {
         }
 #pragma unroll
         for (int i = 0; i < BATCH; ++i) {
-            const int obj = kept_object(lab[i], z[i], fr.B);
+            const int obj = kept_object(lab[i], z[i], fr.n);
             const unsigned peers = __match_any_sync(0xffffffffu, obj);
             f(base + (r0 + i) * 32 + lane, z[i], obj, peers);
         }
@@ -90,12 +126,21 @@ __device__ __forceinline__ void walk_tile(const Frame &fr, F &&f) {
     }
 }
 
-__global__ void __launch_bounds__(WARPS * 32) count_kernel(Frame fr, int *__restrict__ hist) {
-    extern __shared__ int cnt[];   // [WARPS][B]
-    for (int i = threadIdx.x; i < WARPS * fr.B; i += blockDim.x) cnt[i] = 0;
+__global__ void __launch_bounds__(WARPS * 32) count_kernel(Frames frs, int *__restrict__ hist) {
+    extern __shared__ int cnt[];   // [WARPS][n]
+    int lo = 0, hi = frs.B;
+    if (frs.frame_offsets) {
+        clamp_range(frs, blockIdx.y, lo, hi);
+        if (blockIdx.x == 0 && threadIdx.x == 0) {
+            frs.ranges[blockIdx.y + 1] = hi;
+            if (blockIdx.y == 0) frs.ranges[0] = 0;
+        }
+    }
+    const FrameView fr = frame_view(frs, lo, hi - lo);
+    for (int i = threadIdx.x; i < WARPS * fr.n; i += blockDim.x) cnt[i] = 0;
     __syncthreads();
     const int lane = threadIdx.x & 31;
-    int *mine = cnt + (threadIdx.x >> 5) * fr.B;
+    int *mine = cnt + (threadIdx.x >> 5) * fr.n;
     walk_tile(fr, [&](int, float, int obj, unsigned peers) {
         if (obj >= 0 && lane == __ffs(peers) - 1) mine[obj] += __popc(peers);
         __syncwarp();
@@ -103,9 +148,9 @@ __global__ void __launch_bounds__(WARPS * 32) count_kernel(Frame fr, int *__rest
     __syncthreads();
     // hist[obj][tile]: the WARPS tiles of a block are contiguous in each object's row
     const int tiles_here = min(WARPS, fr.n_tiles - (int)blockIdx.x * WARPS);
-    for (int i = threadIdx.x; i < WARPS * fr.B; i += blockDim.x) {
+    for (int i = threadIdx.x; i < WARPS * fr.n; i += blockDim.x) {
         const int obj = i / WARPS, w = i % WARPS;
-        if (w < tiles_here) hist[(size_t)obj * fr.n_tiles + blockIdx.x * WARPS + w] = cnt[w * fr.B + obj];
+        if (w < tiles_here) hist[(size_t)(fr.lo + obj) * fr.n_tiles + blockIdx.x * WARPS + w] = cnt[w * fr.n + obj];
     }
 }
 
@@ -125,37 +170,48 @@ __global__ void __launch_bounds__(SCAN_THREADS) scan_kernel(int *__restrict__ hi
     if (threadIdx.x == 0) totals[blockIdx.x] = total;
 }
 
-__global__ void __launch_bounds__(WARPS * 32) scatter_kernel(Frame fr, int W, float fx, float fy, float cx, float cy,
+__global__ void __launch_bounds__(WARPS * 32) scatter_kernel(Frames frs, int W, float fx, float fy, float cx, float cy,
                                                              const int *__restrict__ hist,
                                                              const int *__restrict__ totals, float *__restrict__ xyz,
                                                              int32_t *__restrict__ offsets) {
     extern __shared__ int sm[];
     int *obj_off = sm;              // [B + 1]
-    int *cnt = sm + fr.B + 1;       // [WARPS][B]: next output row of each object in each warp's tile
-    const int B = fr.B;
+    int *cnt = sm + frs.B + 1;      // [WARPS][n]: next output row of each object of the frame in each warp's tile
+    const int B = frs.B;
+    int lo = 0, n = B;
+    if (frs.frame_offsets) {
+        lo = frs.ranges[blockIdx.y];
+        n = frs.ranges[blockIdx.y + 1] - lo;
+        const float *in = frs.intrinsics + (size_t)blockIdx.y * 4;
+        fx = in[0];
+        fy = in[1];
+        cx = in[2];
+        cy = in[3];
+    }
+    const FrameView fr = frame_view(frs, lo, n);
     // object offsets = exclusive scan of totals (each block redoes this small scan: no fourth launch)
     const int per = (B + blockDim.x - 1) / blockDim.x;
-    const int lo = min(B, (int)threadIdx.x * per), hi = min(B, lo + per);
+    const int o_lo = min(B, (int)threadIdx.x * per), o_hi = min(B, o_lo + per);
     int s = 0;
-    for (int i = lo; i < hi; ++i) s += totals[i];
+    for (int i = o_lo; i < o_hi; ++i) s += totals[i];
     int total;
     int run = block_exclusive_scan(s, total);
-    for (int i = lo; i < hi; ++i) {
+    for (int i = o_lo; i < o_hi; ++i) {
         obj_off[i] = run;
         run += totals[i];
     }
     if (threadIdx.x == 0) obj_off[B] = total;
     __syncthreads();
-    if (blockIdx.x == 0)
+    if (blockIdx.x == 0 && blockIdx.y == 0)
         for (int i = threadIdx.x; i <= B; i += blockDim.x) offsets[i] = obj_off[i];
-    for (int i = threadIdx.x; i < WARPS * B; i += blockDim.x) {
+    for (int i = threadIdx.x; i < WARPS * n; i += blockDim.x) {
         const int obj = i / WARPS, w = i % WARPS, tile = blockIdx.x * WARPS + w;
-        if (tile < fr.n_tiles) cnt[w * B + obj] = obj_off[obj] + hist[(size_t)obj * fr.n_tiles + tile];
+        if (tile < fr.n_tiles) cnt[w * n + obj] = obj_off[lo + obj] + hist[(size_t)(lo + obj) * fr.n_tiles + tile];
     }
     __syncthreads();
     const int lane = threadIdx.x & 31;
     const unsigned lanes_below = (1u << lane) - 1u;
-    int *mine = cnt + (threadIdx.x >> 5) * B;
+    int *mine = cnt + (threadIdx.x >> 5) * n;
     walk_tile(fr, [&](int p, float z, int obj, unsigned peers) {
         const int next = obj >= 0 ? mine[obj] : 0;
         __syncwarp();
@@ -262,6 +318,22 @@ __global__ void __launch_bounds__(SAMPLE_THREADS) sample_kernel(const float *__r
 
 inline int n_tiles(int H, int W) { return (int)(((long long)H * W + TILE - 1) / TILE); }
 
+// The three launches of stage A over F frames; the workspace holds hist [B][n_tiles], totals [B] and (F frames given
+// by frame_offsets) the clamped offsets [F+1].
+inline int launch_stage_a(const Frames &fr, int F, int W, float fx, float fy, float cx, float cy, float *xyz,
+                          int32_t *offsets, int *hist, cudaStream_t st, const char *name) {
+    int *totals = hist + (size_t)fr.B * fr.n_tiles;
+    const dim3 grid((unsigned)((fr.n_tiles + WARPS - 1) / WARPS), (unsigned)F);
+    count_kernel<<<grid, WARPS * 32, WARPS * fr.B * sizeof(int), st>>>(fr, hist);
+    GP_CHECK_LAUNCH(name);
+    scan_kernel<<<(unsigned)fr.B, SCAN_THREADS, 0, st>>>(hist, fr.n_tiles, totals);
+    GP_CHECK_LAUNCH(name);
+    scatter_kernel<<<grid, WARPS * 32, ((WARPS + 1) * fr.B + 1) * sizeof(int), st>>>(fr, W, fx, fy, cx, cy, hist,
+                                                                                   totals, xyz, offsets);
+    GP_CHECK_LAUNCH(name);
+    return GP_OK;
+}
+
 }  // namespace clouds
 }  // namespace gp
 
@@ -290,19 +362,43 @@ extern "C" int gp_backproject_instances(const float *depth, const int32_t *label
         gp::set_error("gp_backproject_instances: workspace of %zu bytes, %zu needed", workspace_bytes, need);
         return GP_ERR_WORKSPACE;
     }
-    const Frame fr{depth, labels, H * W, B, n_tiles(H, W)};
+    const Frames fr{depth, labels, H * W, B, n_tiles(H, W), nullptr, nullptr, nullptr};
+    return launch_stage_a(fr, 1, W, fx, fy, cx, cy, xyz, offsets, (int *)workspace, gp::as_stream(s),
+                          "gp_backproject_instances");
+}
+
+extern "C" size_t gp_backproject_frames_workspace_bytes(int F, int H, int W, int B) {
+    if (F < 1 || F > GP_MAX_FRAMES || H < 1 || W < 1 || B < 1 || B > GP_MAX_FRAME_OBJECTS ||
+        (long long)F * H * W > GP_MAX_FRAME_PIXELS)
+        return 0;
+    return ((size_t)B * n_tiles(H, W) + (size_t)B + (size_t)F + 1) * sizeof(int);
+}
+
+extern "C" int gp_backproject_frames(const float *depth, const int32_t *labels, int F, int H, int W,
+                                     const float *intrinsics, const int32_t *frame_offsets, int B, float *xyz,
+                                     int32_t *offsets, void *workspace, size_t workspace_bytes, gp_stream_t s) {
+    GP_REQUIRE(F >= 1 && H >= 1 && W >= 1 && B >= 1, "gp_backproject_frames: bad sizes F=%d H=%d W=%d B=%d", F, H, W,
+               B);
+    GP_REQUIRE((long long)F * H * W <= GP_MAX_FRAME_PIXELS, "gp_backproject_frames: %d frames of %d x %d too large", F,
+               H, W);
+    if (B > GP_MAX_FRAME_OBJECTS || F > GP_MAX_FRAMES) {
+        gp::set_error("gp_backproject_frames: F=%d frames and B=%d objects, at most %d and %d supported", F, B,
+                      (int)GP_MAX_FRAMES, (int)GP_MAX_FRAME_OBJECTS);
+        return GP_ERR_UNSUPPORTED;
+    }
+    GP_REQUIRE(depth && labels && intrinsics && frame_offsets && xyz && offsets && workspace,
+               "gp_backproject_frames: null pointer");
+    const size_t need = gp_backproject_frames_workspace_bytes(F, H, W, B);
+    if (workspace_bytes < need) {
+        gp::set_error("gp_backproject_frames: workspace of %zu bytes, %zu needed", workspace_bytes, need);
+        return GP_ERR_WORKSPACE;
+    }
+    const int T = n_tiles(H, W);
     int *hist = (int *)workspace;
-    int *totals = hist + (size_t)B * fr.n_tiles;
-    const cudaStream_t st = gp::as_stream(s);
-    const unsigned blocks = (unsigned)((fr.n_tiles + WARPS - 1) / WARPS);
-    count_kernel<<<blocks, WARPS * 32, WARPS * B * sizeof(int), st>>>(fr, hist);
-    GP_CHECK_LAUNCH("gp_backproject_instances (count)");
-    scan_kernel<<<(unsigned)B, SCAN_THREADS, 0, st>>>(hist, fr.n_tiles, totals);
-    GP_CHECK_LAUNCH("gp_backproject_instances (scan)");
-    scatter_kernel<<<blocks, WARPS * 32, ((WARPS + 1) * B + 1) * sizeof(int), st>>>(fr, W, fx, fy, cx, cy, hist,
-                                                                                   totals, xyz, offsets);
-    GP_CHECK_LAUNCH("gp_backproject_instances (scatter)");
-    return GP_OK;
+    int *ranges = hist + (size_t)B * T + B;
+    const Frames fr{depth, labels, H * W, B, T, intrinsics, frame_offsets, ranges};
+    return launch_stage_a(fr, F, W, 0.0f, 0.0f, 0.0f, 0.0f, xyz, offsets, hist, gp::as_stream(s),
+                          "gp_backproject_frames");
 }
 
 extern "C" int gp_sample_points(const float *xyz, long long rows, const int32_t *offsets, const int64_t *keys, int B,

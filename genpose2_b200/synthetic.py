@@ -214,3 +214,17 @@ def make_instance_frame(H, W, num_objects, seed=0, bad_depth=0.0, stray_labels=0
     stray = rng.random((H, W)) < stray_labels
     labels[stray] = rng.choice(np.array([0, -1, B + 1, 1 << 30], dtype=np.int32), int(stray.sum()))
     return depth, labels
+
+
+def make_instance_frames(H, W, objects_per_frame, seed=0, bad_depth=0.0, stray_labels=0.0):
+    """F frames of make_instance_frame (the input of clouds.object_clouds_frames), frame f with objects_per_frame[f]
+    objects and seed + f; a frame of 0 objects is a 1-object frame whose labels are all background (label 1 is above
+    its count).  Each frame gets its own camera: focal lengths 0.9-1.1 x 600 * W / 640, the principal point within a
+    few pixels of the centre.  Returns (depth float32 [F,H,W], labels int32 [F,H,W], intrinsics float64 [F,4])."""
+    depth, labels = zip(*(make_instance_frame(H, W, max(n, 1), seed=seed + f, bad_depth=bad_depth,
+                                              stray_labels=stray_labels) for f, n in enumerate(objects_per_frame)))
+    rng = np.random.default_rng(seed)
+    F = len(objects_per_frame)
+    focal = 600.0 * W / 640 * rng.uniform(0.9, 1.1, size=(F, 2))
+    centre = np.array([W / 2.0, H / 2.0]) + rng.uniform(-4.0, 4.0, size=(F, 2))
+    return np.stack(depth), np.stack(labels), np.concatenate([focal, centre], axis=1)

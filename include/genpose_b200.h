@@ -379,9 +379,9 @@ GP_API int gp_object_noise(const int64_t *keys, const float *sigma, int B, int R
  * (datasets/datasets_omni6dpose.py:459-473).
  * ------------------------------------------------------------------------------------------ */
 
-/* Most objects and pixels one gp_backproject_instances call takes (2^30 pixels keeps every pixel index of the
- * 1024-pixel tiles inside int). */
-enum { GP_MAX_FRAME_OBJECTS = 1024, GP_MAX_FRAME_PIXELS = 1 << 30 };
+/* Most objects and pixels one gp_backproject_instances or gp_backproject_frames call takes (2^30 pixels keeps every
+ * pixel index of the 1024-pixel tiles inside int), and most frames one gp_backproject_frames call takes. */
+enum { GP_MAX_FRAME_OBJECTS = 1024, GP_MAX_FRAME_PIXELS = 1 << 30, GP_MAX_FRAMES = 1024 };
 
 /* Stage A, back-projection and stable per-object compaction.
  *   depth  [H,W] f32 metres;  labels [H,W] i32: value b+1 is object b, values outside 1..B are background.
@@ -398,6 +398,27 @@ GP_API size_t gp_backproject_instances_workspace_bytes(int H, int W, int B);
 GP_API int gp_backproject_instances(const float *depth, const int32_t *labels, int H, int W, float fx, float fy,
                                     float cx, float cy, int B, float *xyz, int32_t *offsets, void *workspace,
                                     size_t workspace_bytes, gp_stream_t s);
+
+/* Stage A over F frames of one size in one pass (a batch of tracked videos, a multi-camera rig).
+ *   depth [F,H,W] f32, labels [F,H,W] i32, intrinsics [F][4] f32 (fx, fy, cx, cy of each frame, device),
+ *   frame_offsets [F+1] i32 (device): frame f holds the objects frame_offsets[f] .. frame_offsets[f+1]-1, numbered
+ *   frame-major; label l of frame f with 1 <= l <= n_f = frame_offsets[f+1] - frame_offsets[f] is object
+ *   frame_offsets[f] + l - 1, any other label (one above n_f too) is background.  Pixel rules and arithmetic are
+ *   gp_backproject_instances', with the pixel's own frame's intrinsics.
+ *   xyz [F*H*W, 3] f32 (capacity-sized), offsets [B+1] i32: bit for bit the concatenation, in frame order, of F
+ *   gp_backproject_instances calls (object b in rows offsets[b] .. offsets[b+1]-1, row-major pixel order of its frame).
+ * frame_offsets is never read on the host, so one captured graph replays new per-frame object counts.  Whatever it
+ * holds, the kernels read and write in bounds: frame_offsets[0] is taken as 0 and frame_offsets[F] as B, and each
+ * frame_offsets[f] in between is raised to the largest of frame_offsets[1..f] and clamped into [0, B] (malformed
+ * offsets give wrong clouds, never an out-of-bounds access).  Zero or non-finite intrinsics give non-finite points.
+ * B > GP_MAX_FRAME_OBJECTS or F > GP_MAX_FRAMES returns GP_ERR_UNSUPPORTED, F * H * W > GP_MAX_FRAME_PIXELS
+ * GP_ERR_BAD_ARG (the workspace query returns 0 for these and for bad sizes).  Workspace:
+ * (B * ceil(H*W / 1024) + B + F + 1) ints.  Three kernel launches, no host synchronisation; with F = 1, objects
+ * [0, B) and the same intrinsics the result equals gp_backproject_instances'. */
+GP_API size_t gp_backproject_frames_workspace_bytes(int F, int H, int W, int B);
+GP_API int gp_backproject_frames(const float *depth, const int32_t *labels, int F, int H, int W,
+                                 const float *intrinsics, const int32_t *frame_offsets, int B, float *xyz,
+                                 int32_t *offsets, void *workspace, size_t workspace_bytes, gp_stream_t s);
 
 /* Stage B, sample_points (datasets_omni6dpose.py:459-473) with a keyed random choice.  Object b has the K points
  * xyz[offsets[b] .. offsets[b+1]-1] (offsets clamped into [0, rows] first; K = 0 when they cross); pts [B,N,3] f32:
